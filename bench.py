@@ -2,7 +2,7 @@
 """bench.py - env-steps/s of 11x11 random self-play (BASELINE.json config 3) on N B200s, with the HBM roofline of the
 fused step kernel and the CPU restatement of the reference loop timed beside it.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path (one JSON line on rank 0)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path (one JSON line on rank 0)
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   # the CPU reference arm (rank 0 only)
 
 A "step" is one fused env step (agent ply + random-opponent reply + win check + reward/done + auto-reset + observation
@@ -250,7 +250,8 @@ def pin_rank_cpus(local, local_world):
 
 
 def capture_steps(env, dev, n, **kw):
-    """n calls of env.step(**kw) as ONE CUDA graph (a replay = n step-kernel launches, no host work in between)."""
+    """n calls of env.step(**kw) as ONE CUDA graph (a replay = n step-kernel launches, no host work in between).
+    g.outputs holds the tensors the last captured step writes."""
     import torch
     side = torch.cuda.Stream(device=dev)
     side.wait_stream(torch.cuda.current_stream(dev))
@@ -258,9 +259,27 @@ def capture_steps(env, dev, n, **kw):
     with torch.cuda.stream(side):
         with torch.cuda.graph(g, stream=side):
             for _ in range(n):
-                env.step(**kw)
+                g.outputs = env.step(**kw)
     torch.cuda.current_stream(dev).wait_stream(side)
     return g
+
+
+DUMP_BYTES = 48 << 20    # --dump-outputs: at most this much float32 in all
+
+
+def dump_outputs(out_dir, step_out, G, game_offset, max_bytes=DUMP_BYTES):
+    """Write the last timed step's outputs (obs, mask, reward, done: what env.step() returns) as float32 .npy files, for a
+    fixed, seeded sample of the games that fits max_bytes, and the sample's global game indices as game_index.npy (float64)."""
+    import numpy as np
+    import torch
+    per_game = sum(4 * (t[0].numel() if t.dim() > 1 else 1) for t in step_out.values()) + 8
+    S = min(G, max_bytes // per_game)
+    idx = np.sort(np.random.default_rng(0).choice(G, S, replace=False))
+    rows = torch.from_numpy(idx).to(next(iter(step_out.values())).device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "game_index.npy"), (idx + game_offset).astype(np.float64))
+    for name, t in step_out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, rows).to(torch.float32).cpu().numpy())
 
 
 def time_steps(env, dev, K, use_graph, reps=1):
@@ -373,9 +392,10 @@ def run_gpu(args):
     e0.record()
     if graph is not None:
         graph.replay()                   # exactly K step launches
+        last = graph.outputs
     else:
         for _ in range(K):
-            env.step()
+            last = env.step()
     e1.record()
     # K7 + the path's only collective (64 bytes), on a side stream that waits for the K steps: it is never between two step
     # kernels, and it is outside the [e0, e1] bracket (timed on its own as collective_ms)
@@ -396,6 +416,8 @@ def run_gpu(args):
     launches = K
     value = world * G * K / (ms * 1e-3)
     ds = (stats - s0).cpu().tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, G, rank * G)
 
     peaks = {}
     try:
@@ -550,7 +572,13 @@ def main():
     ap.add_argument("--preroll", type=int, default=2000, help="untimed env steps (one hexb_rollout launch) before warm-up: de-synchronises the games")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_configs block of the 1-GPU line")
     ap.add_argument("--ref-budget", type=float, default=45.0, help="--impl reference: seconds of CPU sampling in total")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's obs / mask / reward / done "
+                    "(rank 0's games, a fixed sample of at most 48 MiB) as DIR/<name>.npy in float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device path's outputs; the reference arm has none")
     args.out = _claim_stdout()
     if args.impl == "reference":
         run_reference(args)

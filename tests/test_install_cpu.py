@@ -2,6 +2,7 @@
 kept identical to the repository's canonical include/hexb.h), every source the library is built from, and a prebuilt library
 loads from it with every declared symbol."""
 import os
+import shutil
 import subprocess
 import sys
 
@@ -19,19 +20,14 @@ def test_packaged_header_is_the_canonical_one():
 def test_pip_install_target_is_self_contained(tmp_path):
     target = tmp_path / "site"
     work = tmp_path / "src"          # build from a copy: setuptools writes build/ and *.egg-info next to pyproject.toml
-    subprocess.run(["git", "-C", ROOT, "checkout-index", "-a", "--prefix=%s/" % work], check=True)
-    for so in ("libhexb.so",):       # the prebuilt library travels like on the GPU box (git-ignored, present in the tree)
-        src = os.path.join(ROOT, "hex_gym_env_b200", so)
-        if not os.path.exists(src):
-            pytest.skip("libhexb.so has not been built in this tree")
-        subprocess.run(["cp", "-p", src, str(work / "hex_gym_env_b200" / so)], check=True)
-    # the working tree may be ahead of the index: take the package's current sources
-    subprocess.run(["cp", "-rp", os.path.join(ROOT, "hex_gym_env_b200", "csrc"), os.path.join(ROOT, "hex_gym_env_b200", "include"),
-                    str(work / "hex_gym_env_b200")], check=True)
-    subprocess.run(["cp", os.path.join(ROOT, "pyproject.toml"), str(work)], check=True)
-    for f in os.listdir(os.path.join(ROOT, "hex_gym_env_b200")):
-        if f.endswith(".py"):
-            subprocess.run(["cp", os.path.join(ROOT, "hex_gym_env_b200", f), str(work / "hex_gym_env_b200" / f)], check=True)
+    lib = os.path.join(ROOT, "hex_gym_env_b200", "libhexb.so")
+    if not os.path.exists(lib):
+        pytest.skip("libhexb.so has not been built in this tree")
+    # the package's current sources (the tree need not be a git checkout), without the products of an in-tree build
+    shutil.copytree(os.path.join(ROOT, "hex_gym_env_b200"), str(work / "hex_gym_env_b200"),
+                    ignore=shutil.ignore_patterns("build", "__pycache__", "*.so", "*.lock", "*.tmp"))
+    shutil.copy(os.path.join(ROOT, "pyproject.toml"), str(work))
+    shutil.copy2(lib, str(work / "hex_gym_env_b200" / "libhexb.so"))   # the prebuilt library ships with the package
     os.utime(str(work / "hex_gym_env_b200" / "libhexb.so"))     # the library is newer than its sources: the install must not rebuild
     r = subprocess.run([sys.executable, "-m", "pip", "install", "--no-index", "--no-build-isolation", "--no-deps", "--quiet",
                         "--target", str(target), str(work)], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
