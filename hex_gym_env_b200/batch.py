@@ -15,6 +15,8 @@ What each method replaces in the reference (MBPrdctns/hex_gym_env, paths relativ
   sample_actions()   BaseRandomPolicy.choose_action (SelfplayWrapper.py:17-22) / random_policy (minihex/__init__.py:8-12)
   export_state()     attribute reads .board / .regions / .region_counter / .current_player_num / .done / .winner
   import_boards()    HexGame.__init__ with a preset board (HexGame.py:53-61, HexSingleGame.py:57-65)
+  copy_games()       copy.deepcopy(env.simulator) into a raw batch (tree search: branching a position)
+  playouts()         random playouts to the end from the current position (tree search: Monte-Carlo value estimates)
 """
 import ctypes
 import os
@@ -538,6 +540,39 @@ class HexBatch(object):
         im = self._in(import_mask, (self.G,), torch.uint8, "import_mask")
         with torch.cuda.device(self.device):
             check(self._lib.hexb_import_labels(self._h, _ptr(b), _ptr(r), _ptr(tm), _ptr(im), self._stream()))
+
+    # ------------------------------------------------------------------ tree search
+    def copy_games(self, src, src_index=None, dst_index=None):
+        """copy.deepcopy(env.simulator) for many games: game dst_index[i] of this RAW batch becomes a bare HexGame holding the
+        position of game src_index[i] of `src` (any HexBatch of the same board size and variant on the same device), with the exact
+        region counters; an env game whose agent is WHITE is converted to true coordinates. Indices are int64[count] (None = the
+        identity; count = the length of a given index, else min of the two batch sizes); dst_index entries must be distinct and, when
+        src is self, disjoint from the src games. Out-of-range pairs write nothing; games not named are untouched."""
+        if not self.raw:
+            raise ValueError("copy_games writes into a raw HexBatch (bare HexGame games)")
+        if not isinstance(src, HexBatch) or src.N != self.N or src.variant != self.variant or src.device != self.device:
+            raise ValueError("copy_games: src must be a HexBatch with the same board size and variant on %s" % self.device)
+        lens = [int(torch.as_tensor(x).numel()) for x in (src_index, dst_index) if x is not None]
+        if len(set(lens)) > 1:
+            raise ValueError("src_index and dst_index must have the same length, got %s" % lens)
+        count = lens[0] if lens else min(self.G, src.G)
+        si = self._in(src_index, (count,), torch.int64, "src_index")
+        di = self._in(dst_index, (count,), torch.int64, "dst_index")
+        with torch.cuda.device(self.device):
+            check(self._lib.hexb_copy_games(self._h, src._h, _ptr(si), _ptr(di), count, self._stream()))
+
+    def playouts(self, num_playouts, first_playout=0, game_mask=None, out=None):
+        """num_playouts random playouts per game from its current position (random_policy for both sides, filled to the end);
+        returns int32[G]: playouts won by the side to move, -1 for finished, never-reset and masked-off (game_mask u8[G] == 0)
+        games. Playout p uses its own stream (Philox counter c3 = p + 1), p in [first_playout, first_playout + num_playouts)."""
+        num_playouts, first_playout = int(num_playouts), int(first_playout)
+        if num_playouts < 1 or first_playout < 0 or first_playout + num_playouts >= 1 << 32:
+            raise ValueError("need num_playouts >= 1, first_playout >= 0 and first_playout + num_playouts < 2**32")
+        gm = self._in(game_mask, (self.G,), torch.uint8, "game_mask")
+        out = self._chk(out, (self.G,), torch.int32, "out") if out is not None else torch.empty(self.G, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self._lib.hexb_playouts(self._h, num_playouts, first_playout, _ptr(gm), _ptr(out), self._stream()))
+        return out
 
     def opponent_catch_up(self):
         """Let the built-in random opponent move in every game where it is to move (after import_boards on an env handle):

@@ -1,14 +1,14 @@
 // hexb_host.h - host-side declarations shared by the translation units of libhexb.so (not part of the C ABI).
 //
 // The library is built from one object per board size (hexb_step_inst.cu compiled with -DHEXB_INST_N=n: every instantiation of
-// the step kernels for that N plus the two small per-N kernels) and hexb_kernels.cu (the C ABI, the size-independent kernels and
+// the step kernels for that N plus the small per-N kernels: sampler, import, playouts) and hexb_kernels.cu (the C ABI, the size-independent kernels and
 // the dispatch tables). The per-N objects are independent, so hex_gym_env_b200/_native.py compiles them in parallel.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "../include/hexb.h"
-#include "hexb_views.cuh"
+#include "hexb_search.cuh"
 
 #define HEXB_LOCAL __attribute__((visibility("hidden")))
 
@@ -46,6 +46,7 @@ HEXB_LOCAL int hexb_cuda_fail(cudaError_t e);   // records the code for hexb_las
     HEXB_LOCAL int hexb_launch_tile_##n(const hexb_env *e, const hexb::Params &P, cudaStream_t s);                          \
     HEXB_LOCAL int hexb_launch_sample_##n(const hexb::View &V, int view, const double *u, int32_t *out, cudaStream_t s);     \
     HEXB_LOCAL int hexb_launch_import_##n(const hexb::Params &P, const int8_t *board_true, const int8_t *to_move,           \
-                                          const uint8_t *import_mask, cudaStream_t s);
+                                          const uint8_t *import_mask, cudaStream_t s);                                      \
+    HEXB_LOCAL int hexb_launch_playouts_##n(const hexb::View &V, const hexb::PlayoutArgs &A, cudaStream_t s);
 HEXB_FOR_N(HEXB_DECL_N)
 #undef HEXB_DECL_N

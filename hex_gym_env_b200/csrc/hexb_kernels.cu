@@ -13,6 +13,8 @@
 //   K8        hexb_masked_sample_kernel   masked categorical sampling (the rollout feed)
 //   K9        hexb_gae_kernel         GAE(lambda) advantages / returns over a [T,G] rollout (SB3 RolloutBuffer semantics)
 //   K10       hexb_pack_obs_kernel    2-bit observation transport for hexb_step_host_packed
+//   K11       hexb_copy_kernel        copy.deepcopy(env.simulator) into a raw batch, one warp per copied game (hexb_search.cuh)
+//   K12       hexb_playout_kernel<N>  random playouts from the current position, one warp per game (hexb_step_inst.cu)
 #include <cuda.h>   // types of the driver's virtual-memory API only (entry points come from cudaGetDriverEntryPoint)
 #include <cuda_runtime.h>
 #include <math.h>
@@ -44,6 +46,26 @@ __global__ void hexb_import_labels_kernel(Params P, int N, const int8_t *board_t
                                           const uint8_t *import_mask) {
     const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (g < P.G) import_labels_game(P, N, g, board_true, planes, to_move, import_mask);
+}
+
+// K11: one warp per copied game; lane l writes cells l, l + 32, ... and the ballot of their stones is the occupancy word
+__global__ void __launch_bounds__(128) hexb_copy_kernel(CopyArgs A) {
+    const int lane = threadIdx.x & 31;
+    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    long long s, d;
+    if (i >= A.count || !copy_pair(A, i, s, d)) return;
+    const int C = A.N * A.N, W = (C + 31) / 32;
+    const uint32_t meta = copy_src_meta(A, s);
+    const int tr = (meta & M_TRANSPOSED) ? 1 : 0;
+    for (int w = 0; w < W; ++w) {
+        const int c = 32 * w + lane;
+        const uint32_t occ = __ballot_sync(0xffffffffu, c < C && copy_cell(A, s, d, c, tr));
+        if (lane == 0) copy_store_rec(A, d, w, occ);
+    }
+    if (lane == 0) {
+        copy_store_rec(A, d, W, copy_meta(meta));
+        copy_store_rec(A, d, W + 1, 0u);   // draws: a raw game has no stream
+    }
 }
 
 __global__ void hexb_stats_kernel(const long long *src, int64_t *dst) {
@@ -219,6 +241,10 @@ static const sample_fn k_sample[] = {HEXB_FOR_N(X)};
 #define X(n) hexb_launch_import_##n,
 static const import_fn k_import[] = {HEXB_FOR_N(X)};
 #undef X
+typedef int (*playouts_fn)(const View &, const PlayoutArgs &, cudaStream_t);
+#define X(n) hexb_launch_playouts_##n,
+static const playouts_fn k_playouts[] = {HEXB_FOR_N(X)};
+#undef X
 
 static int dispatch_tile(const hexb_env *e, const Params &P, cudaStream_t s) {
     const int n = e->cfg.board_size;
@@ -249,7 +275,7 @@ extern "C" HEXB_LOCAL void hexb_hostpack_finish(int abort);
 
 extern "C" {
 
-int32_t hexb_version(void) { return (1 << 16) | 4; }   // 1.3: obs_dtype, launch forms, hexb_gae, packed / asynchronous host step (+ hexb_mem_alloc: additive); 1.4: hexb_set_eval, hexb_set_opponent_eps
+int32_t hexb_version(void) { return (1 << 16) | 5; }   // 1.3: obs_dtype, launch forms, hexb_gae, packed / asynchronous host step (+ hexb_mem_alloc: additive); 1.4: hexb_set_eval, hexb_set_opponent_eps; 1.5: hexb_copy_games, hexb_playouts
 
 const char *hexb_strerror(int32_t code) {
     switch (code) {
@@ -890,6 +916,42 @@ int32_t hexb_import_labels(hexb_env *env, const int8_t *board_true, const uint8_
                                                                                                 to_move, import_mask);
     CK(cudaGetLastError());
     return HEXB_OK;
+}
+
+int32_t hexb_copy_games(hexb_env *dst, const hexb_env *src, const int64_t *src_index, const int64_t *dst_index, int64_t count,
+                        void *stream) {
+    if (!dst || !src || !dst->cfg.raw || count < 0) return HEXB_ERR_ARG;
+    if (dst->cfg.board_size != src->cfg.board_size || dst->cfg.variant != src->cfg.variant || dst->cfg.device != src->cfg.device)
+        return HEXB_ERR_ARG;
+    if (count == 0) return HEXB_OK;
+    CK(cudaSetDevice(dst->cfg.device));
+    CopyArgs A;
+    A.dst = dst->base.state;
+    A.src = src->base.state;
+    A.dst_G = dst->base.G;
+    A.src_G = src->base.G;
+    A.count = count;
+    A.src_index = src_index;
+    A.dst_index = dst_index;
+    A.N = dst->cfg.board_size;
+    hexb_copy_kernel<<<(unsigned)((count + 3) / 4), 128, 0, (cudaStream_t)stream>>>(A);
+    CK(cudaGetLastError());
+    return HEXB_OK;
+}
+
+int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout, const uint8_t *game_mask, int32_t *wins,
+                      void *stream) {
+    if (!env || !wins || num_playouts < 1 || first_playout < 0 || first_playout + (int64_t)num_playouts >= (1ll << 32)) return HEXB_ERR_ARG;
+    CK(cudaSetDevice(env->cfg.device));
+    const View V = view_of(env);
+    PlayoutArgs A;
+    A.seed = env->base.seed;
+    A.game_offset = (unsigned long long)env->base.game_offset;
+    A.first = first_playout;
+    A.num = num_playouts;
+    A.game_mask = game_mask;
+    A.wins = wins;
+    return k_playouts[V.N - HEXB_MIN_BOARD](V, A, (cudaStream_t)stream);
 }
 
 int32_t hexb_stats(hexb_env *env, int64_t *out8, void *stream) {

@@ -20,6 +20,27 @@ __global__ void hexb_import_kernel(Params P, const int8_t *board_true, const int
     if (g < P.G) import_game<N>(P, g, board_true, to_move, import_mask);
 }
 
+// hexb_playouts: one warp per game, lane l takes playouts first + l, first + l + 32, ... (every playout of a game fills the same
+// number of cells, so the lanes stay converged until the connectivity test)
+template <int N>
+__global__ void __launch_bounds__(256) hexb_playout_kernel(View V, PlayoutArgs A) {
+    const int lane = threadIdx.x & 31;
+    const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (g >= V.G) return;
+    uint32_t black[N], empty[N];
+    const int to_move = (A.game_mask && !A.game_mask[g]) ? -1 : playout_rows<N>(V, g, black, empty);
+    if (to_move < 0) {
+        if (lane == 0) A.wins[g] = -1;
+        return;
+    }
+    const unsigned long long gid = A.game_offset + (unsigned long long)g;
+    int won = 0;
+    for (int j = lane; j < A.num; j += 32)
+        won += playout_winner<N>(black, empty, to_move, A.seed, gid, (uint32_t)(A.first + j)) == to_move;
+    won = __reduce_add_sync(0xffffffffu, won);
+    if (lane == 0) A.wins[g] = won;
+}
+
 int HEXB_CAT(hexb_launch_tile_, HEXB_INST_N)(const hexb_env *e, const Params &P, cudaStream_t s) { return launch_tile<HEXB_INST_N>(e, P, s); }
 
 int HEXB_CAT(hexb_launch_sample_, HEXB_INST_N)(const View &V, int view, const double *u, int32_t *out, cudaStream_t s) {
@@ -31,6 +52,12 @@ int HEXB_CAT(hexb_launch_sample_, HEXB_INST_N)(const View &V, int view, const do
 int HEXB_CAT(hexb_launch_import_, HEXB_INST_N)(const Params &P, const int8_t *board_true, const int8_t *to_move, const uint8_t *import_mask,
                                                cudaStream_t s) {
     hexb_import_kernel<HEXB_INST_N><<<(unsigned)((P.G + 127) / 128), 128, 0, s>>>(P, board_true, to_move, import_mask);
+    CK(cudaGetLastError());
+    return HEXB_OK;
+}
+
+int HEXB_CAT(hexb_launch_playouts_, HEXB_INST_N)(const View &V, const PlayoutArgs &A, cudaStream_t s) {
+    hexb_playout_kernel<HEXB_INST_N><<<(unsigned)((V.G + 7) / 8), 256, 0, s>>>(V, A);
     CK(cudaGetLastError());
     return HEXB_OK;
 }

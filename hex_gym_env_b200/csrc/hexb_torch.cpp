@@ -158,6 +158,30 @@ void op_set_eval(int64_t handle, bool eval_state, OptT eval_episode) {
     check_rc(hexb_set_eval(k.e, eval_state ? 1 : 0, ptr<int32_t>(eval_episode, at::kInt, k.G, k.c.device, "eval_episode"), k.stream), "set_eval");
 }
 
+// copy.deepcopy(env.simulator) into a raw handle: dst game dst_index[i] <- src game src_index[i] (int64[count], None = identity)
+void op_copy_games(int64_t dst, int64_t src, OptT src_index, OptT dst_index, int64_t count) {
+    Call k(dst);
+    const hexb_config sc = config_of(env_of(src));
+    TORCH_CHECK(k.c.raw, "hexb::copy_games: dst must be a raw handle");
+    TORCH_CHECK(sc.board_size == k.c.board_size && sc.variant == k.c.variant && sc.device == k.c.device,
+                "hexb::copy_games: src and dst differ in board_size, variant or device");
+    TORCH_CHECK(count >= 0, "hexb::copy_games: count must be >= 0");
+    const int d = k.c.device;
+    check_rc(hexb_copy_games(k.e, env_of(src), ptr<const int64_t>(src_index, at::kLong, count, d, "src_index"),
+                             ptr<const int64_t>(dst_index, at::kLong, count, d, "dst_index"), count, k.stream),
+             "copy_games");
+}
+
+void op_playouts(int64_t handle, int64_t num_playouts, int64_t first_playout, OptT game_mask, Tensor wins) {
+    Call k(handle);
+    const int d = k.c.device;
+    TORCH_CHECK(num_playouts >= 1 && num_playouts <= INT32_MAX && first_playout >= 0 && first_playout + num_playouts < (1ll << 32),
+                "hexb::playouts: need num_playouts >= 1, first_playout >= 0 and first_playout + num_playouts < 2^32");
+    check_rc(hexb_playouts(k.e, (int32_t)num_playouts, first_playout, ptr<const uint8_t>(game_mask, at::kByte, k.G, d, "game_mask"),
+                           ptr<int32_t>(wins, at::kInt, k.G, d, "wins"), k.stream),
+             "playouts");
+}
+
 int64_t op_version() { return hexb_version(); }
 
 }  // namespace
@@ -178,6 +202,8 @@ TORCH_LIBRARY(hexb, m) {
     m.def("gae(Tensor rewards, Tensor values, Tensor dones, float gamma, float gae_lambda, Tensor(a!) advantages, Tensor(b!)? returns) -> ()");
     m.def("set_launch_form(int env, int warps_per_chunk) -> ()", &op_set_launch_form);
     m.def("set_eval(int env, bool eval_state, Tensor(a!)? eval_episode) -> ()");
+    m.def("copy_games(int dst, int src, Tensor? src_index, Tensor? dst_index, int count) -> ()");
+    m.def("playouts(int env, int num_playouts, int first_playout, Tensor? game_mask, Tensor(a!) wins) -> ()");
 }
 
 // The handle is an int, so these operators have no tensor argument to dispatch on when every optional is None: register them
@@ -194,4 +220,6 @@ TORCH_LIBRARY_IMPL(hexb, CompositeExplicitAutograd, m) {
     m.impl("masked_sample", &op_masked_sample);
     m.impl("gae", &op_gae);
     m.impl("set_eval", &op_set_eval);
+    m.impl("copy_games", &op_copy_games);
+    m.impl("playouts", &op_playouts);
 }

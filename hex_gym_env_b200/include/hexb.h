@@ -223,6 +223,34 @@ int32_t hexb_import_boards(hexb_env *env, const int8_t *board_true, const int8_t
 int32_t hexb_import_labels(hexb_env *env, const int8_t *board_true, const uint8_t *regions, const int8_t *to_move,
                            const uint8_t *import_mask, void *stream);
 
+/* Tree-search primitives (library version 1.5).
+ *
+ * copy.deepcopy(env.simulator) for many games at once (the HexGame.__init__ state, HexGame.py:21-68, HexSingleGame.py:26-71: board,
+ * regions, region_counter, current_player_num, done, winner). dst game dst_index[i] becomes a bare HexGame holding the position of
+ * src game src_index[i], for i < count. dst must be a raw=1 handle; src may be any handle of the same board_size and variant on the
+ * same device (else HEXB_ERR_ARG before any launch; obs_dtype, seed, num_games and game_offset may differ). src_index / dst_index
+ * are device i64[count]; null = the identity 0..count-1. Broadcasting one root into many children is the main use
+ * (src_index = roots.repeat_interleave(C)). The copy is exact: hexb_export_state gives the same regions, region_counter (the
+ * counters themselves, not max(plane) + 1 as hexb_import_labels sets them), cur, done and winner for both games, and the next
+ * hexb_ply on the copy does what the reference's make_move (HexGame.py:85-111, HexSingleGame.py:88-122) does on the copied
+ * simulator. An env game whose agent is WHITE is converted from its agent's orientation into true coordinates. Entries of dst_index
+ * must be distinct and, when dst == src, disjoint from the src games read; otherwise the result is undefined. A pair with an
+ * out-of-range index writes nothing; dst games not named in dst_index are untouched. */
+int32_t hexb_copy_games(hexb_env *dst, const hexb_env *src, const int64_t *src_index, const int64_t *dst_index, int64_t count,
+                        void *stream);
+
+/* Random playouts: playout p of global game g starts from the game's current position with simulator.current_player_num to move,
+ * colours alternating; ply k plays the int(u * n_empty)-th empty cell in true row-major order (random_policy,
+ * minihex/__init__.py:8-12) with u built like every other draw (CPython's random.random() recipe) from Philox4x32-10 at counter
+ * (k, g_lo, g_hi, p + 1) under the handle's seed (c3 = p + 1: the env streams use c3 = 0, so the two never overlap). The playout's
+ * winner is the colour whose edges connect on the filled board (BLACK rows 0 and N-1, WHITE columns 0 and N-1; the reference's
+ * neighbourhood, HexGame.py:124-142); a full Hex board has exactly one. p runs over [first_playout, first_playout + num_playouts):
+ * calls with different first_playout give independent samples. first_playout >= 0, num_playouts >= 1 and
+ * first_playout + num_playouts < 2^32. wins i32[G] = playouts won by the side to move, or -1 for a finished game, a game never
+ * reset and a game with game_mask[i] == 0 (u8[G], null = every game). Any handle: raw, variant A or variant B env. */
+int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout, const uint8_t *game_mask, int32_t *wins,
+                      void *stream);
+
 /* Episode statistics accumulated by hexb_step since creation, int64[8] on the device:
  * [0] episodes finished, [1] BLACK wins, [2] WHITE wins, [3] agent wins, [4] plies of finished episodes,
  * [5] episodes ended by an illegal agent move, [6] env steps, [7] plies. Copies them to out8 (device). The multi-GPU

@@ -10,6 +10,8 @@ torch headers to build.
     env = HexBatch(11, 1 << 20, variant=1, agent_mode=2)
     ops.reset(env.handle, None, None, obs, mask)
     ops.step(env.handle, None, None, obs, mask, reward, done, None, None)
+    ops.copy_games(children.handle, env.handle, roots, None, roots.numel())   # children: a raw HexBatch
+    ops.playouts(children.handle, 64, 0, None, wins)
 
 There is no CPU implementation behind the operators: they raise unless their tensors live on the handle's CUDA device.
 """
