@@ -6,7 +6,8 @@ does not need a GPU; creating a simulator does, and fails loudly without one (no
 """
 from ._native import HexbError, build, lib  # noqa: F401
 from .batch import (AGENT_BLACK, AGENT_RANDOM, AGENT_WHITE, STAT_NAMES, VARIANT_A, VARIANT_B, HexBatch)  # noqa: F401
+from .mcts import MCTS  # noqa: F401
 from .opponents import OpponentPool, StackedMlpOpponents, evaluate_pool  # noqa: F401
 
 __all__ = ["HexBatch", "HexbError", "build", "lib", "VARIANT_A", "VARIANT_B", "AGENT_BLACK", "AGENT_WHITE", "AGENT_RANDOM",
-           "STAT_NAMES", "OpponentPool", "StackedMlpOpponents", "evaluate_pool"]
+           "STAT_NAMES", "MCTS", "OpponentPool", "StackedMlpOpponents", "evaluate_pool"]

@@ -16,7 +16,7 @@ HEADER = os.path.join(_HERE, "include", "hexb.h")                           # th
 ROOT_HEADER = os.path.join(os.path.dirname(_HERE), "include", "hexb.h")      # the repository's canonical include/hexb.h
 BUILD_DIR = os.path.join(_HERE, "build")
 BOARD_SIZES = list(range(3, 20))
-_DEVICE_HEADERS = ["hexb_core.cuh", "hexb_phases.cuh", "hexb_views.cuh", "hexb_search.cuh", "hexb_step.cuh", "hexb_host.h"]
+_DEVICE_HEADERS = ["hexb_core.cuh", "hexb_phases.cuh", "hexb_views.cuh", "hexb_search.cuh", "hexb_mcts.cuh", "hexb_step.cuh", "hexb_host.h"]
 SOURCES = [os.path.join(_CSRC, f) for f in ["hexb_kernels.cu", "hexb_step_inst.cu", "hexb_hostpack.cpp"] + _DEVICE_HEADERS] + [HEADER]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
@@ -164,6 +164,12 @@ SYMBOLS = {
     "hexb_masked_sample": (_i32, [_vp, _vp, _vp, ctypes.c_int64, _i32, _vp, _vp, _vp, _i32, _vp]),
     "hexb_copy_games": (_i32, [_vp, _vp, _vp, _vp, ctypes.c_int64, _vp]),
     "hexb_playouts": (_i32, [_vp, _i32, ctypes.c_int64, _vp, _vp, _vp]),
+    "hexb_mcts_tree_bytes": (_i32, [_vp, _i32, ctypes.POINTER(_sz)]),
+    "hexb_mcts_init": (_i32, [_vp, _vp, _sz, _i32, ctypes.c_double, ctypes.c_double, ctypes.c_int64, _vp, _vp]),
+    "hexb_mcts_search": (_i32, [_vp, _vp, _sz, _i32, _i32, _vp]),
+    "hexb_mcts_select": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp, _vp]),
+    "hexb_mcts_expand": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp]),
+    "hexb_mcts_root": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp]),
 }
 
 _LIB = None

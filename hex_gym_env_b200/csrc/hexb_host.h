@@ -1,14 +1,14 @@
 // hexb_host.h - host-side declarations shared by the translation units of libhexb.so (not part of the C ABI).
 //
 // The library is built from one object per board size (hexb_step_inst.cu compiled with -DHEXB_INST_N=n: every instantiation of
-// the step kernels for that N plus the small per-N kernels: sampler, import, playouts) and hexb_kernels.cu (the C ABI, the size-independent kernels and
+// the step kernels for that N plus the small per-N kernels: sampler, import, playouts, tree search) and hexb_kernels.cu (the C ABI, the size-independent kernels and
 // the dispatch tables). The per-N objects are independent, so hex_gym_env_b200/_native.py compiles them in parallel.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "../include/hexb.h"
-#include "hexb_search.cuh"
+#include "hexb_mcts.cuh"
 
 #define HEXB_LOCAL __attribute__((visibility("hidden")))
 
@@ -40,6 +40,8 @@ HEXB_LOCAL int hexb_cuda_fail(cudaError_t e);   // records the code for hexb_las
         if (e_ != cudaSuccess) return hexb_cuda_fail(e_); \
     } while (0)
 
+enum : int { MCTS_INIT = 0, MCTS_SEARCH, MCTS_SELECT, MCTS_EXPAND, MCTS_ROOT };   // op of hexb_launch_mcts_<n>
+
 // per-board-size entry points, defined by hexb_step_inst.cu
 #define HEXB_FOR_N(X) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19)
 #define HEXB_DECL_N(n)                                                                                                      \
@@ -47,6 +49,7 @@ HEXB_LOCAL int hexb_cuda_fail(cudaError_t e);   // records the code for hexb_las
     HEXB_LOCAL int hexb_launch_sample_##n(const hexb::View &V, int view, const double *u, int32_t *out, cudaStream_t s);     \
     HEXB_LOCAL int hexb_launch_import_##n(const hexb::Params &P, const int8_t *board_true, const int8_t *to_move,           \
                                           const uint8_t *import_mask, cudaStream_t s);                                      \
-    HEXB_LOCAL int hexb_launch_playouts_##n(const hexb::View &V, const hexb::PlayoutArgs &A, cudaStream_t s);
+    HEXB_LOCAL int hexb_launch_playouts_##n(const hexb::View &V, const hexb::PlayoutArgs &A, cudaStream_t s);             \
+    HEXB_LOCAL int hexb_launch_mcts_##n(int op, const hexb::View &V, const hexb::MctsArgs &A, cudaStream_t s);
 HEXB_FOR_N(HEXB_DECL_N)
 #undef HEXB_DECL_N

@@ -15,6 +15,7 @@
 //   K10       hexb_pack_obs_kernel    2-bit observation transport for hexb_step_host_packed
 //   K11       hexb_copy_kernel        copy.deepcopy(env.simulator) into a raw batch, one warp per copied game (hexb_search.cuh)
 //   K12       hexb_playout_kernel<N>  random playouts from the current position, one warp per game (hexb_step_inst.cu)
+//   K13       hexb_mcts_*_kernel<N>   batched PUCT tree search: init, fused search, select, expand, root readout (hexb_mcts.cuh)
 #include <cuda.h>   // types of the driver's virtual-memory API only (entry points come from cudaGetDriverEntryPoint)
 #include <cuda_runtime.h>
 #include <math.h>
@@ -240,6 +241,10 @@ static const sample_fn k_sample[] = {HEXB_FOR_N(X)};
 #undef X
 #define X(n) hexb_launch_import_##n,
 static const import_fn k_import[] = {HEXB_FOR_N(X)};
+#undef X
+typedef int (*mcts_fn)(int, const View &, const MctsArgs &, cudaStream_t);
+#define X(n) hexb_launch_mcts_##n,
+static const mcts_fn k_mcts[] = {HEXB_FOR_N(X)};
 #undef X
 typedef int (*playouts_fn)(const View &, const PlayoutArgs &, cudaStream_t);
 #define X(n) hexb_launch_playouts_##n,
@@ -952,6 +957,92 @@ int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout
     A.game_mask = game_mask;
     A.wins = wins;
     return k_playouts[V.N - HEXB_MIN_BOARD](V, A, (cudaStream_t)stream);
+}
+
+// ---- tree search (hexb_mcts.cuh). The host checks the arguments; the kernels check the tree header init wrote, so that no
+// call on a buffer that holds no tree of this handle writes anything.
+static bool mcts_buffer_ok(const void *tree, size_t tree_bytes) { return tree && tree_bytes >= 128 && ((uintptr_t)tree & 15) == 0; }
+
+static MctsArgs mcts_args(const hexb_env *env, const void *tree, size_t tree_bytes) {
+    MctsArgs A;
+    memset(&A, 0, sizeof(A));
+    A.tree = (uint8_t *)tree;
+    A.tree_bytes = tree_bytes;
+    A.seed = env->base.seed;
+    A.game_offset = (unsigned long long)env->base.game_offset;
+    return A;
+}
+
+static int mcts_launch(const hexb_env *env, int op, const MctsArgs &A, void *stream) {
+    CK(cudaSetDevice(env->cfg.device));
+    const View V = view_of(env);
+    return k_mcts[V.N - HEXB_MIN_BOARD](op, V, A, (cudaStream_t)stream);
+}
+
+int32_t hexb_mcts_tree_bytes(const hexb_env *env, int32_t max_nodes, size_t *bytes) {
+    if (!env || !bytes || max_nodes < 1 || max_nodes > kMctsMaxNodes) return HEXB_ERR_ARG;
+    const unsigned long long root = (unsigned long long)mc_root_bytes(env->cfg.board_size, max_nodes);
+    const unsigned long long G = (unsigned long long)env->base.G;
+    if (root > (SIZE_MAX - 128) / G) return HEXB_ERR_ARG;
+    *bytes = (size_t)(128 + root * G);
+    return HEXB_OK;
+}
+
+int32_t hexb_mcts_init(const hexb_env *env, void *tree, size_t tree_bytes, int32_t max_nodes, double c_puct, double fpu,
+                       int64_t first_playout, const uint8_t *root_mask, void *stream) {
+    size_t need = 0;
+    if (!env || hexb_mcts_tree_bytes(env, max_nodes, &need) != HEXB_OK) return HEXB_ERR_ARG;
+    if (!(c_puct == c_puct) || !(fpu == fpu) || first_playout < 0 || first_playout >= (1ll << 32)) return HEXB_ERR_ARG;
+    if (!mcts_buffer_ok(tree, tree_bytes) || tree_bytes < need) return HEXB_ERR_STATE;
+    MctsArgs A = mcts_args(env, tree, tree_bytes);
+    A.max_nodes = max_nodes;
+    A.c_puct = (float)c_puct;
+    A.fpu = (float)fpu;
+    A.first_playout = first_playout;
+    A.root_mask = root_mask;
+    return mcts_launch(env, MCTS_INIT, A, stream);
+}
+
+int32_t hexb_mcts_search(const hexb_env *env, void *tree, size_t tree_bytes, int32_t num_simulations, int32_t playouts_per_leaf,
+                         void *stream) {
+    if (!env || num_simulations < 1 || playouts_per_leaf < 1 || playouts_per_leaf > kMctsMaxPlayouts) return HEXB_ERR_ARG;
+    if (!mcts_buffer_ok(tree, tree_bytes)) return HEXB_ERR_STATE;
+    MctsArgs A = mcts_args(env, tree, tree_bytes);
+    A.sims = num_simulations;
+    A.playouts = playouts_per_leaf;
+    return mcts_launch(env, MCTS_SEARCH, A, stream);
+}
+
+int32_t hexb_mcts_select(const hexb_env *env, void *tree, size_t tree_bytes, void *leaf_obs, uint8_t *leaf_mask, uint8_t *pending,
+                         void *stream) {
+    if (!env || !leaf_obs || !leaf_mask || !pending) return HEXB_ERR_ARG;
+    if (!mcts_buffer_ok(tree, tree_bytes)) return HEXB_ERR_STATE;
+    MctsArgs A = mcts_args(env, tree, tree_bytes);
+    A.leaf_obs = leaf_obs;
+    A.leaf_mask = leaf_mask;
+    A.pending = pending;
+    return mcts_launch(env, MCTS_SELECT, A, stream);
+}
+
+int32_t hexb_mcts_expand(const hexb_env *env, void *tree, size_t tree_bytes, const float *priors, const float *values, void *stream) {
+    if (!env || !priors || !values) return HEXB_ERR_ARG;
+    if (!mcts_buffer_ok(tree, tree_bytes)) return HEXB_ERR_STATE;
+    MctsArgs A = mcts_args(env, tree, tree_bytes);
+    A.priors = priors;
+    A.values = values;
+    return mcts_launch(env, MCTS_EXPAND, A, stream);
+}
+
+int32_t hexb_mcts_root(const hexb_env *env, const void *tree, size_t tree_bytes, int32_t *visits, float *q, float *value,
+                       int32_t *nodes_used, void *stream) {
+    if (!env) return HEXB_ERR_ARG;
+    if (!mcts_buffer_ok(tree, tree_bytes)) return HEXB_ERR_STATE;
+    MctsArgs A = mcts_args(env, tree, tree_bytes);
+    A.visits = visits;
+    A.q = q;
+    A.value = value;
+    A.nodes_used = nodes_used;
+    return mcts_launch(env, MCTS_ROOT, A, stream);
 }
 
 int32_t hexb_stats(hexb_env *env, int64_t *out8, void *stream) {

@@ -41,6 +41,40 @@ __global__ void __launch_bounds__(256) hexb_playout_kernel(View V, PlayoutArgs A
     if (lane == 0) A.wins[g] = won;
 }
 
+// hexb_mcts_*: the tree search of hexb_mcts.cuh. init: one thread per root (thread 0 also writes the header); the others: one warp
+// per root, all S simulations of the fused search in one launch.
+template <int N>
+__global__ void __launch_bounds__(128) hexb_mcts_init_kernel(View V, MctsArgs A) {
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g == 0) mc_write_header(A, N, V.G);
+    if (g < V.G) mc_init_root<N>(V, A, g);
+}
+// 168 registers: the path rows, the playout's own copy and the selection state without a spill at N = 19 (ptxas -v)
+template <int N>
+__global__ void __maxnreg__(168) hexb_mcts_search_kernel(View V, MctsArgs A) {
+    const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    Tree T;
+    if (g < V.G && mc_tree(A, N, V.G, T)) mc_search_root<N>(T, A, V.variant, g);
+}
+template <int N>
+__global__ void __launch_bounds__(128) hexb_mcts_select_kernel(View V, MctsArgs A) {
+    const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    Tree T;
+    if (g < V.G && mc_tree(A, N, V.G, T)) mc_select_root<N>(T, V, A, g);
+}
+template <int N>
+__global__ void __launch_bounds__(128) hexb_mcts_expand_kernel(View V, MctsArgs A) {
+    const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    Tree T;
+    if (g < V.G && mc_tree(A, N, V.G, T)) mc_expand_root<N>(T, V, A, g);
+}
+template <int N>
+__global__ void __launch_bounds__(128) hexb_mcts_root_kernel(View V, MctsArgs A) {
+    const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    Tree T;
+    if (g < V.G && mc_tree(A, N, V.G, T)) mc_root_out(T, V.variant, A, g);
+}
+
 int HEXB_CAT(hexb_launch_tile_, HEXB_INST_N)(const hexb_env *e, const Params &P, cudaStream_t s) { return launch_tile<HEXB_INST_N>(e, P, s); }
 
 int HEXB_CAT(hexb_launch_sample_, HEXB_INST_N)(const View &V, int view, const double *u, int32_t *out, cudaStream_t s) {
@@ -58,6 +92,20 @@ int HEXB_CAT(hexb_launch_import_, HEXB_INST_N)(const Params &P, const int8_t *bo
 
 int HEXB_CAT(hexb_launch_playouts_, HEXB_INST_N)(const View &V, const PlayoutArgs &A, cudaStream_t s) {
     hexb_playout_kernel<HEXB_INST_N><<<(unsigned)((V.G + 7) / 8), 256, 0, s>>>(V, A);
+    CK(cudaGetLastError());
+    return HEXB_OK;
+}
+
+int HEXB_CAT(hexb_launch_mcts_, HEXB_INST_N)(int op, const View &V, const MctsArgs &A, cudaStream_t s) {
+    const unsigned warps = (unsigned)((V.G + 3) / 4), threads = (unsigned)((V.G + 127) / 128);
+    switch (op) {
+        case MCTS_INIT: hexb_mcts_init_kernel<HEXB_INST_N><<<threads, 128, 0, s>>>(V, A); break;
+        case MCTS_SEARCH: hexb_mcts_search_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
+        case MCTS_SELECT: hexb_mcts_select_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
+        case MCTS_EXPAND: hexb_mcts_expand_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
+        case MCTS_ROOT: hexb_mcts_root_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
+        default: return HEXB_ERR_ARG;
+    }
     CK(cudaGetLastError());
     return HEXB_OK;
 }

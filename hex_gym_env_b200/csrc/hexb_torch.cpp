@@ -182,6 +182,57 @@ void op_playouts(int64_t handle, int64_t num_playouts, int64_t first_playout, Op
              "playouts");
 }
 
+// tree search (hexb_mcts_*): the tree is a uint8 tensor of at least hexb_mcts_tree_bytes bytes on the handle's device
+void *tree_of(const Tensor &tree, int device) {
+    TORCH_CHECK(tree.is_cuda() && tree.get_device() == device && tree.scalar_type() == at::kByte && tree.is_contiguous(),
+                "hexb: tree must be a contiguous uint8 tensor on cuda:", device);
+    return tree.data_ptr();
+}
+
+void op_mcts_init(int64_t handle, Tensor tree, int64_t max_nodes, double c_puct, double fpu, int64_t first_playout, OptT root_mask) {
+    Call k(handle);
+    const int d = k.c.device;
+    TORCH_CHECK(max_nodes >= 1 && max_nodes <= INT32_MAX, "hexb::mcts_init: max_nodes out of range");
+    check_rc(hexb_mcts_init(k.e, tree_of(tree, d), (size_t)tree.numel(), (int32_t)max_nodes, c_puct, fpu, first_playout,
+                            ptr<const uint8_t>(root_mask, at::kByte, k.G, d, "root_mask"), k.stream),
+             "mcts_init");
+}
+
+void op_mcts_search(int64_t handle, Tensor tree, int64_t num_simulations, int64_t playouts_per_leaf) {
+    Call k(handle);
+    TORCH_CHECK(num_simulations >= 1 && num_simulations <= INT32_MAX && playouts_per_leaf >= 1 && playouts_per_leaf <= INT32_MAX,
+                "hexb::mcts_search: num_simulations and playouts_per_leaf must be >= 1");
+    check_rc(hexb_mcts_search(k.e, tree_of(tree, k.c.device), (size_t)tree.numel(), (int32_t)num_simulations, (int32_t)playouts_per_leaf,
+                              k.stream),
+             "mcts_search");
+}
+
+void op_mcts_select(int64_t handle, Tensor tree, Tensor leaf_obs, Tensor leaf_mask, Tensor pending) {
+    Call k(handle);
+    const int d = k.c.device;
+    check_rc(hexb_mcts_select(k.e, tree_of(tree, d), (size_t)tree.numel(), ptr<void>(leaf_obs, k.obs_t(), k.G * k.C, d, "leaf_obs"),
+                              ptr<uint8_t>(leaf_mask, at::kByte, k.G * k.C, d, "leaf_mask"), ptr<uint8_t>(pending, at::kByte, k.G, d, "pending"),
+                              k.stream),
+             "mcts_select");
+}
+
+void op_mcts_expand(int64_t handle, Tensor tree, Tensor priors, Tensor values) {
+    Call k(handle);
+    const int d = k.c.device;
+    check_rc(hexb_mcts_expand(k.e, tree_of(tree, d), (size_t)tree.numel(), ptr<const float>(priors, at::kFloat, k.G * k.C, d, "priors"),
+                              ptr<const float>(values, at::kFloat, k.G, d, "values"), k.stream),
+             "mcts_expand");
+}
+
+void op_mcts_root(int64_t handle, Tensor tree, OptT visits, OptT q, OptT value, OptT nodes_used) {
+    Call k(handle);
+    const int d = k.c.device;
+    check_rc(hexb_mcts_root(k.e, tree_of(tree, d), (size_t)tree.numel(), ptr<int32_t>(visits, at::kInt, k.G * k.C, d, "visits"),
+                            ptr<float>(q, at::kFloat, k.G * k.C, d, "q"), ptr<float>(value, at::kFloat, k.G, d, "value"),
+                            ptr<int32_t>(nodes_used, at::kInt, k.G, d, "nodes_used"), k.stream),
+             "mcts_root");
+}
+
 int64_t op_version() { return hexb_version(); }
 
 }  // namespace
@@ -204,6 +255,11 @@ TORCH_LIBRARY(hexb, m) {
     m.def("set_eval(int env, bool eval_state, Tensor(a!)? eval_episode) -> ()");
     m.def("copy_games(int dst, int src, Tensor? src_index, Tensor? dst_index, int count) -> ()");
     m.def("playouts(int env, int num_playouts, int first_playout, Tensor? game_mask, Tensor(a!) wins) -> ()");
+    m.def("mcts_init(int env, Tensor(a!) tree, int max_nodes, float c_puct, float fpu, int first_playout, Tensor? root_mask) -> ()");
+    m.def("mcts_search(int env, Tensor(a!) tree, int num_simulations, int playouts_per_leaf) -> ()");
+    m.def("mcts_select(int env, Tensor(a!) tree, Tensor(b!) leaf_obs, Tensor(c!) leaf_mask, Tensor(d!) pending) -> ()");
+    m.def("mcts_expand(int env, Tensor(a!) tree, Tensor priors, Tensor values) -> ()");
+    m.def("mcts_root(int env, Tensor tree, Tensor(a!)? visits, Tensor(b!)? q, Tensor(c!)? value, Tensor(d!)? nodes_used) -> ()");
 }
 
 // The handle is an int, so these operators have no tensor argument to dispatch on when every optional is None: register them
@@ -222,4 +278,9 @@ TORCH_LIBRARY_IMPL(hexb, CompositeExplicitAutograd, m) {
     m.impl("set_eval", &op_set_eval);
     m.impl("copy_games", &op_copy_games);
     m.impl("playouts", &op_playouts);
+    m.impl("mcts_init", &op_mcts_init);
+    m.impl("mcts_search", &op_mcts_search);
+    m.impl("mcts_select", &op_mcts_select);
+    m.impl("mcts_expand", &op_mcts_expand);
+    m.impl("mcts_root", &op_mcts_root);
 }

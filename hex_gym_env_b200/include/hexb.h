@@ -251,6 +251,59 @@ int32_t hexb_copy_games(hexb_env *dst, const hexb_env *src, const int64_t *src_i
 int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout, const uint8_t *game_mask, int32_t *wins,
                       void *stream);
 
+/* Batched Monte-Carlo tree search (PUCT), one tree per game g of `env` (any handle: raw, variant A or B env), in a device buffer
+ * of hexb_mcts_tree_bytes(env, max_nodes) bytes (16-byte aligned; layout: csrc/hexb_mcts.cuh). Every call is asynchronous on
+ * `stream`, allocates nothing and reads nothing on the host (CUDA-graph capturable). Bad max_nodes (1..2^24), num_simulations
+ * (>= 1), playouts_per_leaf (1..65536), c_puct / fpu (NaN) or first_playout (0..2^32-1): HEXB_ERR_ARG; a null or misaligned
+ * tree, or one smaller than hexb_mcts_tree_bytes: HEXB_ERR_STATE. A buffer that holds no tree of this handle (init never ran on
+ * it, other board size or game count) is left alone by search / select / expand / root.
+ *
+ * init: each root's current position is read in true orientation. A root is inactive (nothing is ever done for it) if its game
+ *   is finished, was never reset or has root_mask[g] == 0 (u8[G], null = all); an active root gets node 0, unexpanded, and
+ *   s = 0 simulations. c_puct, fpu (as float32) and first_playout are kept in the tree.
+ * Nodes are numbered in creation order, at most max_nodes per root; a node's side to move is the root's, alternating with depth.
+ *   An expanded node has one edge per cell: child (-1 none), N (i32), W, P (f32); every node has Nn (simulations whose path
+ *   contained it) and a terminal flag.
+ * One simulation:
+ *   1 select: from node 0, at an expanded non-terminal node take the empty cell with the largest Q + U, Q = W / N if N > 0 else
+ *     fpu, U = c_puct * P * sqrt(Nn) / (1 + N), in float32 with every operation rounded once (no FMA; exactly
+ *     ((c_puct * P) * sqrt(Nn)) / (1 + N), then Q + U), ties to the lowest true row-major cell. An expanded child: descend; a
+ *     terminal child is the leaf; no child: the new position is the leaf. Node 0 before its first simulation, and a node with no
+ *     empty cell, is itself the leaf.
+ *   2 value v for the leaf's side to move: if the move into a new leaf connects the mover's edges the leaf is terminal and
+ *     v = -1 (so is a terminal child's). Otherwise, in hexb_mcts_search, P playouts exactly as hexb_playouts with playout index
+ *     p = first_playout + s * P + j (mod 2^32) of the root's global game index, v = (2 * wins - P) / P, priors 1 / n_empty on
+ *     the empty cells; in the split form v and the priors come from hexb_mcts_expand (cells not empty are ignored, nothing is
+ *     renormalised).
+ *   3 store: if fewer than max_nodes nodes exist, a new leaf becomes a node (expanded with the priors: children -1, N = W = 0;
+ *     or terminal); node 0 is expanded in place. A full pool stores nothing; the value is still backed up.
+ *   4 back up: Nn += 1 on every node of the path (leaf included: a new node starts at 1); every edge of the path gets N += 1 and
+ *     W += the value for the player who made that move (-v into the leaf, sign alternating upwards); the root sums v as seen by
+ *     its side to move; s += 1.
+ * Per-cell arrays (visits, q, priors, leaf_obs, leaf_mask) use hexb_ply's action convention of a raw handle of the same variant
+ * for the side to move at that node: variant A true cells, variant B the mover's view (transposed for WHITE). For an env root at
+ * the agent's turn that is the agent's action space. */
+int32_t hexb_mcts_tree_bytes(const hexb_env *env, int32_t max_nodes, size_t *bytes);
+int32_t hexb_mcts_init(const hexb_env *env, void *tree, size_t tree_bytes, int32_t max_nodes, double c_puct, double fpu,
+                       int64_t first_playout, const uint8_t *root_mask, void *stream);
+/* The fused form: num_simulations simulations with playout evaluation for every active root, in one launch. search(a) followed
+ * by search(b) equals search(a + b). */
+int32_t hexb_mcts_search(const hexb_env *env, void *tree, size_t tree_bytes, int32_t num_simulations, int32_t playouts_per_leaf,
+                         void *stream);
+/* The split form, one simulation per select / expand pair (results are defined only when they alternate). select: step 1 for
+ * every active root. A leaf that needs an evaluation gets leaf_obs[g] (obs_dtype [G,N,N]) and leaf_mask[g] (u8 [G,C]) - what
+ * hexb_encode(view 1) returns for a raw game of the same variant holding the leaf - and pending[g] = 1 (u8 [G]); a terminal
+ * leaf is backed up at once and, like an inactive root, gets pending[g] = 0 and no leaf row. expand: steps 2-4 for the pending
+ * roots with priors f32[G,C] and values f32[G] (rows of the others are ignored). Root Dirichlet noise is the caller's: add it
+ * to the priors of the first expand, whose leaf is the root. */
+int32_t hexb_mcts_select(const hexb_env *env, void *tree, size_t tree_bytes, void *leaf_obs, uint8_t *leaf_mask, uint8_t *pending,
+                         void *stream);
+int32_t hexb_mcts_expand(const hexb_env *env, void *tree, size_t tree_bytes, const float *priors, const float *values, void *stream);
+/* The root's edges: visits i32[G,C], q f32[G,C] (W / N, 0 where N = 0), value f32[G] (the root's value sum / its Nn, 0 before
+ * the first simulation), nodes_used i32[G] (0 = inactive root). Every output is nullable. */
+int32_t hexb_mcts_root(const hexb_env *env, const void *tree, size_t tree_bytes, int32_t *visits, float *q, float *value,
+                       int32_t *nodes_used, void *stream);
+
 /* Episode statistics accumulated by hexb_step since creation, int64[8] on the device:
  * [0] episodes finished, [1] BLACK wins, [2] WHITE wins, [3] agent wins, [4] plies of finished episodes,
  * [5] episodes ended by an illegal agent move, [6] env steps, [7] plies. Copies them to out8 (device). The multi-GPU

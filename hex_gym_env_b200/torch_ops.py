@@ -12,6 +12,8 @@ torch headers to build.
     ops.step(env.handle, None, None, obs, mask, reward, done, None, None)
     ops.copy_games(children.handle, env.handle, roots, None, roots.numel())   # children: a raw HexBatch
     ops.playouts(children.handle, 64, 0, None, wins)
+    ops.mcts_init(env.handle, tree, 801, 1.25, 0.0, 0, None)                    # tree: uint8[hexb_mcts_tree_bytes] (mcts.MCTS)
+    ops.mcts_search(env.handle, tree, 800, 8)
 
 There is no CPU implementation behind the operators: they raise unless their tensors live on the handle's CUDA device.
 """
