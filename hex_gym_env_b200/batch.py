@@ -31,6 +31,7 @@ VARIANT_B = 1  # minihex/HexSingleGame.py + minihex/SelfplayWrapper.py
 AGENT_BLACK, AGENT_WHITE, AGENT_RANDOM = 0, 1, 2
 
 STAT_NAMES = ("episodes", "black_wins", "white_wins", "agent_wins", "episode_plies", "invalid_ends", "env_steps", "plies")
+COMPRESSIBLE_MIN_BYTES = 8 << 20   # smaller buffers stay with torch's allocator even when the object uses compressible memory
 
 
 def _ptr(t):
@@ -73,12 +74,8 @@ class HexBatch(object):
             compressible = (env_c != "0") if env_c is not None else self.state_bytes >= (64 << 20)
         self.compressible = bool(compressible)
         self.memory_kind = "ordinary (torch allocator)"
-        parts = os.environ.get("HEXB_COMPRESSIBLE_PARTS", "state,outputs")   # experiments: which buffers ("state", "outputs")
-        self._comp_state, self._comp_out = "state" in parts, "outputs" in parts
-        self._comp_min = int(float(os.environ.get("HEXB_COMPRESSIBLE_MIN_MB", "8")) * (1 << 20))   # smaller buffers stay with torch
         with torch.cuda.device(self.device):
-            self._state = self._alloc(self.state_bytes + 256) if self._comp_state else \
-                torch.empty(self.state_bytes + 256, dtype=torch.uint8, device=self.device)
+            self._state = self._alloc(self.state_bytes + 256)
             off = (-self._state.data_ptr()) % 256
             self._state_ptr = self._state.data_ptr() + off
             h = ctypes.c_void_p()
@@ -119,7 +116,7 @@ class HexBatch(object):
 
     def _alloc(self, nbytes):
         """uint8[nbytes] on the device: compressible memory from the library for large buffers when enabled, else torch's allocator."""
-        if self.compressible and nbytes >= self._comp_min:
+        if self.compressible and nbytes >= COMPRESSIBLE_MIN_BYTES:
             try:
                 buf = _native.DeviceBuffer(nbytes, self.device.index, True)
                 self.memory_kind = "compressible (cuMemCreate, CU_MEM_ALLOCATION_COMP_GENERIC)" if buf.compressed else \
@@ -137,7 +134,7 @@ class HexBatch(object):
             for d in shape:
                 n *= int(d)
             nbytes = n * torch.empty((), dtype=dtype).element_size()
-            if self.compressible and self._comp_out and nbytes >= self._comp_min:
+            if self.compressible and nbytes >= COMPRESSIBLE_MIN_BYTES:
                 t = self._alloc(nbytes)[:nbytes].view(dtype).reshape(shape)
             else:
                 t = torch.empty(shape, dtype=dtype, device=self.device)
@@ -269,7 +266,7 @@ class HexBatch(object):
         return self._pinned
 
     def set_launch_form(self, warps_per_chunk=0):
-        """0: the kernel form is chosen by launch depth; 1 / 2 / 4 / 8: that many warps per 32-game chunk (tuning, tests)."""
+        """0: the kernel form is chosen by launch depth; 1 / 4: that many warps per 32-game chunk (tests). Other values raise HexbError."""
         check(self._lib.hexb_set_launch_form(self._h, int(warps_per_chunk)))
 
     def set_host_transport(self, dma_fraction=-1.0):

@@ -1,7 +1,7 @@
 // hexb_host.h - host-side declarations shared by the translation units of libhexb.so (not part of the C ABI).
 //
 // The library is built from one object per board size (hexb_step_inst.cu compiled with -DHEXB_INST_N=n: every instantiation of
-// the step kernels for that N plus the small per-N kernels: sampler, import, playouts, tree search) and hexb_kernels.cu (the C ABI, the size-independent kernels and
+// the step kernels for that N (one warp or a CTA of 4 warps per chunk) plus the small per-N kernels: sampler, import, playouts, tree search) and hexb_kernels.cu (the C ABI, the size-independent kernels and
 // the dispatch tables). The per-N objects are independent, so hex_gym_env_b200/_native.py compiles them in parallel.
 #pragma once
 #include <cuda_runtime.h>
@@ -17,7 +17,7 @@
 struct hexb_env {
     hexb_config cfg;
     hexb::Params base;   // state pointers + config, I/O pointers null
-    int launch_form;     // hexb_set_launch_form: 0 = chosen by launch depth, 1 / 2 / 4 / 8 = warps per 32-game chunk
+    int launch_form;     // hexb_set_launch_form: 0 = chosen by launch depth, 1 / 4 = warps per 32-game chunk
     // ---- host-buffer step (hexb_step_host*): events, staging and the adaptive DMA / packed split
     cudaEvent_t host_ev, host_ev_dma0, host_ev_slice[HEXB_HOST_SLICES];   // all copies done; start of the DMA part; each packed slice arrived
     int host_pending, host_adapt, host_frac_fixed;

@@ -5,7 +5,7 @@
 //
 // Kernel inventory (SURVEY.md section 2.3):
 //   K1/K2/K3  hexb_step_kernel<N> / hexb_coop_kernel<N>  (hexb_step.cuh) MODE_RESET / MODE_STEP / MODE_PLY / MODE_HALF, T steps
-//             per launch for hexb_rollout; one warp per 32-game chunk, or a CTA of 2 / 4 / 8 warps per chunk for sub-wave launches
+//             per launch for hexb_rollout; one warp per 32-game chunk, or a CTA of 4 warps per chunk for sub-wave launches
 //   K4        hexb_sample_kernel<N>   standalone k-th-empty-cell sampler (hexb_step_inst.cu)
 //   K5        hexb_encode_kernel      standalone observation + mask encoder (either view)
 //   K6        hexb_export_kernel / hexb_import_kernel<N>   reference-layout dump / preset boards
@@ -330,13 +330,9 @@ int32_t hexb_create(const hexb_config *cfg, void *state, size_t state_bytes, voi
         // 20 MiB of it there across steps and stream the rest. Measured on 11x11: 1 Mi games 99.4 -> 93.0 us per step,
         // 768 Ki 76.2 -> 70.6, 2 Mi 191.2 -> 182.7; 16-24 MiB is the optimum (32: 94.1, 48: 97.2, everything: 99.6 us - the L2
         // holds only so many evict_last lines before they thrash among themselves); below ~64 MiB of state it does not pay.
-        // HEXB_L2_KEEP_MB overrides the amount (0 = never).
         const long long cb = chunk_state_bytes(cfg->board_size * cfg->board_size);
         const long long state = L.Gpad / 32 * cb;
-        long long keep_bytes = state > (64ll << 20) ? (20ll << 20) : 0;
-        const char *kmb = getenv("HEXB_L2_KEEP_MB");
-        if (kmb) keep_bytes = atoll(kmb) * (1ll << 20);
-        P.keep_chunks = keep_bytes > 0 ? keep_bytes / cb : 0;
+        P.keep_chunks = state > (64ll << 20) ? (20ll << 20) / cb : 0;
         enc_consts(P.variant, P.enc_ka, P.enc_kb, P.enc_kc);
     }
     {   // host-buffer step: adaptive DMA / packed split unless HEXB_HOST_DMA_FRACTION pins it (1 = plain DMA only)
@@ -347,11 +343,6 @@ int32_t hexb_create(const hexb_config *cfg, void *state, size_t state_bytes, voi
             if (f >= 0.0 && f <= 1.0) { e->host_dma_frac = f; e->host_frac_fixed = 1; }
         }
         if (hexb_hostpack_threads() < 1) { e->host_dma_frac = 1.0; e->host_frac_fixed = 1; }
-    }
-    {
-        const char *lf = getenv("HEXB_LAUNCH_FORM");   // experiments: the same override as hexb_set_launch_form, for every handle
-        const int f = lf ? atoi(lf) : 0;
-        e->launch_form = (f == 1 || f == 2 || f == 4 || f == 8) ? f : 0;
     }
     *out = e;
     return HEXB_OK;
@@ -377,8 +368,7 @@ int32_t hexb_get_config(const hexb_env *env, hexb_config *out) {
 }
 
 int32_t hexb_set_launch_form(hexb_env *env, int32_t warps_per_chunk) {
-    if (!env || !(warps_per_chunk == 0 || warps_per_chunk == 1 || warps_per_chunk == 2 || warps_per_chunk == 4 || warps_per_chunk == 8))
-        return HEXB_ERR_ARG;
+    if (!env || !(warps_per_chunk == 0 || warps_per_chunk == 1 || warps_per_chunk == 4)) return HEXB_ERR_ARG;
     env->launch_form = warps_per_chunk;
     return HEXB_OK;
 }

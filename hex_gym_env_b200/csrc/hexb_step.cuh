@@ -3,17 +3,11 @@
 //
 //   hexb_step_kernel<N, KIND, BATCHED>   one warp per chunk of 32 games; BATCHED picks the relabel sweep (several rows per pass
 //                                        for launches of at most one wave, one row per pass for deep, HBM-bound launches)
-//   hexb_coop_kernel<N, KIND, WPC>       one CTA of WPC warps per chunk, for sub-wave launches (latency-bound)
+//   hexb_coop_kernel<N, KIND>            one CTA of 4 warps per chunk, for sub-wave launches (latency-bound)
 #pragma once
-#include <stdlib.h>
-
 #include "hexb_host.h"
 
 using namespace hexb;
-
-#ifndef HEXB_PDL_EARLY
-#define HEXB_PDL_EARLY 1
-#endif
 
 // ------------------------------------------------------------------------------------------------ PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -74,16 +68,13 @@ __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.w
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // ------------------------------------------------------------------------------------------------ step kernel
-// One warp = one chunk of 32 games; a CTA is HEXB_WARPS_PER_CTA independent warps (default 1; no __syncthreads anywhere). Per warp:
+// One warp = one chunk of 32 games; a CTA is kWarpsPerCta independent warps (no __syncthreads anywhere). Per warp:
 //   lane 0 starts ONE bulk asynchronous copy (cp.async.bulk = the 1-D TMA path, completion on the warp's own mbarrier)
 //   of the chunk (32 games' label bytes + record words, one contiguous block) into shared memory; meanwhile every lane
 //   fetches its game's meta / stream-position words and runs the Philox rounds of the step's two draws; then the
 //   thread-per-game plies, the rare finished-game rows, the elementwise obs/mask encode with 16-byte coalesced stores, the
 //   warp-per-game relabel sweeps, and one bulk copy of the chunk back to global memory.
-#ifndef HEXB_WARPS_PER_CTA
-#define HEXB_WARPS_PER_CTA 1   // measured (r1h): 1 warp per CTA 90.0 us, 2: 94.0 us, 4: 94.7 us per 1 Mi-game step (finer-grained tail)
-#endif
-constexpr int kWarpsPerCta = HEXB_WARPS_PER_CTA;   // Gpad is a multiple of kTile = 128 games, so 1, 2 and 4 all divide it
+constexpr int kWarpsPerCta = 1;   // measured (r1h): 1 warp per CTA 90.0 us, 2: 94.0 us, 4: 94.7 us per 1 Mi-game step (finer-grained tail)
 constexpr int kCtaThreads = kWarpsPerCta * kWarp;
 // resident CTAs per SM the register allocation should allow (the hardware holds at most 32 CTAs per SM, i.e. 32 warps with one
 // warp per CTA; the step kernel uses 56 registers, so registers are not the limit), for large boards whatever the shared-memory
@@ -408,11 +399,9 @@ __global__ void __launch_bounds__(kCtaThreads, min_ctas(N)) hexb_step_kernel(con
 
     // ---- chunk out. The next grid on the stream (the next env step) may start launching now: it still waits at its
     //      griddepcontrol.wait for this whole grid to complete and flush, but its CTAs are dispatched and set up while this grid's
-    //      chunks drain to global memory: about 1 % on every batch size measured (profiles/r2n_pdl_ab.jsonl; HEXB_PDL_EARLY=0
-    //      compiles the trigger out). Triggering at the TOP of the kernel was measured and rejected in round 1.
-#if HEXB_PDL_EARLY
+    //      chunks drain to global memory: about 1 % on every batch size measured (profiles/r2n_pdl_ab.jsonl). Triggering at the
+    //      TOP of the kernel was measured and rejected in round 1.
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
     fence_async_smem();  // generic-proxy writes to shared memory -> visible to the async proxy
     __syncwarp();
     if (lane == 0) {
@@ -424,7 +413,8 @@ __global__ void __launch_bounds__(kCtaThreads, min_ctas(N)) hexb_step_kernel(con
 
 // ------------------------------------------------------------------------------------------------ cooperative form (sub-wave launches)
 // When a launch holds at most about one wave of warps, a step costs one warp's dependent instruction chain (about 2,300
-// instructions at 11x11), not bandwidth. This form gives a 32-game chunk to a CTA of WPC warps instead of one warp:
+// instructions at 11x11), not bandwidth. This form gives a 32-game chunk to a CTA of WPC = 4 warps instead of one warp (2 and 8
+// warps per chunk were measured too and never won, profiles/r2b_forms.jsonl):
 //   thread-per-game phase   warp w plays games [w*32/WPC, (w+1)*32/WPC) on its first 32/WPC lanes (the chain of ONE game is what
 //                           it is, but a warp now runs the union of the branches of 32/WPC games instead of 32: the restart path
 //                           with its extra Philox draws is taken by far fewer warps per step)
@@ -433,7 +423,8 @@ __global__ void __launch_bounds__(kCtaThreads, min_ctas(N)) hexb_step_kernel(con
 // with one __syncthreads between phases (requests and flags go through shared memory instead of shuffles). Rows that share an
 // edge word (odd N) are never swept in the same pass: passes are split by row parity, as in the batched warp form.
 // Results are bit-identical to the warp form (rows are independent, the encode is elementwise).
-template <int N, int WPC>
+constexpr int WPC = 4;   // warps per chunk of the cooperative form
+template <int N>
 struct CoopSmem {
     static constexpr int CHUNK = Geo<N>::CHUNK_STATE;        // multiple of 16
     static constexpr int BAR = CHUNK;                         // one mbarrier (8 bytes), padded to 16
@@ -444,12 +435,11 @@ struct CoopSmem {
     static constexpr int BYTES = STATS + 64;
 };
 
-template <int N, int KIND, int WPC>
+template <int N, int KIND>
 __global__ void __launch_bounds__(WPC * 32) hexb_coop_kernel(const Params P) {
     static_assert(KIND == KIND_STEP || KIND == KIND_ROLLOUT, "the cooperative form exists for the env step only");
-    static_assert(WPC == 2 || WPC == 4 || WPC == 8, "warps per chunk");
     extern __shared__ __align__(128) uint8_t smem[];
-    using SL = CoopSmem<N, WPC>;
+    using SL = CoopSmem<N>;
     using SW = Sweep<N>;
     constexpr int C = Geo<N>::C;
     constexpr int GPW = kWarp / WPC;          // games per warp
@@ -621,7 +611,7 @@ static long long wave_warps(int device) {
     return v;
 }
 
-// Warps per chunk for a launch of `chunks` chunks (hexb_set_launch_form overrides). Measured on B200 (profiles/r2b_forms.jsonl,
+// Warps per chunk (1 or WPC) for a launch of `chunks` chunks (hexb_set_launch_form overrides). Measured on B200 (profiles/r2b_forms.jsonl,
 // CUDA-graph step time, 1 / 2 / 4 / 8 warps per chunk): 4,096 games of 6x6 6.16 / 6.16 / 5.88 / 5.93 us; 16,384 games of 7x7
 // 6.20 / 6.46 / 6.84 / 9.61; 65,536 games of 7x7 8.12 / 11.2 / 16.1 / 26.0; 131,072 games of 11x11 15.8 / 23.8 / 34.7 / 55.5.
 // The cooperative form only shortens the row sweeps and the encode (about a fifth of one warp's chain, profiles/r2b_*): the
@@ -629,7 +619,7 @@ static long long wave_warps(int device) {
 // slots as soon as an SM holds more than a few chunks. So it is chosen only while there is at most one chunk per SM.
 static int auto_form(long long chunks, int device) {
     const long long sms = wave_warps(device) / 32;
-    return chunks <= sms ? 4 : 1;
+    return chunks <= sms ? WPC : 1;
 }
 
 template <int N>
@@ -646,12 +636,8 @@ static int set_attrs_once(int dev) {
     HEXB_ATTR((hexb_step_kernel<N, KIND_ROLLOUT, false>), smem)
     HEXB_ATTR((hexb_step_kernel<N, KIND_ROLLOUT, true>), smem)
     HEXB_ATTR((hexb_step_kernel<N, KIND_OTHER, false>), smem)
-    HEXB_ATTR((hexb_coop_kernel<N, KIND_STEP, 2>), (CoopSmem<N, 2>::BYTES))
-    HEXB_ATTR((hexb_coop_kernel<N, KIND_STEP, 4>), (CoopSmem<N, 4>::BYTES))
-    HEXB_ATTR((hexb_coop_kernel<N, KIND_STEP, 8>), (CoopSmem<N, 8>::BYTES))
-    HEXB_ATTR((hexb_coop_kernel<N, KIND_ROLLOUT, 2>), (CoopSmem<N, 2>::BYTES))
-    HEXB_ATTR((hexb_coop_kernel<N, KIND_ROLLOUT, 4>), (CoopSmem<N, 4>::BYTES))
-    HEXB_ATTR((hexb_coop_kernel<N, KIND_ROLLOUT, 8>), (CoopSmem<N, 8>::BYTES))
+    HEXB_ATTR((hexb_coop_kernel<N, KIND_STEP>), CoopSmem<N>::BYTES)
+    HEXB_ATTR((hexb_coop_kernel<N, KIND_ROLLOUT>), CoopSmem<N>::BYTES)
 #undef HEXB_ATTR
     if (dev >= 0 && dev < 64) __atomic_store_n(&done[dev], 1, __ATOMIC_RELEASE);   // setting the attributes twice is harmless
     return HEXB_OK;
@@ -666,35 +652,25 @@ static int launch_tile(const hexb_env *e, const Params &P, cudaStream_t s) {
     cudaLaunchAttribute la[1];
     la[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     la[0].val.programmaticStreamSerializationAllowed = 1;
-    static const bool pdl = !(getenv("HEXB_PDL") && atoi(getenv("HEXB_PDL")) == 0);   // HEXB_PDL=0: plain stream-ordered launches
     lc.attrs = la;
-    lc.numAttrs = pdl ? 1 : 0;
+    lc.numAttrs = 1;
     const long long chunks = P.Gpad / kWarp;
     // The record-only half of the step before the chunk has landed (Params::early): while a launch is at most one wave of warps
     // every warp waits for its bulk copy at the same time, and the copy of a whole wave's chunks takes longer than the Philox
     // rounds that used to cover it. Measured on one box (profiles/r2p_early_ab.jsonl, us per step off / on): 11x11 32,768 games
     // 8.01 / 7.88, 65,536 10.29 / 10.14, 131,072 15.43 / 15.14; 7x7 65,536 8.23 / 8.11, 131,072 12.49 / 12.35; 19x19 65,536
     // 17.1 / 16.9; no change at 4,096 games; 1 Mi games of 11x11 99.7 / 101.3 (deep launches hide the wait behind other warps and
-    // pay for the second fetch of the record words), hence by launch depth. HEXB_EARLY=0 / 1 forces it (experiments).
-    static const int force_early = getenv("HEXB_EARLY") ? atoi(getenv("HEXB_EARLY")) : -1;
+    // pay for the second fetch of the record words), hence by launch depth.
     Params Q = P;
-    Q.early = (force_early >= 0 ? force_early != 0 : chunks <= wave_warps(e->cfg.device)) ? 1 : 0;
+    Q.early = chunks <= wave_warps(e->cfg.device) ? 1 : 0;
     int form = 1;
     if (P.mode == MODE_STEP) form = e->launch_form ? e->launch_form : auto_form(chunks, e->cfg.device);
-    if (form > 1) {   // cooperative form: one CTA of `form` warps per chunk
+    if (form == WPC) {   // cooperative form: one CTA of WPC warps per chunk
         lc.gridDim = dim3((unsigned)chunks);
-        lc.blockDim = dim3(form * kWarp);
-#define HEXB_COOP(K, W)                                                       \
-    {                                                                         \
-        lc.dynamicSmemBytes = CoopSmem<N, W>::BYTES;                          \
-        CK(cudaLaunchKernelEx(&lc, hexb_coop_kernel<N, K, W>, Q));            \
-    }
-        if (P.steps == 1) {
-            if (form == 2) HEXB_COOP(KIND_STEP, 2) else if (form == 4) HEXB_COOP(KIND_STEP, 4) else HEXB_COOP(KIND_STEP, 8)
-        } else {
-            if (form == 2) HEXB_COOP(KIND_ROLLOUT, 2) else if (form == 4) HEXB_COOP(KIND_ROLLOUT, 4) else HEXB_COOP(KIND_ROLLOUT, 8)
-        }
-#undef HEXB_COOP
+        lc.blockDim = dim3(WPC * kWarp);
+        lc.dynamicSmemBytes = CoopSmem<N>::BYTES;
+        if (P.steps == 1) CK(cudaLaunchKernelEx(&lc, hexb_coop_kernel<N, KIND_STEP>, Q));
+        else CK(cudaLaunchKernelEx(&lc, hexb_coop_kernel<N, KIND_ROLLOUT>, Q));
         CK(cudaGetLastError());
         return HEXB_OK;
     }
@@ -706,9 +682,8 @@ static int launch_tile(const hexb_env *e, const Params &P, cudaStream_t s) {
     // (profiles/r2i_sweep_ab.jsonl, us per step batched / one-row): 11x11 32,768 games 7.79 / 8.12, 65,536 10.25 / 10.11, 131,072
     // 15.69 / 15.11, 1 Mi 106.4 / 94.9; 7x7 65,536 8.04 / 8.34, 131,072 12.13 / 12.14; 19x19 65,536 17.47 / 17.14. Short rows
     // (small boards) leave most lanes of a one-row pass idle, so the cross-over comes later there.
-    static const int force_sweep = getenv("HEXB_SWEEP_BATCHED") ? atoi(getenv("HEXB_SWEEP_BATCHED")) : -1;   // experiments: 0 / 1
     const long long sms = wave_warps(e->cfg.device) / 32;
-    const bool small = force_sweep >= 0 ? force_sweep != 0 : chunks <= sms * (N <= 8 ? 28 : 12);
+    const bool small = chunks <= sms * (N <= 8 ? 28 : 12);
     if (P.mode == MODE_STEP && P.steps == 1) {
         if (small) CK(cudaLaunchKernelEx(&lc, hexb_step_kernel<N, KIND_STEP, true>, Q));
         else CK(cudaLaunchKernelEx(&lc, hexb_step_kernel<N, KIND_STEP, false>, Q));

@@ -1,4 +1,5 @@
-// hexb_step_inst.cu - everything of libhexb.so that is templated on the board size, for ONE size: compiled once per
+// hexb_step_inst.cu - everything of libhexb.so that is templated on the board size, for ONE size (the step kernels of
+// hexb_step.cuh in their one-warp and 4-warp-per-chunk forms, and the kernels below): compiled once per
 // N = 3..19 with -DHEXB_INST_N=n (hex_gym_env_b200/_native.py builds the 17 objects in parallel and links them with
 // hexb_kernels.cu). nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo.
 #ifndef HEXB_INST_N

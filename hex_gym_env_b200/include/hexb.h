@@ -112,10 +112,11 @@ int32_t hexb_step(hexb_env *env, const int32_t *actions, const double *opp_u, vo
                   uint8_t *done, void *term_obs, int32_t *actions_out, void *stream);
 
 /* How hexb_step / hexb_rollout spread a chunk of 32 games over warps: 0 (default) = chosen by the depth of the launch, 1 = one
- * warp per chunk (the form for deep, bandwidth-bound launches), 2 / 4 / 8 = a CTA of that many warps per chunk (sub-wave
- * launches, where a step costs one warp's instruction latency: the warps split the relabel sweeps of flood_fill,
- * HexGame.py:124-142 / HexSingleGame.py:135-153, the observation + mask encode and the games of the thread-per-game phase).
- * Results do not depend on the form; the call exists for tuning and for tests that cover every form. */
+ * warp per chunk (the form for deep, bandwidth-bound launches), 4 = a CTA of 4 warps per chunk (sub-wave launches, where a step
+ * costs one warp's instruction latency: the warps split the relabel sweeps of flood_fill, HexGame.py:124-142 /
+ * HexSingleGame.py:135-153, the observation + mask encode and the games of the thread-per-game phase). Any other value returns
+ * HEXB_ERR_ARG. Results do not depend on the form; the call lets tests run each form on batch sizes where the depth rule would
+ * pick the other. */
 int32_t hexb_set_launch_form(hexb_env *env, int32_t warps_per_chunk);
 
 /* T env steps in ONE launch with the fused random agent (the reference's random-vs-random rollout loop,

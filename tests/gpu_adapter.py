@@ -11,7 +11,7 @@ class GpuBatch(object):
     def __init__(self, variant, N, G, launch_form=0, obs_f32=False, **kw):
         self.b = HexBatch(N, G, variant=variant, device=0, obs_dtype=torch.float32 if obs_f32 else torch.int8, **kw)
         if launch_form:
-            self.b.set_launch_form(launch_form)   # 1 / 2 / 4 / 8 warps per chunk instead of the depth-based choice
+            self.b.set_launch_form(launch_form)   # 1 / 4 warps per chunk instead of the depth-based choice
         self.N, self.G = N, G
 
     @staticmethod

@@ -1,4 +1,4 @@
-"""GPU (-m gpu): every launch form of the step kernel gives the same bits. hexb_set_launch_form forces 1 / 2 / 4 / 8 warps per
+"""GPU (-m gpu): every launch form of the step kernel gives the same bits. hexb_set_launch_form forces 1 / 4 warps per
 32-game chunk (the cooperative sub-wave form of csrc/hexb_step.cuh); each is run against the oracle on the same seeded inputs
 for every board size, for both env variants, with and without auto-reset, for single steps and hexb_rollout. Also here: float32
 observations (hexb_config.obs_dtype) against the int8 ones."""
@@ -21,7 +21,7 @@ def adapter():
 
 
 @pytest.mark.parametrize("N", list(range(3, 20)))
-@pytest.mark.parametrize("form", [2, 4, 8])
+@pytest.mark.parametrize("form", [4])
 def test_every_board_size_every_form(adapter, N, form):
     """SelfPlayEnv, fused random agent, random agent colour, auto-reset: long enough that games finish, restart and the opponent
     opens; G is ragged (last chunk partly empty)."""
@@ -31,14 +31,14 @@ def test_every_board_size_every_form(adapter, N, form):
                          agent_mode=2, check_state_every=5)
 
 
-@pytest.mark.parametrize("form", [1, 2, 4, 8])
+@pytest.mark.parametrize("form", [1, 4])
 @pytest.mark.parametrize("N", [4, 5, 7, 11])
 def test_forms_external_actions_illegal_moves(adapter, form, N):
     parity.versus_oracle(adapter.make_with(launch_form=form), hexref.KIND_SELFPLAY_B, N, 500, N * N, seed=7 + N, fused=False,
                          agent_mode=1, illegal_rate=0.08, check_state_every=4)
 
 
-@pytest.mark.parametrize("form", [2, 4, 8])
+@pytest.mark.parametrize("form", [4])
 @pytest.mark.parametrize("kind", [hexref.KIND_SELFPLAY_B, hexref.KIND_ENV_A])
 def test_forms_no_auto_reset(adapter, form, kind):
     """Without auto-reset the opponent-view rows (games the agent's own ply finished) are rewritten after the chunk encode."""
@@ -48,36 +48,40 @@ def test_forms_no_auto_reset(adapter, form, kind):
                              illegal_rate=0.1, **kw)
 
 
-@pytest.mark.parametrize("form", [2, 4, 8])
+@pytest.mark.parametrize("form", [4])
 @pytest.mark.parametrize("N", [3, 7, 10])
 def test_forms_variant_a(adapter, form, N):
     parity.versus_oracle(adapter.make_with(launch_form=form), hexref.KIND_ENV_A, N, 700, N * N, seed=5 + N, fused=True,
                          check_state_every=3)
 
 
-@pytest.mark.parametrize("form", [1, 2, 4, 8])
+@pytest.mark.parametrize("form", [1, 4])
 @pytest.mark.parametrize("N", [5, 6, 11])
 def test_forms_rollout_equals_steps(adapter, form, N):
     parity.rollout_equals_steps(adapter.make_with(launch_form=form), hexref.KIND_SELFPLAY_B, N, 200, 20, seed=form + N, agent_mode=2)
 
 
-@pytest.mark.parametrize("form", [2, 4, 8])
+@pytest.mark.parametrize("form", [4])
 def test_forms_api_fuzz(adapter, form):
     for seed in range(6):
         parity.api_fuzz(adapter.make_with(launch_form=form), 50 * form + seed, T=40)
 
 
-def test_forms_same_trajectory_large_batch(adapter):
-    """20,000 games of 7x7 and 11x11: the four forms against each other (obs, mask, reward, done, actions, state, statistics)."""
+def test_forms_1_and_4_same_trajectory_large_batch(adapter):
+    """20,000 games of 7x7 and 11x11: the two forms against each other (obs, mask, reward, done, actions, state, statistics);
+    no other form is accepted."""
     import torch
-    from hex_gym_env_b200 import HexBatch
+    from hex_gym_env_b200 import HexBatch, HexbError
     for N, G, T in ((7, 20000, 45), (11, 20000, 70)):
         envs = []
-        for form in (1, 2, 4, 8):
+        for form in (1, 4):
             b = HexBatch(N, G, variant=1, device=0, seed=5, agent_mode=2)
             b.set_launch_form(form)
             b.reset()
             envs.append(b)
+        for form in (2, 8):
+            with pytest.raises(HexbError):
+                envs[0].set_launch_form(form)
         for t in range(T):
             outs = [b.step(want_actions=True, want_term=True) for b in envs]
             for o in outs[1:]:

@@ -23,7 +23,7 @@ def intact(raw, n):
     return bool((a[:GUARD] == SENT).all() and (a[GUARD + n:] == SENT).all())
 
 
-@pytest.mark.parametrize("form", [1, 2, 4, 8])
+@pytest.mark.parametrize("form", [1, 4])
 @pytest.mark.parametrize("f32", [False, True])
 def test_outputs_stay_inside_their_buffers(form, f32):
     import torch

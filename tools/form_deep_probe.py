@@ -5,7 +5,7 @@ from hex_gym_env_b200 import HexBatch, VARIANT_B, AGENT_RANDOM
 from bench import capture_steps
 dev = torch.device("cuda", 0)
 for N, G, K in ((19, 1 << 20, 40), (15, 1 << 20, 60), (13, 1 << 20, 60)):
-    for form in (0, 1, 2, 4):
+    for form in (0, 1, 4):
         env = HexBatch(N, G, variant=VARIANT_B, device=0, seed=0, agent_mode=AGENT_RANDOM)
         if form: env.set_launch_form(form)
         env.reset(); env.rollout(400, outputs=False)

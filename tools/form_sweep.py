@@ -1,4 +1,4 @@
-"""Step time of every launch form (1 / 2 / 4 / 8 warps per 32-game chunk, hexb_set_launch_form) on sub-wave and near-wave
+"""Step time of every launch form (1 / 4 warps per 32-game chunk, hexb_set_launch_form) on sub-wave and near-wave
 batches, timed as ONE CUDA graph of K steps after a pre-roll (the same method as bench.py's extra_configs). One JSON line per
 (config, form); `auto` is what the library picks by itself. Also times hexb_rollout (T steps per launch) per form."""
 import json, os, sys
@@ -21,7 +21,7 @@ only = sys.argv[1:]
 for name, N, G, variant, am in CONFIGS:
     if only and not any(o in name for o in only):
         continue
-    for form in (0, 1, 2, 4, 8):
+    for form in (0, 1, 4):
         env = HexBatch(N, G, variant=variant, device=0, seed=0, agent_mode=am)
         env.set_launch_form(form)
         env.reset()
