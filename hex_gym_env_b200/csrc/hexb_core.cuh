@@ -158,6 +158,10 @@ HEXB_HD uint32_t mulhi32(uint32_t a, uint32_t b) {
 }
 HEXB_HD uint32_t splat(uint32_t b) { return b * 0x01010101u; }
 HEXB_HD uint32_t umin32(uint32_t a, uint32_t b) { return a < b ? a : b; }
+// a + b issued as a multiply-add (IMAD, FMA pipe) instead of an add (IADD3 / VIADD, ALU pipe). `one` is Params::one: the
+// step kernel is bound by the ALU pipe (LOP3 / SHF / PRMT / ISETP, rt 2 cycles per warp instruction and SMSP) while the FMA
+// pipe idles, so the adds and shifts of the byte-SIMD loops are steered there.
+HEXB_HD uint32_t fma_add(uint32_t a, uint32_t b, uint32_t one) { return a * one + b; }
 
 // Philox4x32-10 (Random123); pinned by the Random123 known-answer vectors in tests/test_philox.py.
 HEXB_HD void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t &o0, uint32_t &o1) {
@@ -208,18 +212,15 @@ HEXB_HD int choice_of(double u, int n) {
 template <int N>
 HEXB_HD int select_kth_set(const uint32_t (&bits)[Geo<N>::W], int k) {
     constexpr int W = Geo<N>::W;
-    uint32_t z = 0;
-    int base = 0;
-    bool found = false;
+    // the word holding it is the last word w whose preceding words hold at most k set bits (the counts below only grow)
+    uint32_t z = bits[0];
+    int base = 0, below = 0, before = popc32(bits[0]);   // set bits in the words before w
 #pragma unroll
-    for (int w = 0; w < W; ++w) {
-        const uint32_t zw = bits[w];
-        const int c = popc32(zw);
-        if (!found) {
-            if (k < c) { z = zw; base = 32 * w; found = true; }
-            else k -= c;
-        }
+    for (int w = 1; w < W; ++w) {
+        if (k >= before) { z = bits[w]; base = 32 * w; below = before; }
+        before += popc32(bits[w]);
     }
+    k -= below;
     // k-th set bit of z by halving
     int pos = 0, c;
     c = popc32(z & 0xffffu); if (k >= c) { k -= c; pos += 16; z >>= 16; }
@@ -316,10 +317,23 @@ HEXB_HD bool test_bit(const uint32_t (&bb)[Geo<N>::W], int i) {
     for (int w = 0; w < Geo<N>::W; ++w) v |= bb[w] & (0u - (uint32_t)(w == (i >> 5)));
     return (v >> (i & 31)) & 1u;
 }
+// the bit of cell i in word w of a bitboard, 0 when i lies in another word: one shift by i - 32w, which the device clamps (shl.b32
+// with a count >= 32, negative counts included, gives 0), instead of a compare and a select per word (ALU pipe; the subtraction
+// is a multiply-add, see fma_add)
+HEXB_HD uint32_t word_bit(int i, int w, uint32_t one) {
+    const uint32_t s = fma_add((uint32_t)i, (uint32_t)(-32 * w), one);
+#if defined(__CUDA_ARCH__)
+    uint32_t d;
+    asm("shl.b32 %0, %1, %2;" : "=r"(d) : "r"(1u), "r"(s));
+    return d;
+#else
+    return s < 32u ? 1u << s : 0u;
+#endif
+}
 template <int N>
-HEXB_HD void set_bit(uint32_t (&bb)[Geo<N>::W], int i) {
+HEXB_HD void set_bit(uint32_t (&bb)[Geo<N>::W], int i, uint32_t one = 1u) {
 #pragma unroll
-    for (int w = 0; w < Geo<N>::W; ++w) bb[w] |= (w == (i >> 5)) ? (1u << (i & 31)) : 0u;
+    for (int w = 0; w < Geo<N>::W; ++w) bb[w] |= word_bit(i, w, one);
 }
 
 template <int N>
@@ -333,64 +347,67 @@ HEXB_HD int transpose_cell(int a) {
 // (HexGame.py:124-142, HexSingleGame.py:135-153) on the tagged label plane of ONE game.
 //   L      this game's C label bytes (shared memory on the device)
 //   p      0 = R, 1 = C      cell  stored row-major index, known to be empty
+//   one    Params::one (see fma_add)
 // Writes the new cell's byte, updates occupancy/counters/far flags in `rec`, and returns the relabel
 // request for the cooperative byte pass (regions[regions == label] = new_region_label, :141-142 / :152-153):
 // at most two labels besides the minimum can be adjacent (the six neighbours form a cycle; own stones
 // that are adjacent on the cycle already share a label), so `prm` carries o1, o2 and m.
 // Returns true iff the mover's far border now carries label 1 (regions[-1,-1] == 1, :102 / :111).
 // ----------------------------------------------------------------------------------------------
+// A neighbour's byte as the mover's label biased by tag = p << 7: an own stone gives label + tag (tag + 1 .. tag + 127), an empty
+// cell or a stone of the other colour a value <= tag as a signed int (for R the byte is sign-extended, so C stones are negative
+// and an empty cell is 0; for C the plain byte of an R stone or an empty cell is below 128).
+HEXB_HD int32_t own_biased(uint32_t b, int p) { return p ? (int32_t)b : (int32_t)(int8_t)b; }
+// The smallest biased label above kb among s[], as d = label - (kb + 1) >= 0, or a negative d (as a signed int) if there is none:
+// every s <= kb gives s - (kb + 1) in [-384, -1], i.e. >= 2^31 unsigned, so one unsigned min filters and selects at once. The
+// subtractions are multiply-adds (FMA pipe), the mins VIMNMX3 (ALU pipe).
+HEXB_HD uint32_t next_above(const int32_t (&s)[6], uint32_t kb, uint32_t one) {
+    uint32_t d[6];
+#pragma unroll
+    for (int i = 0; i < 6; ++i) d[i] = fma_add((uint32_t)s[i], ~kb, one);   // s - kb - 1
+    return umin32(umin32(umin32(d[0], d[1]), d[2]), umin32(umin32(d[3], d[4]), d[5]));
+}
 template <int N>
-HEXB_HD bool place_stone(uint8_t *L, Rec<N> &rec, int p, int cell, uint32_t &prm) {
+HEXB_HD bool place_stone(uint8_t *L, Rec<N> &rec, int p, int cell, uint32_t &prm, uint32_t one = 1u) {
     const int y = cell / N, x = cell - y * N;
     const uint32_t tag = (uint32_t)p << 7;
     const bool up = y > 0, dn = y < N - 1, lf = x > 0, rt = x < N - 1;
-    // 3x3 window minus [0,0] and [2,2] (neighborhood[0,0] = neighborhood[2,2] = 0)
-    uint32_t v[8];
-    v[0] = up ? L[cell - N] : 0u;
-    v[1] = (up && rt) ? L[cell - N + 1] : 0u;
-    v[2] = lf ? L[cell - 1] : 0u;
-    v[3] = rt ? L[cell + 1] : 0u;
-    v[4] = (dn && lf) ? L[cell + N - 1] : 0u;
-    v[5] = dn ? L[cell + N] : 0u;
-    // own labels as (label - 1) in 0..126, everything else (empty, the other colour, off the board) as a value >= 127:
-    // (b ^ tag) is the plain label for an own stone, has bit 7 set for a stone of the other colour and is 0 or 0x80 for an
-    // empty cell, so one XOR and one decrement sort all three cases (labels stay below 128)
-    constexpr uint32_t NONE = 127u;
-#pragma unroll
-    for (int i = 0; i < 6; ++i) v[i] = (v[i] ^ tag) - 1u;
-    // implicit borders of the mover's padded plane
+    // implicit borders of the mover's padded plane: near border label 1, far border 1 once connected, else 2. Each takes the place
+    // of the one off-board neighbour that lies on it (R: up = row -1 / down = row N; C: left = column -1 / right = column N), which
+    // is off the board exactly when the cell touches that border; the other off-board neighbours count as nothing (0).
     const uint32_t far1 = p ? (rec.meta & M_FAR_C1) : (rec.meta & M_FAR_R1);
-    const bool near_edge = p ? (x == 0) : (y == 0);
-    const bool far_edge = p ? (x == N - 1) : (y == N - 1);
-    v[6] = near_edge ? 0u : NONE;                     // label 1
-    v[7] = far_edge ? (far1 ? 0u : 1u) : NONE;        // label 1 once connected, else 2
-    uint32_t m = umin32(umin32(umin32(v[0], v[1]), umin32(v[2], v[3])), umin32(umin32(v[4], v[5]), umin32(v[6], v[7])));
-    uint32_t o1 = NONE, o2 = NONE;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) o1 = (v[i] > m && v[i] < o1) ? v[i] : o1;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) o2 = (v[i] > o1 && v[i] < o2) ? v[i] : o2;  // o1 == NONE => nothing valid is > o1
-    // back to labels; 0xff = none
-    m = m < NONE ? m + 1u : 0xffu;
-    o1 = o1 < NONE ? o1 + 1u : 0xffu;
-    o2 = o2 < NONE ? o2 + 1u : 0xffu;
+    const int32_t nb = (int32_t)tag + 1, fb = (int32_t)tag + (far1 ? 1 : 2);
+    // the hex neighbourhood: 3x3 window minus [0,0] and [2,2] (neighborhood[0,0] = neighborhood[2,2] = 0)
+    int32_t s[6];
+    s[0] = up ? own_biased(L[cell - N], p) : (p ? 0 : nb);
+    s[1] = (up && rt) ? own_biased(L[cell - N + 1], p) : 0;
+    s[2] = lf ? own_biased(L[cell - 1], p) : (p ? nb : 0);
+    s[3] = rt ? own_biased(L[cell + 1], p) : (p ? fb : 0);
+    s[4] = (dn && lf) ? own_biased(L[cell + N - 1], p) : 0;
+    s[5] = dn ? own_biased(L[cell + N], p) : (p ? 0 : fb);
+    // m = the smallest adjacent own label, o1 < o2 the next larger ones (biased by tag, i.e. the tagged bytes)
+    const uint32_t dm = next_above(s, tag, one);
     const uint32_t cshift = p ? M_CTR_C_SHIFT : M_CTR_R_SHIFT;
     uint32_t lab;
     prm = 0;
-    if (m == 0xffu) {  // no adjacent region: new label = region_counter, counter += 1
-        lab = (rec.meta >> cshift) & 0xffu;
+    if ((int32_t)dm < 0) {  // no adjacent region: new label = region_counter, counter += 1
+        lab = ((rec.meta >> cshift) & 0xffu) | tag;
         rec.meta += 1u << cshift;
     } else {
-        lab = m;
-        if (o1 != 0xffu) {
-            const uint32_t o2e = (o2 != 0xffu) ? o2 : o1;
-            prm = (o1 | tag) | ((o2e | tag) << 8) | ((m | tag) << 16) | P_NEED;
-            // the relabel runs over the whole padded plane, borders included: 2 -> 1 moves the far border
-            if (m == 1u && !far1 && (o1 == 2u || o2 == 2u)) rec.meta |= p ? M_FAR_C1 : M_FAR_R1;
+        lab = dm + tag + 1u;
+        const uint32_t d1 = next_above(s, lab, one);
+        if ((int32_t)d1 >= 0) {
+            const uint32_t o1 = d1 + lab + 1u;
+            const uint32_t d2 = next_above(s, o1, one);
+            const uint32_t o2e = (int32_t)d2 >= 0 ? d2 + o1 + 1u : o1;
+            prm = o1 | (o2e << 8) | (lab << 16) | P_NEED;
+            // the relabel runs over the whole padded plane, borders included: 2 -> 1 moves the far border (m = 1 < o1 < o2, so
+            // label 2 can only be o1)
+            if (lab == tag + 1u && o1 == tag + 2u && !far1) rec.meta |= p ? M_FAR_C1 : M_FAR_R1;
         }
     }
-    L[cell] = (uint8_t)(lab | tag);
-    set_bit<N>(rec.occ_rm, cell);
+    L[cell] = (uint8_t)lab;
+    set_bit<N>(rec.occ_rm, cell, one);
     return (rec.meta & (p ? M_FAR_C1 : M_FAR_R1)) != 0u;
 }
 
@@ -423,10 +440,6 @@ HEXB_HD uint32_t splat_byte_dyn(uint32_t v, int p) {
     return ((v >> (8 * p)) & 0xffu) * 0x01010101u;
 #endif
 }
-// a + b issued as a multiply-add (IMAD, FMA pipe) instead of an add (IADD3 / VIADD, ALU pipe). `one` is Params::one: the
-// step kernel is bound by the ALU pipe (LOP3 / SHF / PRMT / ISETP, rt 2 cycles per warp instruction and SMSP) while the FMA
-// pipe idles, so the adds and shifts of the byte-SIMD loops are steered there.
-HEXB_HD uint32_t fma_add(uint32_t a, uint32_t b, uint32_t one) { return a * one + b; }
 
 // x >> 7 for a word of 0x80 byte flags, issued as a multiply-high so that it runs on the (idle) FMA pipe instead of the ALU
 // pipe, which is the busy one in the step kernel (ncu: sm__pipe_alu_cycles_active is the top pipe)

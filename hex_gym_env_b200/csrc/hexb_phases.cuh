@@ -110,7 +110,7 @@ HEXB_HD void game_step_pre(const Params &P, long long g, const Rec<N> &rec, doub
     if (q.valid) {
         uint32_t occ2[Geo<N>::W];
 #pragma unroll
-        for (int w = 0; w < Geo<N>::W; ++w) occ2[w] = rec.occ_rm[w] | ((w == (a >> 5)) ? (1u << (a & 31)) : 0u);
+        for (int w = 0; w < Geo<N>::W; ++w) occ2[w] = rec.occ_rm[w] | word_bit(a, w, P.one);
         const double u = P.opp_u ? P.opp_u[2 * g] : u_opp;
         q.n_reply = count_empty<N>(occ2);
         q.cell_reply = select_kth_zero_colmajor<N>(occ2, choice_of(u, q.n_reply), q.x_reply);  // k-th empty cell of the opponent's view
@@ -147,7 +147,7 @@ HEXB_HD void game_step_post(uint8_t *L, const Params &P, long long g, int t, Rec
             rec.meta |= M_DONE | M_INVALID | M_AGENT_ENDED;
             loc.reward = P.variant == VARIANT_A ? -100.f : 0.f;
         } else {
-            const bool won = place_stone<N>(L, rec, 0, a, prmA);
+            const bool won = place_stone<N>(L, rec, 0, a, prmA, P.one);
             loc.st[7]++;
             rec.meta ^= M_TOMOVE;
             if (won) {
@@ -164,7 +164,7 @@ HEXB_HD void game_step_post(uint8_t *L, const Params &P, long long g, int t, Rec
             // (Reading the reply's neighbourhood before the agent's stone is written - stone_merge for both plies side by side,
             // stone_commit afterwards - was measured and rejected: 15.15 vs 15.00 us at 131,072 games of 11x11, 100.0 vs 98.8 at
             // 1 Mi, profiles/r2p_merge2_ab.jsonl: the reply does not always happen, and the extra live registers cost more.)
-            const bool won = place_stone<N>(L, rec, 1, cell, prmB);
+            const bool won = place_stone<N>(L, rec, 1, cell, prmB, P.one);
             // A: the env transposes the move back to the true cell (HexGame.py:341-346); B: the index in the opponent's own view
             if (P.info_opp) opp_move = P.variant == VARIANT_A ? cell : x * N + (cell - x) / N;
             loc.st[7]++;
@@ -268,7 +268,7 @@ HEXB_HD void game_half(uint8_t *L, const Params &P, long long g, Rec<N> &rec, Lo
             rec.meta |= M_DONE | M_INVALID | (side == 0 ? M_AGENT_ENDED : 0u);
             loc.reward = (P.variant == VARIANT_A && side == 0) ? -100.f : 0.f;
         } else {
-            const bool won = place_stone<N>(L, rec, side, cell, side == 0 ? prmA : prmB);
+            const bool won = place_stone<N>(L, rec, side, cell, side == 0 ? prmA : prmB, P.one);
             loc.st[7]++;
             rec.meta ^= M_TOMOVE;
             if (won) {
@@ -315,7 +315,7 @@ HEXB_HD void game_ply(uint8_t *L, const Params &P, long long g, Rec<N> &rec, uin
     if ((unsigned)a < (unsigned)C) {
         const int cell = (P.variant == VARIANT_B && p) ? transpose_cell<N>(a) : a;
         if (!test_bit<N>(rec.occ_rm, cell)) {
-            const bool won = place_stone<N>(L, rec, p, cell, prmA);
+            const bool won = place_stone<N>(L, rec, p, cell, prmA, P.one);
             rec.meta ^= M_TOMOVE;
             r = -1;
             if (won) {
@@ -373,14 +373,14 @@ struct RowSpan {
 // prepared once per game by its own lane (thread-per-game, all lanes in parallel) instead of being decoded by every lane in
 // every pass: the sweeps are the largest consumer of the ALU pipe, which bounds the step kernel in the steady state.
 struct RowDesc {
-    int w0, wl;            // first and last word of the row's label bytes
-    uint32_t first, last;  // row_mask() of those two words (all ones when rows are word aligned)
+    int w0;                // first word of the row's label bytes (the last one is w0 + RowLanes<N>::SPAN)
+    uint32_t first, last;  // row_mask() of the first and the last word (all ones when rows are word aligned)
 };
 template <int N>
 HEXB_HD constexpr RowDesc make_row_desc(int r) {
     constexpr int C = Geo<N>::C;
     const int rs = r * C, re = rs + C;
-    return RowDesc{rs >> 2, (re - 1) >> 2, (C % 4 == 0) ? 0xffffffffu : 0xffffffffu << (8 * (rs & 3)),
+    return RowDesc{rs >> 2, (C % 4 == 0) ? 0xffffffffu : 0xffffffffu << (8 * (rs & 3)),
                    (C % 4 == 0) ? 0xffffffffu : 0xffffffffu >> (8 * (3 - ((re - 1) & 3)))};
 }
 #if defined(__CUDACC__) && !defined(HEXB_HOST_EMU)
@@ -418,16 +418,32 @@ HEXB_HD void prep_request(uint32_t prmA, uint32_t prmB, RelabelReq &q) {
     q.xn = news >> 8;
     q.nx = n - 1u;
 }
+// Every row spans the same number of words, SPAN + 1 (C = N * N is a multiple of 4 for even N and 1 more than one for odd N, so a
+// row that starts at byte offset r & 3 of its first word ends in word w0 + SPAN), so which lane holds a row's first or last word,
+// and which lanes have nothing to do, depends on the lane alone: those tests do not depend on the row and are hoisted out of the
+// warp's loop over rows.
+template <int N>
+struct RowLanes {
+    static constexpr int SPAN = (Geo<N>::C + 3) / 4 - 1;
+    static constexpr bool check() {
+        for (int r = 0; r < kWarp; ++r)
+            if (((r * Geo<N>::C + Geo<N>::C - 1) >> 2) - ((r * Geo<N>::C) >> 2) != SPAN) return false;
+        return true;
+    }
+    static_assert(check(), "every row of a chunk spans SPAN + 1 words");
+};
 template <int N, bool EXTRA = true>
 HEXB_HD void relabel_row_lane2(uint32_t *lab32, const RowDesc &d, int lane, uint32_t so0, uint32_t sn0, uint32_t xo, uint32_t xn, int nx,
                                uint32_t one) {
+    constexpr int SPAN = RowLanes<N>::SPAN;
 #pragma unroll
     for (int it = 0; it < RowSpan<N>::SWEEPS; ++it) {
-        const int w = d.w0 + lane + it * kWarp;
-        if (w > d.wl) break;
+        const int j = lane + it * kWarp;   // word j of the row
+        if (j > SPAN) break;
+        const int w = d.w0 + j;
         const uint32_t x = lab32[w];
         // bytes of the neighbouring games in the row's first / last word are blanked before the compare (labels are never 0)
-        const uint32_t rm = ((it == 0 && lane == 0) ? d.first : 0xffffffffu) & (w == d.wl ? d.last : 0xffffffffu);
+        const uint32_t rm = (d.first | (j == 0 ? 0u : 0xffffffffu)) & (d.last | (j == SPAN ? 0u : 0xffffffffu));
         uint32_t mk = sign_fill(zero_flags((x & rm) ^ so0, one));
         uint32_t x2 = (x & ~mk) | (sn0 & mk);
 #pragma unroll 1
@@ -436,7 +452,7 @@ HEXB_HD void relabel_row_lane2(uint32_t *lab32, const RowDesc &d, int lane, uint
             mk = sign_fill(zero_flags((x2 & rm) ^ so, one));
             x2 = (x2 & ~mk) | (sn & mk);
         }
-        if (x2 != x) lab32[w] = x2;
+        lab32[w] = x2;   // (unconditional: a predicated store issues all the same, and the compare is one ALU op more)
     }
 }
 

@@ -2,7 +2,7 @@
 // translation unit (hexb_step_inst.cu instantiates launch_tile<N> for N = HEXB_INST_N).
 //
 //   hexb_step_kernel<N, KIND, BATCHED>   one warp per chunk of 32 games; BATCHED picks the relabel sweep (several rows per pass
-//                                        for launches of at most one wave, one row per pass for deep, HBM-bound launches)
+//                                        for launches of at most one wave, one row per pass for deep, issue-bound launches)
 //   hexb_coop_kernel<N, KIND>            one CTA of 4 warps per chunk, for sub-wave launches (latency-bound)
 #pragma once
 #include "hexb_host.h"
@@ -347,7 +347,7 @@ __global__ void __launch_bounds__(kCtaThreads, min_ctas(N)) hexb_step_kernel(con
 
         // ---- row jobs, part 2: relabel sweeps (regions[regions == label] = new label, both plies of the step at once)
         if (!BATCHED) {
-            // one row per pass, one word per lane: the faster form when the launch is several waves deep (HBM-bound regime)
+            // one row per pass, one word per lane: the faster form when the launch is several waves deep (issue-bound regime)
             const bool need = (flg & (F_RELABEL | F_RESET)) == F_RELABEL;
             RelabelReq q = {0u, 0u, 0u, 0u, 0u};
             if (need) prep_request(prmA, prmB, q);   // each game's own lane decodes its requests once
