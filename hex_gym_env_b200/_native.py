@@ -170,6 +170,7 @@ SYMBOLS = {
     "hexb_mcts_select": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp, _vp]),
     "hexb_mcts_expand": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp]),
     "hexb_mcts_root": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp]),
+    "hexb_mcts_advance": (_i32, [_vp, _vp, _sz, ctypes.c_int64, _vp, _vp]),
 }
 
 _LIB = None

@@ -15,7 +15,7 @@
 //   K10       hexb_pack_obs_kernel    2-bit observation transport for hexb_step_host_packed
 //   K11       hexb_copy_kernel        copy.deepcopy(env.simulator) into a raw batch, one warp per copied game (hexb_search.cuh)
 //   K12       hexb_playout_kernel<N>  random playouts from the current position, one warp per game (hexb_step_inst.cu)
-//   K13       hexb_mcts_*_kernel<N>   batched PUCT tree search: init, fused search, select, expand, root readout (hexb_mcts.cuh)
+//   K13       hexb_mcts_*_kernel<N>   batched PUCT tree search: init, fused search, select, expand, root readout, advance (hexb_mcts.cuh)
 #include <cuda.h>   // types of the driver's virtual-memory API only (entry points come from cudaGetDriverEntryPoint)
 #include <cuda_runtime.h>
 #include <math.h>
@@ -1033,6 +1033,16 @@ int32_t hexb_mcts_root(const hexb_env *env, const void *tree, size_t tree_bytes,
     A.value = value;
     A.nodes_used = nodes_used;
     return mcts_launch(env, MCTS_ROOT, A, stream);
+}
+
+int32_t hexb_mcts_advance(const hexb_env *env, void *tree, size_t tree_bytes, int64_t first_playout, const uint8_t *root_mask,
+                          void *stream) {
+    if (!env || first_playout < 0 || first_playout >= (1ll << 32)) return HEXB_ERR_ARG;
+    if (!mcts_buffer_ok(tree, tree_bytes)) return HEXB_ERR_STATE;
+    MctsArgs A = mcts_args(env, tree, tree_bytes);
+    A.first_playout = first_playout;
+    A.root_mask = root_mask;
+    return mcts_launch(env, MCTS_ADVANCE, A, stream);
 }
 
 int32_t hexb_stats(hexb_env *env, int64_t *out8, void *stream) {

@@ -19,6 +19,8 @@
 //     + off_edges + n * 16 Cp      node n's edges, structure of arrays over the true row-major cell c < Cp:
 //                                  child i32[Cp] (-1 = none), N i32[Cp], W f32[Cp], P f32[Cp] (0 for cells not empty at the node)
 // Edge arrays are written only when a node is expanded; a terminal node has none.
+// Within one advance launch (mc_advance_root) a flag word also carries scratch: bit 2 marks a node of the kept subtree and bits
+// 3.. hold its new number. Every flag word is 0, 1 or 2 again when the launch ends.
 #pragma once
 #include <math.h>
 #include <string.h>
@@ -54,6 +56,12 @@ HEXB_HD unsigned long long mc_max(unsigned long long k) {
     return k;
 }
 HEXB_HD int mc_sum(int v) { return __reduce_add_sync(0xffffffffu, v); }
+// the lanes below this one with p set; total: the lanes with p set
+HEXB_HD int mc_prefix(bool p, int &total) {
+    const unsigned b = __ballot_sync(0xffffffffu, p);
+    total = __popc(b);
+    return __popc(b & ((1u << (threadIdx.x & 31)) - 1u));
+}
 HEXB_HD void mc_sync() { __syncwarp(); }
 // float32 arithmetic rounded once per operation, never contracted into an FMA (numpy float32 reproduces it)
 HEXB_HD float f_mul(float a, float b) { return __fmul_rn(a, b); }
@@ -67,6 +75,10 @@ HEXB_HD int mc_lane() { return 0; }
 HEXB_HD int mc_width() { return 1; }
 HEXB_HD unsigned long long mc_max(unsigned long long k) { return k; }
 HEXB_HD int mc_sum(int v) { return v; }
+HEXB_HD int mc_prefix(bool p, int &total) {
+    total = p ? 1 : 0;
+    return 0;
+}
 HEXB_HD void mc_sync() {}
 HEXB_HD float f_mul(float a, float b) { return a * b; }   // SSE: one rounding per operation (no FMA on the baseline x86-64 target)
 HEXB_HD float f_div(float a, float b) { return a / b; }
@@ -83,8 +95,8 @@ struct MctsArgs {
     unsigned long long seed, game_offset;
     int max_nodes;                 // init
     float c_puct, fpu;             // init
-    long long first_playout;       // init
-    const uint8_t *root_mask;      // init, [G] nullable
+    long long first_playout;       // init, advance
+    const uint8_t *root_mask;      // init, advance: [G] nullable
     int sims, playouts;            // search
     void *leaf_obs;                // select: obs dtype [G, C]
     uint8_t *leaf_mask, *pending;  // select: [G, C], [G]
@@ -336,14 +348,9 @@ HEXB_HD void mc_backup(const Tree &T, long long g, int D, int used, float v) {
 }
 
 // ---------------------------------------------------------------------------------------------- per-root calls
-// init: one thread per root
+// init's state of root g (one thread): node 0 unexpanded on (black, empty) with true colour to_move to move; -1 = inactive
 template <int N>
-HEXB_HD void mc_init_root(const View &V, const MctsArgs &A, long long g) {
-    Tree T;
-    mc_layout(T, N, V.G, A.max_nodes);
-    T.base = A.tree;
-    uint32_t black[N], empty[N];
-    const int to_move = (A.root_mask && !A.root_mask[g]) ? -1 : playout_rows<N>(V, g, black, empty);
+HEXB_HD void mc_fresh_root(const Tree &T, long long g, int to_move, const uint32_t (&black)[N], const uint32_t (&empty)[N]) {
     int32_t *m = mc_meta(T, g);
     for (int i = 0; i < 32; ++i) m[i] = 0;
     m[MM_NODE] = -1;
@@ -359,6 +366,17 @@ HEXB_HD void mc_init_root(const View &V, const MctsArgs &A, long long g) {
     }
     mc_nn(T, g)[0] = 0;
     mc_flag(T, g)[0] = MF_UNEXPANDED;
+}
+
+// init: one thread per root
+template <int N>
+HEXB_HD void mc_init_root(const View &V, const MctsArgs &A, long long g) {
+    Tree T;
+    mc_layout(T, N, V.G, A.max_nodes);
+    T.base = A.tree;
+    uint32_t black[N], empty[N];
+    const int to_move = (A.root_mask && !A.root_mask[g]) ? -1 : playout_rows<N>(V, g, black, empty);
+    mc_fresh_root<N>(T, g, to_move, black, empty);
 }
 
 // fused form: all simulations of one root (one warp)
@@ -505,6 +523,152 @@ HEXB_HD void mc_root_out(const Tree &T, int variant, const MctsArgs &A, long lon
         const int nn = on ? mc_nn(T, g)[0] : 0;
         if (A.value) A.value[g] = nn > 0 ? f_div(bits_f((uint32_t)m[MM_VSUM]), (float)nn) : 0.0f;
         if (A.nodes_used) A.nodes_used[g] = on ? m[MM_USED] : 0;
+    }
+}
+
+// advance's header field (written once per launch; no per-root code of that launch reads it)
+HEXB_HD void mc_write_first_playout(const MctsArgs &A) { *reinterpret_cast<long long *>(A.tree + 32) = A.first_playout; }
+
+// advance (one warp per root): keep the subtree under the game's current position, or start a fresh tree as init does
+template <int N>
+HEXB_HD void mc_advance_root(const Tree &T, const View &V, const MctsArgs &A, long long g) {
+    int32_t *m = mc_meta(T, g);
+    const int lane = mc_lane(), width = mc_width();
+    const bool lead = lane == 0;
+    uint32_t black[N], empty[N];
+    const int tn = (A.root_mask && !A.root_mask[g]) ? -1 : playout_rows<N>(V, g, black, empty);
+    // the moves from the old root's position P to the new one P': k = 0, 1 or 2 (c1 by the old side to move), -1 = no path
+    int k = -1, c1 = -1, c2 = -1;
+    if (tn >= 0 && m[MM_ACTIVE]) {
+        const int t0 = m[MM_TOMOVE] & 1;
+        const uint32_t *rows = mc_rows(T, g);
+        bool same = true;
+        int nb = 0, nw = 0, cb = -1, cw = -1;
+#pragma unroll
+        for (int y = 0; y < N; ++y) {
+            const uint32_t ob = rows[y], oe = rows[N + y], stones = ~oe & ((1u << N) - 1u);
+            same = same && (stones & empty[y]) == 0u && ((ob ^ black[y]) & stones) == 0u;   // every stone of P stays, same colour
+            const uint32_t add = oe & ~empty[y], ab = add & black[y], aw = add & ~black[y];
+            nb += popc32(ab);
+            nw += popc32(aw);
+            if (ab) cb = y * N + nth_set_bit(ab, 0);
+            if (aw) cw = y * N + nth_set_bit(aw, 0);
+        }
+        const int mine = t0 == 0 ? nb : nw, c_mine = t0 == 0 ? cb : cw, c_other = t0 == 0 ? cw : cb;
+        if (same && nb + nw == 0 && tn == t0) {
+            k = 0;
+        } else if (same && nb + nw == 1 && mine == 1 && tn == (t0 ^ 1)) {
+            k = 1;
+            c1 = c_mine;
+        } else if (same && nb == 1 && nw == 1 && tn == t0) {
+            k = 2;
+            c1 = c_mine;
+            c2 = c_other;
+        }
+    }
+    // walk the path from node 0: every node on it, and the node r reached, expanded; every child on it stored
+    const int used = m[MM_USED] < 1 ? 1 : (m[MM_USED] > T.max_nodes ? T.max_nodes : m[MM_USED]);
+    int32_t *fl = mc_flag(T, g);
+    int r = 0, parent = -1, cell = -1;
+    if (k >= 0 && fl[0] != MF_EXPANDED) k = -1;
+    for (int d = 0; d < k; ++d) {
+        const int c = d == 0 ? c1 : c2, j = mc_child(T, g, r)[c];
+        if (j < 0 || j >= used || fl[j] != MF_EXPANDED) {
+            k = -1;
+            break;
+        }
+        parent = r;
+        cell = c;
+        r = j;
+    }
+    if (k < 0) {
+        mc_sync();   // every lane has read the meta and the flags before lane 0 rewrites them
+        if (lead) mc_fresh_root<N>(T, g, tn, black, empty);
+        return;
+    }
+    int kept = used;
+    if (k > 0) {
+        const int32_t en = mc_edge_n(T, g, parent)[cell];   // the edge into r (its parent's slot is reused below)
+        const float ew = mc_edge_w(T, g, parent)[cell];
+        int32_t *nn = mc_nn(T, g);
+        // 1 mark r and every node reachable from it: a node is numbered after its parent, so one ascending pass sees a node's
+        //   mark before it reaches the node's children
+        mc_sync();
+        if (lead) fl[r] |= 4;
+        mc_sync();
+        for (int n = r; n < used; ++n) {
+            if (fl[n] == (4 | MF_EXPANDED)) {
+                const int32_t *ch = mc_child(T, g, n);
+                for (int c = lane; c < T.C; c += width) {
+                    const int j = ch[c];
+                    if (j >= 0 && j < used) fl[j] |= 4;
+                }
+            }
+            mc_sync();
+        }
+        // 2 new numbers in increasing old number (bits 3..)
+        kept = 0;
+        for (int base = r; base < used; base += width) {
+            const int n = base + lane;
+            const int f = n < used ? fl[n] : 0;
+            int total;
+            const int before = mc_prefix((f & 4) != 0, total);
+            if (f & 4) fl[n] = (f & 7) | ((kept + before) << 3);
+            kept += total;
+        }
+        mc_sync();
+        // 3 move node n to its new number m <= n with its children renumbered: a child j > n has not moved yet, so its slot still
+        //   holds its new number; every slot below n has been read already
+        for (int n = r; n < used; ++n) {
+            const int f = fl[n];
+            if (f & 4) {
+                const int to = f >> 3;
+                if ((f & 3) == MF_EXPANDED) {
+                    const int32_t *ch = mc_child(T, g, n), *eN = mc_edge_n(T, g, n);
+                    const float *eW = mc_edge_w(T, g, n), *eP = mc_edge_p(T, g, n);
+                    int32_t *ch2 = mc_child(T, g, to), *eN2 = mc_edge_n(T, g, to);
+                    float *eW2 = mc_edge_w(T, g, to), *eP2 = mc_edge_p(T, g, to);
+                    for (int c = lane; c < T.Cp; c += width) {
+                        const int j = ch[c];
+                        const int fj = j >= 0 && j < used ? fl[j] : 0;
+                        const int32_t x = eN[c];
+                        const float w = eW[c], p = eP[c];
+                        ch2[c] = (fj & 4) ? fj >> 3 : -1;
+                        eN2[c] = x;
+                        eW2[c] = w;
+                        eP2[c] = p;
+                    }
+                }
+                mc_sync();   // every lane has read the children's flags before lane 0 writes flags
+                if (lead) {
+                    nn[to] = nn[n];
+                    fl[n] = f & 3;
+                    fl[to] = f & 3;
+                }
+            }
+            mc_sync();
+        }
+        if (lead) {
+            nn[0] = en;
+            m[MM_SIMS] = en;
+            m[MM_VSUM] = (int32_t)(f_bits(ew) ^ 0x80000000u);
+            m[MM_TOMOVE] = tn;
+            uint32_t *rw = mc_rows(T, g);
+#pragma unroll
+            for (int y = 0; y < N; ++y) {
+                rw[y] = black[y];
+                rw[N + y] = empty[y];
+            }
+        }
+    }
+    mc_sync();   // every lane has read the meta
+    if (lead) {
+        m[MM_USED] = kept;
+        m[MM_PENDING] = 0;
+        m[MM_DEPTH] = 0;
+        m[MM_NODE] = -1;
+        m[MM_PARENT] = 0;
+        m[MM_CELL] = 0;
     }
 }
 

@@ -43,7 +43,7 @@ __global__ void __launch_bounds__(256) hexb_playout_kernel(View V, PlayoutArgs A
 }
 
 // hexb_mcts_*: the tree search of hexb_mcts.cuh. init: one thread per root (thread 0 also writes the header); the others: one warp
-// per root, all S simulations of the fused search in one launch.
+// per root, all S simulations of the fused search in one launch, and advance's subtree compaction.
 template <int N>
 __global__ void __launch_bounds__(128) hexb_mcts_init_kernel(View V, MctsArgs A) {
     const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -75,6 +75,16 @@ __global__ void __launch_bounds__(128) hexb_mcts_root_kernel(View V, MctsArgs A)
     Tree T;
     if (g < V.G && mc_tree(A, N, V.G, T)) mc_root_out(T, V.variant, A, g);
 }
+// advance: thread 0 writes the header's first_playout once the header has been checked; one warp per root
+template <int N>
+__global__ void __launch_bounds__(128) hexb_mcts_advance_kernel(View V, MctsArgs A) {
+    const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    Tree T;
+    if (g < V.G && mc_tree(A, N, V.G, T)) {
+        if (blockIdx.x == 0 && threadIdx.x == 0) mc_write_first_playout(A);
+        mc_advance_root<N>(T, V, A, g);
+    }
+}
 
 int HEXB_CAT(hexb_launch_tile_, HEXB_INST_N)(const hexb_env *e, const Params &P, cudaStream_t s) { return launch_tile<HEXB_INST_N>(e, P, s); }
 
@@ -105,6 +115,7 @@ int HEXB_CAT(hexb_launch_mcts_, HEXB_INST_N)(int op, const View &V, const MctsAr
         case MCTS_SELECT: hexb_mcts_select_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
         case MCTS_EXPAND: hexb_mcts_expand_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
         case MCTS_ROOT: hexb_mcts_root_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
+        case MCTS_ADVANCE: hexb_mcts_advance_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
         default: return HEXB_ERR_ARG;
     }
     CK(cudaGetLastError());

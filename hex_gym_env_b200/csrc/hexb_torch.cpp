@@ -233,6 +233,14 @@ void op_mcts_root(int64_t handle, Tensor tree, OptT visits, OptT q, OptT value, 
              "mcts_root");
 }
 
+void op_mcts_advance(int64_t handle, Tensor tree, int64_t first_playout, OptT root_mask) {
+    Call k(handle);
+    const int d = k.c.device;
+    check_rc(hexb_mcts_advance(k.e, tree_of(tree, d), (size_t)tree.numel(), first_playout,
+                               ptr<const uint8_t>(root_mask, at::kByte, k.G, d, "root_mask"), k.stream),
+             "mcts_advance");
+}
+
 int64_t op_version() { return hexb_version(); }
 
 }  // namespace
@@ -260,6 +268,7 @@ TORCH_LIBRARY(hexb, m) {
     m.def("mcts_select(int env, Tensor(a!) tree, Tensor(b!) leaf_obs, Tensor(c!) leaf_mask, Tensor(d!) pending) -> ()");
     m.def("mcts_expand(int env, Tensor(a!) tree, Tensor priors, Tensor values) -> ()");
     m.def("mcts_root(int env, Tensor tree, Tensor(a!)? visits, Tensor(b!)? q, Tensor(c!)? value, Tensor(d!)? nodes_used) -> ()");
+    m.def("mcts_advance(int env, Tensor(a!) tree, int first_playout, Tensor? root_mask) -> ()");
 }
 
 // The handle is an int, so these operators have no tensor argument to dispatch on when every optional is None: register them
@@ -283,4 +292,5 @@ TORCH_LIBRARY_IMPL(hexb, CompositeExplicitAutograd, m) {
     m.impl("mcts_select", &op_mcts_select);
     m.impl("mcts_expand", &op_mcts_expand);
     m.impl("mcts_root", &op_mcts_root);
+    m.impl("mcts_advance", &op_mcts_advance);
 }

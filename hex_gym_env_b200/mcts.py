@@ -13,6 +13,10 @@
         priors, values = net(obs, mask)         # f32[G,C], f32[G]; rows with pending == 0 are ignored
         tree.expand(priors, values)
 
+    visits = tree.root()[0]
+    env.ply(visits.argmax(1).int())             # play the move (raw handle; an env step adds the reply too)
+    tree.advance()                              # keep the subtree under the position reached, then search on from it
+
 Per-cell arrays use the batch's action convention for the side to move at that node (variant B: the mover's view), so for an
 env root at the agent's turn `visits.argmax(1)` is an action for `env.step`.
 """
@@ -92,6 +96,19 @@ class MCTS(object):
         h, t, nb = self._args()
         with torch.cuda.device(self.device):
             check(self._lib.hexb_mcts_expand(h, t, nb, _ptr(p), _ptr(v), self.batch._stream()))
+
+    def advance(self, root_mask=None, first_playout=0):
+        """Keep each root's subtree under the position its game has reached since the last reset / advance (one or two stones
+        on along explored moves: a ply, or an env step with the opponent's reply), or start a fresh tree there as reset() would.
+        Roots that are finished, never reset or have root_mask[g] == 0 become inactive. The kept root's counters are those of
+        the edge into it; later fused simulations use playout indices from first_playout (include/hexb.h, hexb_mcts_advance)."""
+        first_playout = int(first_playout)
+        if not 0 <= first_playout < 1 << 32:
+            raise ValueError("first_playout must be in [0, 2**32)")
+        rm = self.batch._in(root_mask, (self.batch.G,), torch.uint8, "root_mask")
+        h, t, nb = self._args()
+        with torch.cuda.device(self.device):
+            check(self._lib.hexb_mcts_advance(h, t, nb, first_playout, _ptr(rm), self.batch._stream()))
 
     def root(self):
         """(visits i32[G,C], q f32[G,C], value f32[G], nodes_used i32[G]) of every root; nodes_used == 0 marks an inactive root."""

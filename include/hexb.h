@@ -257,7 +257,7 @@ int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout
  * `stream`, allocates nothing and reads nothing on the host (CUDA-graph capturable). Bad max_nodes (1..2^24), num_simulations
  * (>= 1), playouts_per_leaf (1..65536), c_puct / fpu (NaN) or first_playout (0..2^32-1): HEXB_ERR_ARG; a null or misaligned
  * tree, or one smaller than hexb_mcts_tree_bytes: HEXB_ERR_STATE. A buffer that holds no tree of this handle (init never ran on
- * it, other board size or game count) is left alone by search / select / expand / root.
+ * it, other board size or game count) is left alone by search / select / expand / root / advance.
  *
  * init: each root's current position is read in true orientation. A root is inactive (nothing is ever done for it) if its game
  *   is finished, was never reset or has root_mask[g] == 0 (u8[G], null = all); an active root gets node 0, unexpanded, and
@@ -304,6 +304,28 @@ int32_t hexb_mcts_expand(const hexb_env *env, void *tree, size_t tree_bytes, con
  * the first simulation), nodes_used i32[G] (0 = inactive root). Every output is nullable. */
 int32_t hexb_mcts_root(const hexb_env *env, const void *tree, size_t tree_bytes, int32_t *visits, float *q, float *value,
                        int32_t *nodes_used, void *stream);
+/* Tree reuse across moves: re-root every root's tree on the position its game has reached. For each root g:
+ *   1 a root whose game is finished, was never reset or has root_mask[g] == 0 (u8[G], null = all) becomes inactive, as in init.
+ *   2 the game's position P' (true orientation, side to move t') is compared with the root's position P (side to move t0): every
+ *     stone of P must still be in P' with the same colour; A = the stones P' adds. |A| = 0 and t' = t0: the tree is kept as it
+ *     is. |A| = 1, a stone of t0 and t' = t0 ^ 1: the path is (c1). |A| = 2, one stone of each colour and t' = t0: the path is
+ *     (c1 = t0's stone, c2 = the other). Anything else, or a root that was inactive: a fresh tree, exactly as init leaves it.
+ *   3 the path is walked from node 0: every node on it must be expanded, its child at the path cell a stored node
+ *     (0 <= child < nodes used), and the node r reached expanded; otherwise the root gets a fresh tree (a move never visited, a
+ *     pool that was full when the child would have been stored, node 0 before its first simulation).
+ *   4 the kept nodes are r and every node reachable from it through child pointers, renumbered in increasing old number (r
+ *     becomes node 0); each keeps its flag, Nn and edges (child pointers renumbered). Nodes used = the kept count, the root's
+ *     position = P' with t' to move, s and node 0's Nn = N of the edge into r, the root's value sum = -W of that edge (an exact
+ *     float32 sign flip). Usually that N equals Nn(r); they differ only when r was stored after its edge had been visited (a
+ *     pool that was full, then freed by an earlier advance). A pending split-form leaf is cleared.
+ *   5 first_playout (0..2^32-1) replaces the tree's: later fused simulations use playout index first_playout + s * P + j with
+ *     the root's new s. c_puct, fpu and max_nodes are unchanged.
+ * So after a one-move advance the root's visits are the old edge's N and its value is -(the old root's q at the played cell).
+ * Stones are matched, not moves: ply() on a raw handle adds one stone, an env step the agent's move and the opponent's reply, and
+ * an episode end or auto-reset gives a fresh or inactive root. A select / expand pair must not straddle an advance. Argument
+ * checks as above; asynchronous, no allocation, no host read. */
+int32_t hexb_mcts_advance(const hexb_env *env, void *tree, size_t tree_bytes, int64_t first_playout, const uint8_t *root_mask,
+                          void *stream);
 
 /* Episode statistics accumulated by hexb_step since creation, int64[8] on the device:
  * [0] episodes finished, [1] BLACK wins, [2] WHITE wins, [3] agent wins, [4] plies of finished episodes,
