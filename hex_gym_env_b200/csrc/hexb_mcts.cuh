@@ -237,7 +237,9 @@ HEXB_HD int mc_action(int variant, int colour, int N, int c) {
 
 // ---------------------------------------------------------------------------------------------- one simulation
 // PUCT key of every empty cell of an expanded node; the largest wins. Score bits made order-preserving as unsigned, in the high
-// half; 0xffffffff - cell in the low half breaks ties towards the lowest cell. 0 = no empty cell.
+// half; 0xffffffff - cell in the low half breaks ties towards the lowest cell. 0 = no empty cell. Adding +0 turns -0 into +0, so
+// the two zeros tie; a NaN score gets 0 in the high half, below every number (the host and the device make NaNs of different
+// bits, so the bits must not rank them).
 template <int N>
 HEXB_HD int mc_best_cell(const Tree &T, long long g, int node, const uint32_t (&empty)[N]) {
     const int32_t *en = mc_edge_n(T, g, node);
@@ -249,8 +251,9 @@ HEXB_HD int mc_best_cell(const Tree &T, long long g, int node, const uint32_t (&
         const int n = en[c];
         const float q = n > 0 ? f_div(ew[c], (float)n) : T.fpu;
         const float u = f_div(f_mul(f_mul(T.c_puct, ep[c]), sq), (float)(1 + n));
-        const uint32_t b = f_bits(f_add(q, u));
-        const uint32_t ord = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+        const float x = f_add(f_add(q, u), 0.0f);
+        const uint32_t b = f_bits(x);
+        const uint32_t ord = x != x ? 0u : (b & 0x80000000u) ? ~b : (b | 0x80000000u);
         const unsigned long long key = ((unsigned long long)ord << 32) | (0xffffffffu - (uint32_t)c);
         best = key > best ? key : best;
     }

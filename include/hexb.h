@@ -268,7 +268,10 @@ int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout
  * One simulation:
  *   1 select: from node 0, at an expanded non-terminal node take the empty cell with the largest Q + U, Q = W / N if N > 0 else
  *     fpu, U = c_puct * P * sqrt(Nn) / (1 + N), in float32 with every operation rounded once (no FMA; exactly
- *     ((c_puct * P) * sqrt(Nn)) / (1 + N), then Q + U), ties to the lowest true row-major cell. An expanded child: descend; a
+ *     ((c_puct * P) * sqrt(Nn)) / (1 + N), then Q + U), ties to the lowest true row-major cell; -0 and +0 tie. A NaN Q + U
+ *     ranks below every number: such a cell is taken only when every empty cell's Q + U is NaN, and then the lowest such cell
+ *     wins. (A NaN can come from infinite or NaN values, c_puct = inf with a zero prior, or fpu = -inf against an infinite U.
+ *     Which NaN bit pattern W, q and value then hold is not part of this definition.) An expanded child: descend; a
  *     terminal child is the leaf; no child: the new position is the leaf. Node 0 before its first simulation, and a node with no
  *     empty cell, is itself the leaf.
  *   2 value v for the leaf's side to move: if the move into a new leaf connects the mover's edges the leaf is terminal and

@@ -20,9 +20,11 @@ def action(variant, colour, N, c):
 
 
 def key(score, cell):
-    """Order-preserving bits of the float32 score, ties to the lowest cell: the largest key wins."""
-    b = int(np.array(score, np.float32).view(np.uint32))
-    ordered = (~b & 0xFFFFFFFF) if b & 0x80000000 else (b | 0x80000000)
+    """Order-preserving bits of the float32 score, ties to the lowest cell: the largest key wins. -0 counts as +0 (adding +0
+    turns it into +0), and a NaN score ranks below every number, whatever its bits."""
+    s = np.float32(score) + F(0)
+    b = int(np.array(s, np.float32).view(np.uint32))
+    ordered = 0 if np.isnan(s) else (~b & 0xFFFFFFFF) if b & 0x80000000 else (b | 0x80000000)
     return (ordered << 32) | (0xFFFFFFFF - cell)
 
 

@@ -50,8 +50,19 @@ def oracle_trees(export, seed, game_offset, variant, max_nodes, c_puct, fpu, fir
     return out
 
 
+def same_bits(a, b):
+    """Float32 arrays (or scalars) equal bit for bit, except that any NaN matches any NaN: which NaN a sum makes differs between the
+    host and the device and is not part of the search's definition (include/hexb.h)."""
+    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
+    if a.shape != b.shape:
+        return False
+    na, nb = np.isnan(a), np.isnan(b)
+    return bool(np.array_equal(na, nb) and np.array_equal(a.view(np.uint32)[~na], b.view(np.uint32)[~nb]))
+
+
 def assert_trees_equal(roots, oracle):
-    """Bit for bit over the whole tree: every node's flag and Nn, every expanded node's edge arrays, the root's counters and sum."""
+    """Bit for bit over the whole tree (same_bits for the floats): every node's flag and Nn, every expanded node's edge arrays, the
+    root's counters and sum."""
     assert len(roots) == len(oracle)
     for g, (r, o) in enumerate(zip(roots, oracle)):
         if o is None:
@@ -59,15 +70,15 @@ def assert_trees_equal(roots, oracle):
             continue
         assert r["active"] == 1 and r["to_move"] == o.t0, g
         assert r["used"] == len(o.nodes) and r["s"] == o.s, (g, r["used"], len(o.nodes), r["s"], o.s)
-        assert r["vsum"].view(np.uint32) == np.float32(o.vsum).view(np.uint32), (g, r["vsum"], o.vsum)
+        assert same_bits(r["vsum"], o.vsum), (g, r["vsum"], o.vsum)
         for k, (a, b) in enumerate(zip(r["nodes"], o.nodes)):
             assert a["flag"] == b.flag and a["nn"] == b.nn, (g, k, a["flag"], b.flag, a["nn"], b.nn)
             if b.flag != mcts.EXPANDED:
                 continue
             assert np.array_equal(a["child"], b.child), (g, k)
             assert np.array_equal(a["n"], b.n), (g, k)
-            assert np.array_equal(a["w"].view(np.uint32), b.w.view(np.uint32)), (g, k)
-            assert np.array_equal(a["p"].view(np.uint32), b.p.view(np.uint32)), (g, k)
+            assert same_bits(a["w"], b.w), (g, k)
+            assert same_bits(a["p"], b.p), (g, k)
 
 
 def one_move_win_positions(rng, G, N):
@@ -109,3 +120,26 @@ def as_oracle(r):
 def assert_same_tree(a, b, N, G):
     """Two tree buffers hold the same trees (bytes the layout leaves unused, e.g. free node slots, are not compared)."""
     assert_trees_equal(parse_tree(a, N, G), [as_oracle(r) for r in parse_tree(b, N, G)])
+
+
+# ---------------------------------------------------------------------------------------------- float edges of the split form
+# (test_mcts_edges_cpu.py, test_gpu_mcts_edges.py) c_puct x fpu, and the priors and values expand is handed: zeros of both signs,
+# subnormals, numbers near the float32 limit (W overflows to inf), infinities and NaNs of both signs.
+EDGE_SETTINGS = [(c, f) for c in (0.0, 1e-30, 1e30, np.inf) for f in (-np.inf, -0.0, np.inf)]
+EDGE_PRIORS = np.array([0.0, -0.0, 1e-45, 1e-39, 3e38, -0.5, -3e38, 0.25, 1.0], np.float32)
+EDGE_VALUES = np.array([0.0, -0.0, 1.0, -1.0, 3e38, -3e38, np.inf, -np.inf, np.nan, -np.nan], np.float32)
+
+
+def edge_inputs(rng, G, C):
+    """priors f32[G, C] and values f32[G] for one expand: each entry an edge value or, one time in three, an ordinary one."""
+    priors = np.where(rng.uniform(size=(G, C)) < 2 / 3, rng.choice(EDGE_PRIORS, size=(G, C)),
+                      rng.uniform(0, 1, size=(G, C))).astype(np.float32)
+    values = np.where(rng.uniform(size=G) < 2 / 3, rng.choice(EDGE_VALUES, size=G), rng.uniform(-1, 1, size=G)).astype(np.float32)
+    return priors, values
+
+
+def assert_root_outputs_equal(got, want):
+    """root() outputs (visits, q, value, nodes_used) of two sides: the counts exactly, the floats by same_bits."""
+    visits, q, value, used = (np.asarray(x) for x in got)
+    assert np.array_equal(visits, np.asarray(want[0])) and np.array_equal(used, np.asarray(want[3]))
+    assert same_bits(q, want[1]) and same_bits(value, want[2])
