@@ -164,9 +164,11 @@ SYMBOLS = {
     "hexb_masked_sample": (_i32, [_vp, _vp, _vp, ctypes.c_int64, _i32, _vp, _vp, _vp, _i32, _vp]),
     "hexb_copy_games": (_i32, [_vp, _vp, _vp, _vp, ctypes.c_int64, _vp]),
     "hexb_playouts": (_i32, [_vp, _i32, ctypes.c_int64, _vp, _vp, _vp]),
+    "hexb_playouts_policy": (_i32, [_vp, _i32, ctypes.c_int64, _i32, _vp, _vp, _vp]),
     "hexb_mcts_tree_bytes": (_i32, [_vp, _i32, ctypes.POINTER(_sz)]),
     "hexb_mcts_init": (_i32, [_vp, _vp, _sz, _i32, ctypes.c_double, ctypes.c_double, ctypes.c_int64, _vp, _vp]),
     "hexb_mcts_search": (_i32, [_vp, _vp, _sz, _i32, _i32, _vp]),
+    "hexb_mcts_search_policy": (_i32, [_vp, _vp, _sz, _i32, _i32, _i32, _vp]),
     "hexb_mcts_select": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp, _vp]),
     "hexb_mcts_expand": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp]),
     "hexb_mcts_root": (_i32, [_vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp]),

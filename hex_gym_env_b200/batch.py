@@ -16,7 +16,7 @@ What each method replaces in the reference (MBPrdctns/hex_gym_env, paths relativ
   export_state()     attribute reads .board / .regions / .region_counter / .current_player_num / .done / .winner
   import_boards()    HexGame.__init__ with a preset board (HexGame.py:53-61, HexSingleGame.py:57-65)
   copy_games()       copy.deepcopy(env.simulator) into a raw batch (tree search: branching a position)
-  playouts()         random playouts to the end from the current position (tree search: Monte-Carlo value estimates)
+  playouts()         random or bridge-reply playouts to the end from the current position (tree search: Monte-Carlo values)
 """
 import ctypes
 import os
@@ -29,6 +29,8 @@ from ._native import HexbConfig, check
 VARIANT_A = 0  # minihex/HexGame.py
 VARIANT_B = 1  # minihex/HexSingleGame.py + minihex/SelfplayWrapper.py
 AGENT_BLACK, AGENT_WHITE, AGENT_RANDOM = 0, 1, 2
+PLAYOUT_RANDOM = 0  # playouts: random_policy for both sides (include/hexb.h, HEXB_PLAYOUT_RANDOM)
+PLAYOUT_BRIDGE = 1  # playouts: answer an intrusion into a two-bridge of the mover in its other carrier cell (HEXB_PLAYOUT_BRIDGE)
 
 STAT_NAMES = ("episodes", "black_wins", "white_wins", "agent_wins", "episode_plies", "invalid_ends", "env_steps", "plies")
 COMPRESSIBLE_MIN_BYTES = 8 << 20   # smaller buffers stay with torch's allocator even when the object uses compressible memory
@@ -37,6 +39,13 @@ COMPRESSIBLE_MIN_BYTES = 8 << 20   # smaller buffers stay with torch's allocator
 def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
+
+
+def _playout_policy(policy):
+    """PLAYOUT_RANDOM or PLAYOUT_BRIDGE as an int; ValueError for anything else."""
+    if isinstance(policy, bool) or policy not in (PLAYOUT_RANDOM, PLAYOUT_BRIDGE):
+        raise ValueError("policy must be PLAYOUT_RANDOM (0) or PLAYOUT_BRIDGE (1), got %r" % (policy,))
+    return int(policy)
 
 class HexBatch(object):
     def __init__(self, board_size, num_games, variant=VARIANT_B, device=None, seed=0, game_offset=0,
@@ -558,17 +567,20 @@ class HexBatch(object):
         with torch.cuda.device(self.device):
             check(self._lib.hexb_copy_games(self._h, src._h, _ptr(si), _ptr(di), count, self._stream()))
 
-    def playouts(self, num_playouts, first_playout=0, game_mask=None, out=None):
-        """num_playouts random playouts per game from its current position (random_policy for both sides, filled to the end);
-        returns int32[G]: playouts won by the side to move, -1 for finished, never-reset and masked-off (game_mask u8[G] == 0)
-        games. Playout p uses its own stream (Philox counter c3 = p + 1), p in [first_playout, first_playout + num_playouts)."""
+    def playouts(self, num_playouts, first_playout=0, game_mask=None, out=None, policy=PLAYOUT_RANDOM):
+        """num_playouts playouts per game from its current position, filled to the end; returns int32[G]: playouts won by the
+        side to move, -1 for finished, never-reset and masked-off (game_mask u8[G] == 0) games. Playout p uses its own stream
+        (Philox counter c3 = p + 1), p in [first_playout, first_playout + num_playouts). policy: PLAYOUT_RANDOM (random_policy for
+        both sides) or PLAYOUT_BRIDGE (the same draws; a ply answers an intrusion into one of its side's bridges in the other
+        carrier cell, include/hexb.h)."""
         num_playouts, first_playout = int(num_playouts), int(first_playout)
         if num_playouts < 1 or first_playout < 0 or first_playout + num_playouts >= 1 << 32:
             raise ValueError("need num_playouts >= 1, first_playout >= 0 and first_playout + num_playouts < 2**32")
+        policy = _playout_policy(policy)
         gm = self._in(game_mask, (self.G,), torch.uint8, "game_mask")
         out = self._chk(out, (self.G,), torch.int32, "out") if out is not None else torch.empty(self.G, dtype=torch.int32, device=self.device)
         with torch.cuda.device(self.device):
-            check(self._lib.hexb_playouts(self._h, num_playouts, first_playout, _ptr(gm), _ptr(out), self._stream()))
+            check(self._lib.hexb_playouts_policy(self._h, num_playouts, first_playout, policy, _ptr(gm), _ptr(out), self._stream()))
         return out
 
     def opponent_catch_up(self):

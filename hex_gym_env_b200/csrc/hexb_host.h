@@ -49,7 +49,7 @@ enum : int { MCTS_INIT = 0, MCTS_SEARCH, MCTS_SELECT, MCTS_EXPAND, MCTS_ROOT, MC
     HEXB_LOCAL int hexb_launch_sample_##n(const hexb::View &V, int view, const double *u, int32_t *out, cudaStream_t s);     \
     HEXB_LOCAL int hexb_launch_import_##n(const hexb::Params &P, const int8_t *board_true, const int8_t *to_move,           \
                                           const uint8_t *import_mask, cudaStream_t s);                                      \
-    HEXB_LOCAL int hexb_launch_playouts_##n(const hexb::View &V, const hexb::PlayoutArgs &A, cudaStream_t s);             \
-    HEXB_LOCAL int hexb_launch_mcts_##n(int op, const hexb::View &V, const hexb::MctsArgs &A, cudaStream_t s);
+    HEXB_LOCAL int hexb_launch_playouts_##n(const hexb::View &V, const hexb::PlayoutArgs &A, int policy, cudaStream_t s);  \
+    HEXB_LOCAL int hexb_launch_mcts_##n(int op, const hexb::View &V, const hexb::MctsArgs &A, int policy, cudaStream_t s);
 HEXB_FOR_N(HEXB_DECL_N)
 #undef HEXB_DECL_N

@@ -14,7 +14,7 @@
 //   K9        hexb_gae_kernel         GAE(lambda) advantages / returns over a [T,G] rollout (SB3 RolloutBuffer semantics)
 //   K10       hexb_pack_obs_kernel    2-bit observation transport for hexb_step_host_packed
 //   K11       hexb_copy_kernel        copy.deepcopy(env.simulator) into a raw batch, one warp per copied game (hexb_search.cuh)
-//   K12       hexb_playout_kernel<N>  random playouts from the current position, one warp per game (hexb_step_inst.cu)
+//   K12       hexb_playout_kernel<N, policy>  random or bridge-reply playouts from the current position, one warp per game (hexb_step_inst.cu)
 //   K13       hexb_mcts_*_kernel<N>   batched PUCT tree search: init, fused search, select, expand, root readout, advance (hexb_mcts.cuh)
 #include <cuda.h>   // types of the driver's virtual-memory API only (entry points come from cudaGetDriverEntryPoint)
 #include <cuda_runtime.h>
@@ -242,11 +242,11 @@ static const sample_fn k_sample[] = {HEXB_FOR_N(X)};
 #define X(n) hexb_launch_import_##n,
 static const import_fn k_import[] = {HEXB_FOR_N(X)};
 #undef X
-typedef int (*mcts_fn)(int, const View &, const MctsArgs &, cudaStream_t);
+typedef int (*mcts_fn)(int, const View &, const MctsArgs &, int, cudaStream_t);
 #define X(n) hexb_launch_mcts_##n,
 static const mcts_fn k_mcts[] = {HEXB_FOR_N(X)};
 #undef X
-typedef int (*playouts_fn)(const View &, const PlayoutArgs &, cudaStream_t);
+typedef int (*playouts_fn)(const View &, const PlayoutArgs &, int, cudaStream_t);
 #define X(n) hexb_launch_playouts_##n,
 static const playouts_fn k_playouts[] = {HEXB_FOR_N(X)};
 #undef X
@@ -280,7 +280,7 @@ extern "C" HEXB_LOCAL void hexb_hostpack_finish(int abort);
 
 extern "C" {
 
-int32_t hexb_version(void) { return (1 << 16) | 5; }   // 1.3: obs_dtype, launch forms, hexb_gae, packed / asynchronous host step (+ hexb_mem_alloc: additive); 1.4: hexb_set_eval, hexb_set_opponent_eps; 1.5: hexb_copy_games, hexb_playouts
+int32_t hexb_version(void) { return (1 << 16) | 5; }   // 1.3: obs_dtype, launch forms, hexb_gae, packed / asynchronous host step (+ hexb_mem_alloc: additive); 1.4: hexb_set_eval, hexb_set_opponent_eps; 1.5: hexb_copy_games, hexb_playouts (+ hexb_mcts_*, hexb_playouts_policy, hexb_mcts_search_policy: additive)
 
 const char *hexb_strerror(int32_t code) {
     switch (code) {
@@ -934,9 +934,19 @@ int32_t hexb_copy_games(hexb_env *dst, const hexb_env *src, const int64_t *src_i
     return HEXB_OK;
 }
 
+static_assert(HEXB_PLAYOUT_RANDOM == PLAYOUT_RANDOM && HEXB_PLAYOUT_BRIDGE == PLAYOUT_BRIDGE, "playout policy codes");
+
+static bool playout_policy_ok(int32_t policy) { return policy >= 0 && policy < PLAYOUT_POLICIES; }
+
 int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout, const uint8_t *game_mask, int32_t *wins,
                       void *stream) {
+    return hexb_playouts_policy(env, num_playouts, first_playout, HEXB_PLAYOUT_RANDOM, game_mask, wins, stream);
+}
+
+int32_t hexb_playouts_policy(hexb_env *env, int32_t num_playouts, int64_t first_playout, int32_t policy, const uint8_t *game_mask,
+                             int32_t *wins, void *stream) {
     if (!env || !wins || num_playouts < 1 || first_playout < 0 || first_playout + (int64_t)num_playouts >= (1ll << 32)) return HEXB_ERR_ARG;
+    if (!playout_policy_ok(policy)) return HEXB_ERR_ARG;
     CK(cudaSetDevice(env->cfg.device));
     const View V = view_of(env);
     PlayoutArgs A;
@@ -946,7 +956,7 @@ int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout
     A.num = num_playouts;
     A.game_mask = game_mask;
     A.wins = wins;
-    return k_playouts[V.N - HEXB_MIN_BOARD](V, A, (cudaStream_t)stream);
+    return k_playouts[V.N - HEXB_MIN_BOARD](V, A, policy, (cudaStream_t)stream);
 }
 
 // ---- tree search (hexb_mcts.cuh). The host checks the arguments; the kernels check the tree header init wrote, so that no
@@ -963,10 +973,10 @@ static MctsArgs mcts_args(const hexb_env *env, const void *tree, size_t tree_byt
     return A;
 }
 
-static int mcts_launch(const hexb_env *env, int op, const MctsArgs &A, void *stream) {
+static int mcts_launch(const hexb_env *env, int op, const MctsArgs &A, void *stream, int policy = HEXB_PLAYOUT_RANDOM) {
     CK(cudaSetDevice(env->cfg.device));
     const View V = view_of(env);
-    return k_mcts[V.N - HEXB_MIN_BOARD](op, V, A, (cudaStream_t)stream);
+    return k_mcts[V.N - HEXB_MIN_BOARD](op, V, A, policy, (cudaStream_t)stream);
 }
 
 int32_t hexb_mcts_tree_bytes(const hexb_env *env, int32_t max_nodes, size_t *bytes) {
@@ -995,12 +1005,18 @@ int32_t hexb_mcts_init(const hexb_env *env, void *tree, size_t tree_bytes, int32
 
 int32_t hexb_mcts_search(const hexb_env *env, void *tree, size_t tree_bytes, int32_t num_simulations, int32_t playouts_per_leaf,
                          void *stream) {
+    return hexb_mcts_search_policy(env, tree, tree_bytes, num_simulations, playouts_per_leaf, HEXB_PLAYOUT_RANDOM, stream);
+}
+
+int32_t hexb_mcts_search_policy(const hexb_env *env, void *tree, size_t tree_bytes, int32_t num_simulations, int32_t playouts_per_leaf,
+                                int32_t policy, void *stream) {
     if (!env || num_simulations < 1 || playouts_per_leaf < 1 || playouts_per_leaf > kMctsMaxPlayouts) return HEXB_ERR_ARG;
+    if (!playout_policy_ok(policy)) return HEXB_ERR_ARG;
     if (!mcts_buffer_ok(tree, tree_bytes)) return HEXB_ERR_STATE;
     MctsArgs A = mcts_args(env, tree, tree_bytes);
     A.sims = num_simulations;
     A.playouts = playouts_per_leaf;
-    return mcts_launch(env, MCTS_SEARCH, A, stream);
+    return mcts_launch(env, MCTS_SEARCH, A, stream, policy);
 }
 
 int32_t hexb_mcts_select(const hexb_env *env, void *tree, size_t tree_bytes, void *leaf_obs, uint8_t *leaf_mask, uint8_t *pending,

@@ -382,8 +382,9 @@ HEXB_HD void mc_init_root(const View &V, const MctsArgs &A, long long g) {
     mc_fresh_root<N>(T, g, to_move, black, empty);
 }
 
-// fused form: all simulations of one root (one warp)
-template <int N>
+// fused form: all simulations of one root (one warp), playouts of policy POLICY; a leaf at depth >= 1 gives its playouts the move
+// into it as the move before ply 0
+template <int N, int POLICY = PLAYOUT_RANDOM>
 HEXB_HD void mc_search_root(const Tree &T, const MctsArgs &A, int variant, long long g) {
     int32_t *m = mc_meta(T, g);
     if (!m[MM_ACTIVE]) return;
@@ -404,7 +405,7 @@ HEXB_HD void mc_search_root(const Tree &T, const MctsArgs &A, int variant, long 
             const uint32_t p0 = (uint32_t)T.first + s * (uint32_t)P;
             int won = 0;
             for (int j = mc_lane(); j < P; j += mc_width())
-                won += playout_winner<N>(black, empty, mover, A.seed, gid, p0 + (uint32_t)j) == mover;
+                won += playout_winner<N, POLICY>(black, empty, mover, A.seed, gid, p0 + (uint32_t)j, L.depth >= 1 ? L.cell : -1) == mover;
             won = mc_sum(won);
             v = f_div((float)(2 * won - P), (float)P);
         }

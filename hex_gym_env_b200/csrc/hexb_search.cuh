@@ -165,11 +165,56 @@ HEXB_HD int nth_set_bit(uint32_t z, int k) {
     return pos;
 }
 
-// One playout from rows (black0, empty0) with true colour `to_move` first; returns the winning true colour (0 BLACK, 1 WHITE).
-// Rows are selected by unrolled compare-and-mask, never by a run-time index, so that the arrays stay in registers.
+// Playout policies (include/hexb.h, HEXB_PLAYOUT_*): the kernels that run playouts are instantiated once per policy.
+enum : int { PLAYOUT_RANDOM = 0, PLAYOUT_BRIDGE = 1, PLAYOUT_POLICIES = 2 };
+
+// Bridge replies of `mover` to the opponent's move prev = (py, px) (include/hexb.h, HEXB_PLAYOUT_BRIDGE). The rows py - 1, py,
+// py + 1 are gathered by an unrolled mask-and-or over all rows and cut to 3-bit windows over the columns px - 1 .. px + 1
+// (bit 0 = px - 1), so that the six directions are shifts: o = the points that are the mover's (off-board points of the mover's edges included),
+// e = the empty cells. r[j]: the replies in row py - 1 + j as window bits. No prev (py far off the board): every e is 0.
 template <int N>
+HEXB_HD void bridge_replies(const uint32_t (&black)[N], const uint32_t (&empty)[N], int mover, int py, int px, uint32_t (&r)[3]) {
+    const uint32_t full = (1u << N) - 1u;
+    // row y is selected through bits of a one-hot row mask, not by comparing y with py: compared, the compiler turns the selects
+    // back into an indexed load and moves the rows to local memory
+    const uint32_t at = (uint32_t)py < (uint32_t)N ? 1u << py : 0u;
+    uint32_t b[3] = {0u, 0u, 0u}, em[3] = {0u, 0u, 0u};
+#pragma unroll
+    for (int y = 0; y < N; ++y) {
+        const uint32_t up = 0u - ((at >> (y + 1)) & 1u), mid = 0u - ((at >> y) & 1u), down = 0u - (((at << 1) >> y) & 1u);
+        b[0] |= black[y] & up;
+        b[1] |= black[y] & mid;
+        b[2] |= black[y] & down;
+        em[0] |= empty[y] & up;
+        em[1] |= empty[y] & mid;
+        em[2] |= empty[y] & down;
+    }
+    uint32_t o[3], e[3];
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+        const int y = py - 1 + j;
+        // bit x + 1 = point (y, x), x = -1 .. N: BLACK owns the rows beyond its edges, WHITE the columns -1 and N of the board
+        const uint32_t own = (y >= 0 && y < N) ? (((mover == 0 ? b[j] : ~(b[j] | em[j]) & full) << 1) | (mover == 0 ? 0u : 1u | (2u << N)))
+                                               : (mover == 0 ? full << 1 : 0u);
+        o[j] = (own >> px) & 7u;
+        e[j] = ((em[j] << 1) >> px) & 7u;
+    }
+    // e = prev + D[i] with both prev + D[i - 1] and prev + D[i + 1] the mover's, D = (-1,0) (-1,1) (0,1) (1,0) (1,-1) (0,-1)
+    r[0] = e[0] & ((((o[1] & (o[0] >> 2)) & 1u) << 1) |            // D[0] (-1, 0): carriers (0, -1), (-1, 1)
+                   ((((o[0] >> 1) & (o[1] >> 2)) & 1u) << 2));     // D[1] (-1, 1): carriers (-1, 0), (0, 1)
+    r[1] = e[1] & (((o[2] & (o[0] >> 1)) & 1u) |                   // D[5] (0, -1): carriers (1, -1), (-1, 0)
+                   ((((o[0] >> 2) & (o[2] >> 1)) & 1u) << 2));     // D[2] (0, 1): carriers (-1, 1), (1, 0)
+    r[2] = e[2] & ((((o[2] >> 1) & o[1]) & 1u) |                   // D[4] (1, -1): carriers (1, 0), (0, -1)
+                   ((((o[1] >> 2) & o[2]) & 1u) << 1));            // D[3] (1, 0): carriers (0, 1), (1, -1)
+}
+
+// One playout from rows (black0, empty0) with true colour `to_move` first; returns the winning true colour (0 BLACK, 1 WHITE).
+// Rows are selected by unrolled compare-and-mask, never by a run-time index, so that the arrays stay in registers. PLAYOUT_BRIDGE:
+// a ply whose bridge reply set is not empty plays its choice_of(u, |R|)-th cell in row-major order instead; prev is the true cell
+// of the move before ply 0 (-1 = none). PLAYOUT_RANDOM ignores prev.
+template <int N, int POLICY = PLAYOUT_RANDOM>
 HEXB_HD int playout_winner(const uint32_t (&black0)[N], const uint32_t (&empty0)[N], int to_move, unsigned long long seed,
-                           unsigned long long game, uint32_t p) {
+                           unsigned long long game, uint32_t p, int prev = -1) {
     uint32_t black[N], empty[N];
     int n = 0;
 #pragma unroll
@@ -178,8 +223,10 @@ HEXB_HD int playout_winner(const uint32_t (&black0)[N], const uint32_t (&empty0)
         empty[y] = empty0[y];
         n += popc32(empty0[y]);
     }
+    int py = prev < 0 ? -8 : prev / N, px = prev < 0 ? 0 : prev - py * N;   // -8: no row of the window is on the board
     for (uint32_t k = 0; n > 0; ++k, --n) {
-        int left = choice_of(playout_draw(seed, game, k, p), n);
+        const double u = playout_draw(seed, game, k, p);
+        int left = choice_of(u, n);
         uint32_t z = 0u;
         int row = -1, kk = 0;
 #pragma unroll
@@ -188,7 +235,20 @@ HEXB_HD int playout_winner(const uint32_t (&black0)[N], const uint32_t (&empty0)
             if (row < 0 && left < c) { row = y; z = empty[y]; kk = left; }
             left -= c;
         }
-        const uint32_t bit = 1u << nth_set_bit(z, kk);
+        int col = nth_set_bit(z, kk);
+        if constexpr (POLICY == PLAYOUT_BRIDGE) {   // a reply, if there is one, replaces the random cell
+            uint32_t r[3];
+            bridge_replies<N>(black, empty, (k & 1u) ? 1 - to_move : to_move, py, px, r);
+            const int c0 = popc32(r[0]), c1 = popc32(r[1]), nr = c0 + c1 + popc32(r[2]);
+            if (nr > 0) {
+                const int i = choice_of(u, nr), j = i < c0 ? 0 : (i < c0 + c1 ? 1 : 2);
+                row = py - 1 + j;
+                col = px - 1 + nth_set_bit(j == 0 ? r[0] : (j == 1 ? r[1] : r[2]), i - (j == 0 ? 0 : (j == 1 ? c0 : c0 + c1)));
+            }
+            py = row;
+            px = col;
+        }
+        const uint32_t bit = 1u << col;
         const uint32_t bl = ((k & 1u) ? 1 - to_move : to_move) == 0 ? bit : 0u;
 #pragma unroll
         for (int y = 0; y < N; ++y) {

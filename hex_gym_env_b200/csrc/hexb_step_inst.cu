@@ -21,9 +21,9 @@ __global__ void hexb_import_kernel(Params P, const int8_t *board_true, const int
     if (g < P.G) import_game<N>(P, g, board_true, to_move, import_mask);
 }
 
-// hexb_playouts: one warp per game, lane l takes playouts first + l, first + l + 32, ... (every playout of a game fills the same
-// number of cells, so the lanes stay converged until the connectivity test)
-template <int N>
+// hexb_playouts_policy: one warp per game, lane l takes playouts first + l, first + l + 32, ... (every playout of a game fills the
+// same number of cells, so the lanes stay converged until the connectivity test)
+template <int N, int POLICY>
 __global__ void __launch_bounds__(256) hexb_playout_kernel(View V, PlayoutArgs A) {
     const int lane = threadIdx.x & 31;
     const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -37,7 +37,7 @@ __global__ void __launch_bounds__(256) hexb_playout_kernel(View V, PlayoutArgs A
     const unsigned long long gid = A.game_offset + (unsigned long long)g;
     int won = 0;
     for (int j = lane; j < A.num; j += 32)
-        won += playout_winner<N>(black, empty, to_move, A.seed, gid, (uint32_t)(A.first + j)) == to_move;
+        won += playout_winner<N, POLICY>(black, empty, to_move, A.seed, gid, (uint32_t)(A.first + j), -1) == to_move;
     won = __reduce_add_sync(0xffffffffu, won);
     if (lane == 0) A.wins[g] = won;
 }
@@ -50,12 +50,13 @@ __global__ void __launch_bounds__(128) hexb_mcts_init_kernel(View V, MctsArgs A)
     if (g == 0) mc_write_header(A, N, V.G);
     if (g < V.G) mc_init_root<N>(V, A, g);
 }
-// 168 registers: the path rows, the playout's own copy and the selection state without a spill at N = 19 (ptxas -v)
-template <int N>
+// 168 registers: the path rows, the playout's own copy and the selection state without a spill at N = 19 (ptxas -v), for both
+// playout policies
+template <int N, int POLICY>
 __global__ void __maxnreg__(168) hexb_mcts_search_kernel(View V, MctsArgs A) {
     const long long g = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     Tree T;
-    if (g < V.G && mc_tree(A, N, V.G, T)) mc_search_root<N>(T, A, V.variant, g);
+    if (g < V.G && mc_tree(A, N, V.G, T)) mc_search_root<N, POLICY>(T, A, V.variant, g);
 }
 template <int N>
 __global__ void __launch_bounds__(128) hexb_mcts_select_kernel(View V, MctsArgs A) {
@@ -101,17 +102,24 @@ int HEXB_CAT(hexb_launch_import_, HEXB_INST_N)(const Params &P, const int8_t *bo
     return HEXB_OK;
 }
 
-int HEXB_CAT(hexb_launch_playouts_, HEXB_INST_N)(const View &V, const PlayoutArgs &A, cudaStream_t s) {
-    hexb_playout_kernel<HEXB_INST_N><<<(unsigned)((V.G + 7) / 8), 256, 0, s>>>(V, A);
+// policy: PLAYOUT_RANDOM or PLAYOUT_BRIDGE (checked by the caller)
+int HEXB_CAT(hexb_launch_playouts_, HEXB_INST_N)(const View &V, const PlayoutArgs &A, int policy, cudaStream_t s) {
+    const unsigned blocks = (unsigned)((V.G + 7) / 8);
+    if (policy == PLAYOUT_BRIDGE) hexb_playout_kernel<HEXB_INST_N, PLAYOUT_BRIDGE><<<blocks, 256, 0, s>>>(V, A);
+    else hexb_playout_kernel<HEXB_INST_N, PLAYOUT_RANDOM><<<blocks, 256, 0, s>>>(V, A);
     CK(cudaGetLastError());
     return HEXB_OK;
 }
 
-int HEXB_CAT(hexb_launch_mcts_, HEXB_INST_N)(int op, const View &V, const MctsArgs &A, cudaStream_t s) {
+// policy: the fused search's playout policy (MCTS_SEARCH only)
+int HEXB_CAT(hexb_launch_mcts_, HEXB_INST_N)(int op, const View &V, const MctsArgs &A, int policy, cudaStream_t s) {
     const unsigned warps = (unsigned)((V.G + 3) / 4), threads = (unsigned)((V.G + 127) / 128);
     switch (op) {
         case MCTS_INIT: hexb_mcts_init_kernel<HEXB_INST_N><<<threads, 128, 0, s>>>(V, A); break;
-        case MCTS_SEARCH: hexb_mcts_search_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
+        case MCTS_SEARCH:
+            if (policy == PLAYOUT_BRIDGE) hexb_mcts_search_kernel<HEXB_INST_N, PLAYOUT_BRIDGE><<<warps, 128, 0, s>>>(V, A);
+            else hexb_mcts_search_kernel<HEXB_INST_N, PLAYOUT_RANDOM><<<warps, 128, 0, s>>>(V, A);
+            break;
         case MCTS_SELECT: hexb_mcts_select_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
         case MCTS_EXPAND: hexb_mcts_expand_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;
         case MCTS_ROOT: hexb_mcts_root_kernel<HEXB_INST_N><<<warps, 128, 0, s>>>(V, A); break;

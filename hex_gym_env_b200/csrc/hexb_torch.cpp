@@ -172,13 +172,15 @@ void op_copy_games(int64_t dst, int64_t src, OptT src_index, OptT dst_index, int
              "copy_games");
 }
 
-void op_playouts(int64_t handle, int64_t num_playouts, int64_t first_playout, OptT game_mask, Tensor wins) {
+void op_playouts(int64_t handle, int64_t num_playouts, int64_t first_playout, OptT game_mask, Tensor wins, int64_t policy) {
     Call k(handle);
     const int d = k.c.device;
     TORCH_CHECK(num_playouts >= 1 && num_playouts <= INT32_MAX && first_playout >= 0 && first_playout + num_playouts < (1ll << 32),
                 "hexb::playouts: need num_playouts >= 1, first_playout >= 0 and first_playout + num_playouts < 2^32");
-    check_rc(hexb_playouts(k.e, (int32_t)num_playouts, first_playout, ptr<const uint8_t>(game_mask, at::kByte, k.G, d, "game_mask"),
-                           ptr<int32_t>(wins, at::kInt, k.G, d, "wins"), k.stream),
+    TORCH_CHECK(policy == HEXB_PLAYOUT_RANDOM || policy == HEXB_PLAYOUT_BRIDGE, "hexb::playouts: policy must be 0 (random) or 1 (bridge)");
+    check_rc(hexb_playouts_policy(k.e, (int32_t)num_playouts, first_playout, (int32_t)policy,
+                                  ptr<const uint8_t>(game_mask, at::kByte, k.G, d, "game_mask"), ptr<int32_t>(wins, at::kInt, k.G, d, "wins"),
+                                  k.stream),
              "playouts");
 }
 
@@ -198,12 +200,13 @@ void op_mcts_init(int64_t handle, Tensor tree, int64_t max_nodes, double c_puct,
              "mcts_init");
 }
 
-void op_mcts_search(int64_t handle, Tensor tree, int64_t num_simulations, int64_t playouts_per_leaf) {
+void op_mcts_search(int64_t handle, Tensor tree, int64_t num_simulations, int64_t playouts_per_leaf, int64_t policy) {
     Call k(handle);
     TORCH_CHECK(num_simulations >= 1 && num_simulations <= INT32_MAX && playouts_per_leaf >= 1 && playouts_per_leaf <= INT32_MAX,
                 "hexb::mcts_search: num_simulations and playouts_per_leaf must be >= 1");
-    check_rc(hexb_mcts_search(k.e, tree_of(tree, k.c.device), (size_t)tree.numel(), (int32_t)num_simulations, (int32_t)playouts_per_leaf,
-                              k.stream),
+    TORCH_CHECK(policy == HEXB_PLAYOUT_RANDOM || policy == HEXB_PLAYOUT_BRIDGE, "hexb::mcts_search: policy must be 0 (random) or 1 (bridge)");
+    check_rc(hexb_mcts_search_policy(k.e, tree_of(tree, k.c.device), (size_t)tree.numel(), (int32_t)num_simulations,
+                                     (int32_t)playouts_per_leaf, (int32_t)policy, k.stream),
              "mcts_search");
 }
 
@@ -262,9 +265,9 @@ TORCH_LIBRARY(hexb, m) {
     m.def("set_launch_form(int env, int warps_per_chunk) -> ()", &op_set_launch_form);
     m.def("set_eval(int env, bool eval_state, Tensor(a!)? eval_episode) -> ()");
     m.def("copy_games(int dst, int src, Tensor? src_index, Tensor? dst_index, int count) -> ()");
-    m.def("playouts(int env, int num_playouts, int first_playout, Tensor? game_mask, Tensor(a!) wins) -> ()");
+    m.def("playouts(int env, int num_playouts, int first_playout, Tensor? game_mask, Tensor(a!) wins, int policy=0) -> ()");
     m.def("mcts_init(int env, Tensor(a!) tree, int max_nodes, float c_puct, float fpu, int first_playout, Tensor? root_mask) -> ()");
-    m.def("mcts_search(int env, Tensor(a!) tree, int num_simulations, int playouts_per_leaf) -> ()");
+    m.def("mcts_search(int env, Tensor(a!) tree, int num_simulations, int playouts_per_leaf, int policy=0) -> ()");
     m.def("mcts_select(int env, Tensor(a!) tree, Tensor(b!) leaf_obs, Tensor(c!) leaf_mask, Tensor(d!) pending) -> ()");
     m.def("mcts_expand(int env, Tensor(a!) tree, Tensor priors, Tensor values) -> ()");
     m.def("mcts_root(int env, Tensor tree, Tensor(a!)? visits, Tensor(b!)? q, Tensor(c!)? value, Tensor(d!)? nodes_used) -> ()");

@@ -252,6 +252,25 @@ int32_t hexb_copy_games(hexb_env *dst, const hexb_env *src, const int64_t *src_i
 int32_t hexb_playouts(hexb_env *env, int32_t num_playouts, int64_t first_playout, const uint8_t *game_mask, int32_t *wins,
                       void *stream);
 
+/* Playout policies. Both play the same plies with the same draws u; they differ only in the cell a ply takes.
+ * HEXB_PLAYOUT_RANDOM: the playout above (hexb_playouts).
+ * HEXB_PLAYOUT_BRIDGE: save bridges. D = ((-1,0), (-1,1), (0,1), (1,0), (1,-1), (0,-1)) lists the six neighbours (dy, dx) of a
+ *   cell in cyclic order; the common neighbours of c and c + D[i] are c + D[i-1] and c + D[i+1] (indices mod 6). A point is
+ *   colour m's if it is on the board and holds a stone of m, or if it is off the board on m's side: BLACK owns the points with
+ *   y < 0 or y >= N and 0 <= x < N, WHITE the points with x < 0 or x >= N and 0 <= y < N; no one owns the other off-board points
+ *   (so a stone on the second row with both cells to its edge empty is bridged to the edge). At ply k with mover m and prev the
+ *   cell of ply k-1, the reply set R is every cell e = prev + D[i] that is on the board and empty and whose prev + D[i-1] and
+ *   prev + D[i+1] are both m's. If R is not empty, ply k plays the choice_of(u, |R|) = int(u * |R|)-th cell of R in true
+ *   row-major order; otherwise the int(u * n_empty)-th empty cell, as the random policy does. A ply with an empty R therefore
+ *   plays the cell the random policy would play on the same board. Ply 0 has no prev in hexb_playouts_policy (R is empty); in
+ *   hexb_mcts_search_policy a leaf at depth >= 1 uses the move into it (the path's last cell) and node 0 has none.
+ * Any other policy value: HEXB_ERR_ARG before any launch. */
+#define HEXB_PLAYOUT_RANDOM 0
+#define HEXB_PLAYOUT_BRIDGE 1
+/* hexb_playouts with playouts of `policy`; hexb_playouts is policy HEXB_PLAYOUT_RANDOM. */
+int32_t hexb_playouts_policy(hexb_env *env, int32_t num_playouts, int64_t first_playout, int32_t policy, const uint8_t *game_mask,
+                             int32_t *wins, void *stream);
+
 /* Batched Monte-Carlo tree search (PUCT), one tree per game g of `env` (any handle: raw, variant A or B env), in a device buffer
  * of hexb_mcts_tree_bytes(env, max_nodes) bytes (16-byte aligned; layout: csrc/hexb_mcts.cuh). Every call is asynchronous on
  * `stream`, allocates nothing and reads nothing on the host (CUDA-graph capturable). Bad max_nodes (1..2^24), num_simulations
@@ -294,6 +313,10 @@ int32_t hexb_mcts_init(const hexb_env *env, void *tree, size_t tree_bytes, int32
  * by search(b) equals search(a + b). */
 int32_t hexb_mcts_search(const hexb_env *env, void *tree, size_t tree_bytes, int32_t num_simulations, int32_t playouts_per_leaf,
                          void *stream);
+/* hexb_mcts_search with leaf playouts of `policy` (HEXB_PLAYOUT_*; hexb_mcts_search is HEXB_PLAYOUT_RANDOM). The policy is an
+ * argument of the call, not state of the tree: search(a) followed by search(b) equals search(a + b) under one policy. */
+int32_t hexb_mcts_search_policy(const hexb_env *env, void *tree, size_t tree_bytes, int32_t num_simulations, int32_t playouts_per_leaf,
+                                int32_t policy, void *stream);
 /* The split form, one simulation per select / expand pair (results are defined only when they alternate). select: step 1 for
  * every active root. A leaf that needs an evaluation gets leaf_obs[g] (obs_dtype [G,N,N]) and leaf_mask[g] (u8 [G,C]) - what
  * hexb_encode(view 1) returns for a raw game of the same variant holding the leaf - and pending[g] = 1 (u8 [G]); a terminal

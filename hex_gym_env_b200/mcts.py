@@ -5,6 +5,7 @@
     tree = MCTS(env, max_nodes=801)
     tree.reset()
     tree.search(800, 8)                         # fused form: 800 simulations with 8 playouts per leaf, one launch
+    tree.search(800, 8, policy=PLAYOUT_BRIDGE)  # ... with playouts that save bridges (include/hexb.h, HEXB_PLAYOUT_BRIDGE)
     visits, q, value, nodes_used = tree.root()
 
     tree.reset()                                # split form: a policy / value network evaluates the leaves
@@ -25,7 +26,7 @@ import ctypes
 import torch
 
 from ._native import check
-from .batch import HexBatch, _ptr
+from .batch import PLAYOUT_RANDOM, HexBatch, _playout_policy, _ptr
 
 
 class MCTS(object):
@@ -68,14 +69,18 @@ class MCTS(object):
                                            self.c_puct, self.fpu, first_playout, _ptr(rm), self.batch._stream()))
         self._ready = True
 
-    def search(self, num_simulations, playouts_per_leaf):
-        """num_simulations simulations for every active root with playouts_per_leaf random playouts per leaf, in one launch."""
+    def search(self, num_simulations, playouts_per_leaf, policy=PLAYOUT_RANDOM):
+        """num_simulations simulations for every active root with playouts_per_leaf playouts per leaf, in one launch. policy:
+        PLAYOUT_RANDOM (uniform random playouts) or PLAYOUT_BRIDGE (playouts that save bridges; a leaf's first ply may answer the
+        move into the leaf). The policy belongs to the call, not to the tree: search(a) then search(b) equals search(a + b)
+        under one policy."""
         num_simulations, playouts_per_leaf = int(num_simulations), int(playouts_per_leaf)
         if not (1 <= num_simulations < 1 << 31 and 1 <= playouts_per_leaf <= 1 << 16):
             raise ValueError("need num_simulations >= 1 and 1 <= playouts_per_leaf <= 65536")
+        policy = _playout_policy(policy)
         h, t, nb = self._args()
         with torch.cuda.device(self.device):
-            check(self._lib.hexb_mcts_search(h, t, nb, num_simulations, playouts_per_leaf, self.batch._stream()))
+            check(self._lib.hexb_mcts_search_policy(h, t, nb, num_simulations, playouts_per_leaf, policy, self.batch._stream()))
 
     def select(self):
         """Step 1 of one simulation: (leaf_obs [G,N,N] obs_dtype, leaf_mask u8[G,C], pending u8[G]), encode(view 1) of each pending

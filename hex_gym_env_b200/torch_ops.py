@@ -14,6 +14,7 @@ torch headers to build.
     ops.playouts(children.handle, 64, 0, None, wins)
     ops.mcts_init(env.handle, tree, 801, 1.25, 0.0, 0, None)                    # tree: uint8[hexb_mcts_tree_bytes] (mcts.MCTS)
     ops.mcts_search(env.handle, tree, 800, 8)
+    ops.mcts_search(env.handle, tree, 800, 8, policy=1)                      # bridge playouts (PLAYOUT_BRIDGE)
 
 There is no CPU implementation behind the operators: they raise unless their tensors live on the handle's CUDA device.
 """
