@@ -40,8 +40,6 @@ HEXB_LOCAL int hexb_cuda_fail(cudaError_t e);   // records the code for hexb_las
         if (e_ != cudaSuccess) return hexb_cuda_fail(e_); \
     } while (0)
 
-enum : int { MCTS_INIT = 0, MCTS_SEARCH, MCTS_SELECT, MCTS_EXPAND, MCTS_ROOT, MCTS_ADVANCE };   // op of hexb_launch_mcts_<n>
-
 // per-board-size entry points, defined by hexb_step_inst.cu
 #define HEXB_FOR_N(X) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19)
 #define HEXB_DECL_N(n)                                                                                                      \

@@ -34,6 +34,7 @@ constexpr int kMctsMaxNodes = 1 << 24;          // visit counts stay exact in fl
 constexpr int kMctsMaxPlayouts = 1 << 16;
 enum : int { MF_UNEXPANDED = 0, MF_EXPANDED = 1, MF_TERMINAL = 2 };
 enum : int { MM_ACTIVE = 0, MM_USED, MM_SIMS, MM_VSUM, MM_TOMOVE, MM_PENDING, MM_DEPTH, MM_NODE, MM_PARENT, MM_CELL };
+enum : int { MCTS_INIT = 0, MCTS_SEARCH, MCTS_SELECT, MCTS_EXPAND, MCTS_ROOT, MCTS_ADVANCE };   // op of hexb_launch_mcts_<n>
 
 HEXB_HD long long mc_pad128(long long b) { return (b + 127) & ~127ll; }
 HEXB_HD int mc_cp(int N) { return (N * N + 31) & ~31; }

@@ -1,6 +1,8 @@
-"""TEST INFRASTRUCTURE ONLY - ctypes wrapper of the host emulator of the CUDA tile kernel (tests/emu/hexb_emu.cpp).
+"""TEST INFRASTRUCTURE ONLY - ctypes wrapper of the host emulator of the CUDA kernels (tests/emu/hexb_emu.cpp).
 
-Same method surface as oracle.hexref.RefBatch so that tests/parity.py can drive either side."""
+EmuBatch has the method surface of oracle.hexref.RefBatch, so that tests/parity.py can drive either side. copy_games, playouts and
+EmuMCTS emulate hexb_copy_games, hexb_playouts_policy and the hexb_mcts_* calls on EmuBatch handles; EmuMCTS has the method
+surface of hex_gym_env_b200.MCTS, and its tree is a host uint8 array in the layout of hex_gym_env_b200/csrc/hexb_mcts.cuh."""
 import ctypes
 import os
 import subprocess
@@ -10,14 +12,17 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(os.path.dirname(_HERE))
 _LIB = None
+POLICIES = (0, 1)   # PLAYOUT_RANDOM, PLAYOUT_BRIDGE
+MCTS_INIT, MCTS_SEARCH, MCTS_SELECT, MCTS_EXPAND, MCTS_ROOT, MCTS_ADVANCE = range(6)   # op of emu_mcts (csrc/hexb_mcts.cuh)
 
 
 def build(force=False):
     if os.environ.get("HEXB_EMU_LIB"):      # a prebuilt variant, e.g. the sanitizer build of tools/emu_sanitize.py
         return os.environ["HEXB_EMU_LIB"]
     so = os.path.join(_HERE, "libhexb_emu.so")
-    srcs = [os.path.join(_HERE, "hexb_emu.cpp")] + [os.path.join(_ROOT, "hex_gym_env_b200", "csrc", f)
-                                                     for f in ("hexb_core.cuh", "hexb_phases.cuh", "hexb_views.cuh")]
+    srcs = [os.path.join(_HERE, "hexb_emu.cpp")] + [
+        os.path.join(_ROOT, "hex_gym_env_b200", "csrc", f)
+        for f in ("hexb_core.cuh", "hexb_phases.cuh", "hexb_views.cuh", "hexb_search.cuh", "hexb_mcts.cuh")]
     if force or not os.path.exists(so) or os.path.getmtime(so) < max(os.path.getmtime(s) for s in srcs):
         subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-x", "c++", "-Wall", "-Wno-unknown-pragmas",
                                "-o", so, srcs[0]])
@@ -53,6 +58,11 @@ def lib():
         L.emu_draw01.argtypes = [u64, u64, ctypes.c_uint32]
         L.emu_encode_word.argtypes = [ctypes.c_uint32, i32, vp, vp]
         L.emu_encode_byte.argtypes = [ctypes.c_uint32, i32, vp, vp]
+        L.emu_copy_games.argtypes = [vp, vp, vp, vp, i64]
+        L.emu_playouts.argtypes = [vp, i32, i64, i32, vp, vp]
+        L.emu_mcts_tree_bytes.restype = i64
+        L.emu_mcts_tree_bytes.argtypes = [i32, i64, i32]
+        L.emu_mcts.argtypes = [vp, i32, vp, i64, i32, ctypes.c_double, ctypes.c_double, i64, vp, i32, i32, i32] + [vp] * 9
         _LIB = L
     return _LIB
 
@@ -195,3 +205,67 @@ class EmuBatch(object):
         out = np.zeros(8, np.int64)
         lib().emu_stats(self._h, _p(out))
         return out
+
+
+def copy_games(dst, src, src_index=None, dst_index=None, count=None):
+    """hexb_copy_games between two EmuBatch objects (dst raw, same N and variant)."""
+    si = None if src_index is None else np.ascontiguousarray(src_index, np.int64)
+    di = None if dst_index is None else np.ascontiguousarray(dst_index, np.int64)
+    if count is None:
+        count = len(si) if si is not None else (len(di) if di is not None else min(dst.G, src.G))
+    lib().emu_copy_games(dst._h, src._h, _p(si), _p(di), int(count))
+
+
+def _policy(policy):
+    if policy not in POLICIES:
+        raise ValueError("policy must be 0 (random) or 1 (bridge)")
+    return int(policy)
+
+
+def playouts(batch, num_playouts, first_playout=0, game_mask=None, policy=0):
+    """hexb_playouts_policy on an EmuBatch: wins i32[G]."""
+    policy = _policy(policy)
+    wins = np.empty(batch.G, np.int32)
+    gm = None if game_mask is None else np.ascontiguousarray(game_mask, np.uint8)
+    lib().emu_playouts(batch._h, int(num_playouts), int(first_playout), policy, _p(gm), _p(wins))
+    return wins
+
+
+class EmuMCTS(object):
+    """hexb_mcts_* on an EmuBatch, with the method surface of hex_gym_env_b200.MCTS (numpy in and out)."""
+
+    def __init__(self, batch, max_nodes, c_puct=1.25, fpu=0.0):
+        self.batch, self.max_nodes, self.c_puct, self.fpu = batch, int(max_nodes), float(c_puct), float(fpu)
+        self.tree = np.zeros(int(lib().emu_mcts_tree_bytes(batch.N, batch.G, self.max_nodes)), np.uint8)
+
+    def _call(self, op, first_playout=0, root_mask=None, sims=0, playouts=0, policy=0, **out):
+        ptrs = [_p(out.get(k)) for k in ("leaf_obs", "leaf_mask", "pending", "priors", "values", "visits", "q", "value", "nodes_used")]
+        lib().emu_mcts(self.batch._h, op, _p(self.tree), self.tree.size, self.max_nodes, self.c_puct, self.fpu, int(first_playout),
+                       _p(root_mask), int(sims), int(playouts), policy, *ptrs)
+
+    def reset(self, root_mask=None, first_playout=0):
+        rm = None if root_mask is None else np.ascontiguousarray(root_mask, np.uint8)
+        self._call(MCTS_INIT, first_playout, rm)
+
+    def search(self, num_simulations, playouts_per_leaf, policy=0):
+        self._call(MCTS_SEARCH, sims=num_simulations, playouts=playouts_per_leaf, policy=_policy(policy))
+
+    def select(self):
+        G, N, C = self.batch.G, self.batch.N, self.batch.C
+        obs, mask, pending = np.zeros((G, N, N), np.int8), np.zeros((G, C), np.uint8), np.zeros(G, np.uint8)
+        self._call(MCTS_SELECT, leaf_obs=obs, leaf_mask=mask, pending=pending)
+        return obs, mask, pending
+
+    def expand(self, priors, values):
+        self._call(MCTS_EXPAND, priors=np.ascontiguousarray(priors, np.float32), values=np.ascontiguousarray(values, np.float32))
+
+    def root(self):
+        G, C = self.batch.G, self.batch.C
+        out = dict(visits=np.zeros((G, C), np.int32), q=np.zeros((G, C), np.float32), value=np.zeros(G, np.float32),
+                   nodes_used=np.zeros(G, np.int32))
+        self._call(MCTS_ROOT, **out)
+        return out["visits"], out["q"], out["value"], out["nodes_used"]
+
+    def advance(self, root_mask=None, first_playout=0):
+        rm = None if root_mask is None else np.ascontiguousarray(root_mask, np.uint8)
+        self._call(MCTS_ADVANCE, first_playout, rm)

@@ -1,18 +1,22 @@
-// TEST INFRASTRUCTURE ONLY - host-side emulator of the CUDA step kernel.
+// TEST INFRASTRUCTURE ONLY - host-side emulator of the CUDA kernels.
 //
-// Compiles the SAME phase code the device runs (hex_gym_env_b200/csrc/hexb_phases.cuh, hexb_views.cuh) with
-// HEXB_HOST_EMU and replays one warp (chunk of 32 games) at a time: every phase is run for all 32 "lanes" before the
-// next one, which is what the __syncwarp() between phases guarantees on the GPU. It lets the CPU test-suite check the
-// device logic against the oracle in a container without a GPU. It is not a CPU fallback: the product package
-// never loads it, and it is far too slow to be one.
+// Compiles the SAME device code the kernels run (hex_gym_env_b200/csrc/hexb_phases.cuh, hexb_views.cuh, hexb_search.cuh,
+// hexb_mcts.cuh) with HEXB_HOST_EMU. The step kernel is replayed one warp (chunk of 32 games) at a time: every phase is run for
+// all 32 "lanes" before the next one, which is what the __syncwarp() between phases guarantees on the GPU. In the copy and
+// playout kernels a warp's ballot becomes a loop over its 32 lanes, and in the tree search the warp becomes one lane that owns
+// every cell and every path entry, so its shuffles become loops. The extern "C" entries mirror the device's launchers
+// (hexb_step_inst.cu, hexb_kernels.cu) and are driven through ctypes by tests/emu/emu.py. It lets the CPU test-suite check the
+// device logic against the oracle in a container without a GPU. It is not a CPU fallback: the product package never loads it,
+// and it is far too slow to be one.
 #define HEXB_HOST_EMU 1
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
 
+#include <type_traits>
 #include <vector>
 
-#include "../../hex_gym_env_b200/csrc/hexb_views.cuh"
+#include "../../hex_gym_env_b200/csrc/hexb_mcts.cuh"
 
 using namespace hexb;
 
@@ -129,15 +133,19 @@ static void run_tiles(Params P) {
     }
 }
 
-#define HEXB_FOR_N(X) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19)
-
-static void dispatch(const emu_env *e, const Params &P) {
-    switch (e->N) {
+// f(std::integral_constant<int, N>()) for the board size N, as the device's per-N launcher tables pick hexb_launch_*_<n>
+template <class F>
+static void for_board(int N, F &&f) {
+    switch (N) {
 #define X(n) \
-    case n: run_tiles<n>(P); break;
-        HEXB_FOR_N(X)
+    case n: f(std::integral_constant<int, n>()); break;
+        X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19)
 #undef X
     }
+}
+
+static void dispatch(const emu_env *e, const Params &P) {
+    for_board(e->N, [&](auto n) { run_tiles<n>(P); });
 }
 
 static View view_of(const emu_env *e) {
@@ -150,6 +158,47 @@ static View view_of(const emu_env *e) {
     V.raw = e->base.raw;
     V.obs_f32 = 0;
     return V;
+}
+
+// hexb_playout_kernel<N, POLICY>: one "warp" per game, its lanes' playouts one after another
+template <int N, int POLICY>
+static void playouts_n(const View &V, const PlayoutArgs &A) {
+    for (long long g = 0; g < V.G; ++g) {
+        uint32_t black[N], empty[N];
+        const int to_move = (A.game_mask && !A.game_mask[g]) ? -1 : playout_rows<N>(V, g, black, empty);
+        if (to_move < 0) {
+            A.wins[g] = -1;
+            continue;
+        }
+        int won = 0;
+        for (int j = 0; j < A.num; ++j)
+            won += playout_winner<N, POLICY>(black, empty, to_move, A.seed, A.game_offset + (unsigned long long)g, (uint32_t)(A.first + j),
+                                             -1) == to_move;
+        A.wins[g] = won;
+    }
+}
+
+// hexb_mcts_*_kernel<N>: op and policy as hexb_launch_mcts_<n> takes them; the tree buffer is host memory
+template <int N>
+static void mcts_n(int op, int policy, const View &V, const MctsArgs &A) {
+    if (op == MCTS_INIT) {
+        mc_write_header(A, N, V.G);
+        for (long long g = 0; g < V.G; ++g) mc_init_root<N>(V, A, g);
+        return;
+    }
+    Tree T;
+    if (!mc_tree(A, N, V.G, T)) return;
+    if (op == MCTS_ADVANCE) mc_write_first_playout(A);
+    for (long long g = 0; g < V.G; ++g) switch (op) {
+            case MCTS_SEARCH:
+                if (policy == PLAYOUT_BRIDGE) mc_search_root<N, PLAYOUT_BRIDGE>(T, A, V.variant, g);
+                else mc_search_root<N, PLAYOUT_RANDOM>(T, A, V.variant, g);
+                break;
+            case MCTS_SELECT: mc_select_root<N>(T, V, A, g); break;
+            case MCTS_EXPAND: mc_expand_root<N>(T, V, A, g); break;
+            case MCTS_ROOT: mc_root_out(T, V.variant, A, g); break;
+            case MCTS_ADVANCE: mc_advance_root<N>(T, V, A, g); break;
+        }
 }
 
 extern "C" {
@@ -233,12 +282,9 @@ void emu_encode(void *h, int view, int8_t *obs, uint8_t *mask) {
 void emu_sample_actions(void *h, int view, const double *u, int32_t *out) {
     emu_env *e = (emu_env *)h;
     const View V = view_of(e);
-    for (long long g = 0; g < V.G; ++g) switch (V.N) {
-#define X(n) \
-    case n: sample_at<n>(V, view, g, u, out); break;
-            HEXB_FOR_N(X)
-#undef X
-        }
+    for_board(V.N, [&](auto n) {
+        for (long long g = 0; g < V.G; ++g) sample_at<n>(V, view, g, u, out);
+    });
 }
 void emu_export_state(void *h, double *board, double *regions, double *counter, int8_t *cur, uint8_t *done, int8_t *winner,
                       int8_t *agent, uint32_t *draws) {
@@ -249,12 +295,9 @@ void emu_export_state(void *h, double *board, double *regions, double *counter, 
 }
 void emu_import_boards(void *h, const int8_t *board_true, const int8_t *to_move, const uint8_t *import_mask) {
     emu_env *e = (emu_env *)h;
-    for (long long g = 0; g < e->base.G; ++g) switch (e->N) {
-#define X(n) \
-    case n: import_game<n>(e->base, g, board_true, to_move, import_mask); break;
-            HEXB_FOR_N(X)
-#undef X
-        }
+    for_board(e->N, [&](auto n) {
+        for (long long g = 0; g < e->base.G; ++g) import_game<n>(e->base, g, board_true, to_move, import_mask);
+    });
 }
 void emu_import_labels(void *h, const int8_t *board_true, const uint8_t *planes, const int8_t *to_move, const uint8_t *import_mask) {
     emu_env *e = (emu_env *)h;
@@ -283,6 +326,87 @@ void emu_encode_byte(unsigned int b, int variant, unsigned int *obs, unsigned in
     uint32_t m;
     *obs = encode_byte(b, variant, false, m) & 0xffu;
     *msk = m;
+}
+
+// hexb_copy_games: dst must be a raw emulator batch of the same N and variant
+void emu_copy_games(void *dst_h, void *src_h, const int64_t *src_index, const int64_t *dst_index, long long count) {
+    emu_env *dst = (emu_env *)dst_h, *src = (emu_env *)src_h;
+    CopyArgs A;
+    A.dst = dst->base.state;
+    A.src = src->base.state;
+    A.dst_G = dst->base.G;
+    A.src_G = src->base.G;
+    A.count = count;
+    A.src_index = src_index;
+    A.dst_index = dst_index;
+    A.N = dst->N;
+    const int C = A.N * A.N, W = (C + 31) / 32;
+    for (long long i = 0; i < count; ++i) {   // one "warp" per pair
+        long long s, d;
+        if (!copy_pair(A, i, s, d)) continue;
+        const uint32_t meta = copy_src_meta(A, s);
+        const int tr = (meta & M_TRANSPOSED) ? 1 : 0;
+        for (int w = 0; w < W; ++w) {
+            uint32_t occ = 0;
+            for (int lane = 0; lane < 32; ++lane) {
+                const int c = 32 * w + lane;
+                if (c < C && copy_cell(A, s, d, c, tr)) occ |= 1u << lane;
+            }
+            copy_store_rec(A, d, w, occ);
+        }
+        copy_store_rec(A, d, W, copy_meta(meta));
+        copy_store_rec(A, d, W + 1, 0u);
+    }
+}
+
+// hexb_playouts_policy (policy PLAYOUT_RANDOM or PLAYOUT_BRIDGE)
+void emu_playouts(void *h, int num_playouts, long long first_playout, int policy, const uint8_t *game_mask, int32_t *wins) {
+    emu_env *e = (emu_env *)h;
+    const View V = view_of(e);
+    PlayoutArgs A;
+    A.seed = e->base.seed;
+    A.game_offset = (unsigned long long)e->base.game_offset;
+    A.first = first_playout;
+    A.num = num_playouts;
+    A.game_mask = game_mask;
+    A.wins = wins;
+    for_board(e->N, [&](auto n) {
+        if (policy == PLAYOUT_BRIDGE) playouts_n<n, PLAYOUT_BRIDGE>(V, A);
+        else playouts_n<n, PLAYOUT_RANDOM>(V, A);
+    });
+}
+
+long long emu_mcts_tree_bytes(int N, long long G, int max_nodes) { return 128 + mc_root_bytes(N, max_nodes) * G; }
+
+// every hexb_mcts_* call on a host tree buffer (op MCTS_INIT ... MCTS_ADVANCE); the arguments op does not use are ignored
+void emu_mcts(void *h, int op, uint8_t *tree, long long tree_bytes, int max_nodes, double c_puct, double fpu, long long first_playout,
+              const uint8_t *root_mask, int sims, int playouts, int policy, void *leaf_obs, uint8_t *leaf_mask, uint8_t *pending,
+              const float *priors, const float *values, int32_t *visits, float *q, float *value, int32_t *nodes_used) {
+    emu_env *e = (emu_env *)h;
+    const View V = view_of(e);
+    MctsArgs A;
+    memset(&A, 0, sizeof(A));
+    A.tree = tree;
+    A.tree_bytes = (unsigned long long)tree_bytes;
+    A.seed = e->base.seed;
+    A.game_offset = (unsigned long long)e->base.game_offset;
+    A.max_nodes = max_nodes;
+    A.c_puct = (float)c_puct;
+    A.fpu = (float)fpu;
+    A.first_playout = first_playout;
+    A.root_mask = root_mask;
+    A.sims = sims;
+    A.playouts = playouts;
+    A.leaf_obs = leaf_obs;
+    A.leaf_mask = leaf_mask;
+    A.pending = pending;
+    A.priors = priors;
+    A.values = values;
+    A.visits = visits;
+    A.q = q;
+    A.value = value;
+    A.nodes_used = nodes_used;
+    for_board(e->N, [&](auto n) { mcts_n<n>(op, policy, V, A); });
 }
 
 }  // extern "C"

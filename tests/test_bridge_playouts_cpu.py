@@ -9,8 +9,7 @@ import pytest
 import bridge_oracle as bo
 import mcts_common as mc
 import search_common as sc
-from emu import bridge_emu, mcts_emu, search_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS, playouts
 from oracle import playout
 from hex_gym_env_b200 import PLAYOUT_BRIDGE, PLAYOUT_RANDOM, _native
 
@@ -202,48 +201,47 @@ def test_emulated_bridge_playouts_match_the_rule(N):
     for variant, agent_mode, opp_first in sc.ENV_KINDS:
         seed = 1000 * N + 10 * variant + agent_mode
         env = env_batch(N, G, seed, variant, agent_mode, opp_first)
-        got = bridge_emu.playouts(env, P, first, policy=PLAYOUT_BRIDGE)
+        got = playouts(env, P, first, policy=PLAYOUT_BRIDGE)
         assert np.array_equal(got, oracle_wins(env, seed, 0, first, P, bo.PLAYOUT_BRIDGE)), (variant, agent_mode)
     for variant in (0, 1):
         raw = raw_batch(N, G, 77, variant, rng, game_offset=5)
-        got = bridge_emu.playouts(raw, P, first, policy=PLAYOUT_BRIDGE)
+        got = playouts(raw, P, first, policy=PLAYOUT_BRIDGE)
         assert np.array_equal(got, oracle_wins(raw, 77, 5, first, P, bo.PLAYOUT_BRIDGE)), variant
 
 
 def test_emulated_bridge_playouts_skip_finished_masked_and_unreset_games():
     N, G = 5, 64
     fresh = EmuBatch(1, N, G, seed=3, agent_mode=2)
-    assert (bridge_emu.playouts(fresh, 8, policy=PLAYOUT_BRIDGE) == -1).all()
+    assert (playouts(fresh, 8, policy=PLAYOUT_BRIDGE) == -1).all()
     env = env_batch(N, G, 3, 1, 2, False, steps=7, auto_reset=False)
     done = env.export()["done"].astype(bool)
     assert done.any() and not done.all()
     mask = np.ones(G, np.uint8)
     mask[::3] = 0
-    w = bridge_emu.playouts(env, 8, 0, mask, policy=PLAYOUT_BRIDGE)
+    w = playouts(env, 8, 0, mask, policy=PLAYOUT_BRIDGE)
     assert ((w == -1) == (done | (mask == 0))).all()
     assert np.array_equal(w, oracle_wins(env, 3, 0, 0, 8, bo.PLAYOUT_BRIDGE, mask))
 
 
 def test_bridge_policy_changes_some_results_and_random_is_unchanged():
-    """The two policies differ somewhere on a mid-game batch, and policy 0 is hexb_playouts (the oracle's random playouts, and
-    the emulated hexb_playouts / hexb_mcts_search of search_emu and mcts_emu byte for byte)."""
+    """The two policies differ somewhere on a mid-game batch, and policy 0 is the default of playouts and search and is the
+    oracle's random playouts."""
     env = env_batch(9, 16, 12, 1, 2, False)
-    r = bridge_emu.playouts(env, 64, 3)
-    assert np.array_equal(bridge_emu.playouts(env, 64, 3, policy=PLAYOUT_RANDOM), r)
-    assert np.array_equal(r, search_emu.playouts(env, 64, 3))
+    r = playouts(env, 64, 3)
+    assert np.array_equal(playouts(env, 64, 3, policy=PLAYOUT_RANDOM), r)
     assert np.array_equal(r, oracle_wins(env, 12, 0, 3, 64, bo.PLAYOUT_RANDOM))
-    assert not np.array_equal(bridge_emu.playouts(env, 64, 3, policy=PLAYOUT_BRIDGE), r)
-    old, new = mcts_emu.EmuMCTS(env, 60, 1.3, 0.0), bridge_emu.EmuMCTS(env, 60, 1.3, 0.0)
-    for t in (old, new):
+    assert not np.array_equal(playouts(env, 64, 3, policy=PLAYOUT_BRIDGE), r)
+    default, random = EmuMCTS(env, 60, 1.3, 0.0), EmuMCTS(env, 60, 1.3, 0.0)
+    for t in (default, random):
         t.reset(first_playout=5)
-    old.search(40, 3)
-    new.search(40, 3, PLAYOUT_RANDOM)
-    assert np.array_equal(old.tree, new.tree)
+    default.search(40, 3)
+    random.search(40, 3, PLAYOUT_RANDOM)
+    assert np.array_equal(default.tree, random.tree)
 
 
 def fused(batch, seed, game_offset, variant, max_nodes, S, P, policy, c_puct=1.5, fpu=0.25, first=3, root_mask=None, calls=None):
     """The emulated tree after S simulations of search_policy (in the given split of calls) and the restated trees."""
-    t = bridge_emu.EmuMCTS(batch, max_nodes, c_puct, fpu)
+    t = EmuMCTS(batch, max_nodes, c_puct, fpu)
     t.reset(root_mask, first)
     for k in (calls or (S,)):
         t.search(k, P, policy)
@@ -291,7 +289,7 @@ def test_emulated_bridge_search_masked_finished_unreset_and_full_pool():
     ex = env.export()
     assert ex["done"].any()
     t, orc = fused(env, 6, 0, 1, 9, 30, 2, bo.PLAYOUT_BRIDGE, root_mask=root_mask & reset_mask)
-    t2 = bridge_emu.EmuMCTS(env, 9, 1.5, 0.25)
+    t2 = EmuMCTS(env, 9, 1.5, 0.25)
     t2.reset(root_mask, 3)
     t2.search(30, 2, PLAYOUT_BRIDGE)
     assert np.array_equal(t.tree, t2.tree)                              # never-reset games are inactive without a mask
@@ -302,15 +300,15 @@ def test_emulated_bridge_search_masked_finished_unreset_and_full_pool():
 def test_emulated_bridge_search_calls_add_up():
     """search(a); search(b) equals search(a + b) under the bridge policy: the same bytes for every root."""
     env = env_batch(6, 9, 2, 1, 2, False)
-    a = bridge_emu.EmuMCTS(env, 80, 1.3, 0.0)
-    b = bridge_emu.EmuMCTS(env, 80, 1.3, 0.0)
+    a = EmuMCTS(env, 80, 1.3, 0.0)
+    b = EmuMCTS(env, 80, 1.3, 0.0)
     a.reset(first_playout=11)
     b.reset(first_playout=11)
     a.search(17, 4, PLAYOUT_BRIDGE)
     a.search(29, 4, PLAYOUT_BRIDGE)
     b.search(46, 4, PLAYOUT_BRIDGE)
     assert np.array_equal(a.tree, b.tree)
-    c = bridge_emu.EmuMCTS(env, 80, 1.3, 0.0)
+    c = EmuMCTS(env, 80, 1.3, 0.0)
     c.reset(first_playout=11)
     c.search(46, 4, PLAYOUT_RANDOM)
     assert not np.array_equal(c.tree, b.tree)
@@ -320,11 +318,11 @@ def test_emulated_bridge_search_first_simulation_is_the_playout_value():
     """Node 0's leaf has no previous move: after search(1) the root value is playouts_policy(bridge)'s."""
     P, first = 37, 9
     env = env_batch(7, 20, 3, 1, 2, False)
-    t = bridge_emu.EmuMCTS(env, 10)
+    t = EmuMCTS(env, 10)
     t.reset(first_playout=first)
     t.search(1, P, PLAYOUT_BRIDGE)
     _, _, value, used = t.root()
-    wins = bridge_emu.playouts(env, P, first, policy=PLAYOUT_BRIDGE)
+    wins = playouts(env, P, first, policy=PLAYOUT_BRIDGE)
     ok = wins >= 0
     want = (np.float32(2) * wins.astype(np.float32) - np.float32(P)) / np.float32(P)
     assert ((used > 0) == ok).all() and np.array_equal(value[ok], want[ok].astype(np.float32))
@@ -356,6 +354,6 @@ def test_python_policy_checks_without_a_gpu():
     env = EmuBatch(1, 5, 2, raw=True)
     for bad in (-1, 2):
         with pytest.raises(ValueError):
-            bridge_emu.playouts(env, 4, policy=bad)
+            playouts(env, 4, policy=bad)
         with pytest.raises(ValueError):
-            bridge_emu.EmuMCTS(env, 4).search(1, 1, bad)
+            EmuMCTS(env, 4).search(1, 1, bad)

@@ -9,8 +9,7 @@ import torch
 import bridge_oracle as bo
 import mcts_common as mc
 import search_common as sc
-from emu import bridge_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS, playouts
 from oracle import mcts, playout
 
 pytestmark = pytest.mark.gpu
@@ -118,9 +117,9 @@ def test_bridge_search_and_playouts_match_the_emulator_at_11x11(hb):
     emu = emu_env(N, G, 31, 1, 2, False)
     assert np.array_equal(host(env.export_state())["regions"], emu.export()["regions"])
     assert np.array_equal(env.playouts(96, 3, policy=hb.PLAYOUT_BRIDGE).cpu().numpy(),
-                          bridge_emu.playouts(emu, 96, 3, policy=hb.PLAYOUT_BRIDGE))
+                          playouts(emu, 96, 3, policy=hb.PLAYOUT_BRIDGE))
     t = hb.MCTS(env, 150, c_puct=1.25, fpu=0.5)                            # the pool fills before S + 1
-    e = bridge_emu.EmuMCTS(emu, 150, 1.25, 0.5)
+    e = EmuMCTS(emu, 150, 1.25, 0.5)
     t.reset(first_playout=7)
     e.reset(first_playout=7)
     t.search(S, P, policy=hb.PLAYOUT_BRIDGE)
@@ -284,7 +283,7 @@ def test_bridge_search_answers_intrusions(hb):
         visits = t.root()[0].cpu().numpy()
         emu = EmuBatch(1, N, G, seed=13, raw=True)
         emu.import_boards(boards, movers)
-        e = bridge_emu.EmuMCTS(emu, S + 1, 1.0, 1.0)
+        e = EmuMCTS(emu, S + 1, 1.0, 1.0)
         e.reset()
         e.search(S, P, policy)
         assert np.array_equal(visits, e.root()[0]), policy

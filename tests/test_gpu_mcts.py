@@ -8,8 +8,7 @@ import numpy as np
 import pytest
 import torch
 
-from emu import mcts_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS
 import mcts_common as mc
 import search_common as sc
 
@@ -103,7 +102,7 @@ def test_fused_and_split_match_the_emulator_at_11x11(hb):
     emu = emu_env(N, G, 31, 1, 2, False)
     assert np.array_equal(host(env.export_state())["regions"], emu.export()["regions"])
     t = hb.MCTS(env, 150, c_puct=1.25, fpu=0.5)                       # the pool fills before S + 1
-    e = mcts_emu.EmuMCTS(emu, 150, 1.25, 0.5)
+    e = EmuMCTS(emu, 150, 1.25, 0.5)
     t.reset(first_playout=7)
     e.reset(first_playout=7)
     t.search(S, P)
@@ -264,7 +263,7 @@ def test_one_move_wins(hb):
     visits = t.root()[0].cpu().numpy()
     emu = EmuBatch(1, N, G, seed=11, raw=True)
     emu.import_boards(boards, movers)
-    e = mcts_emu.EmuMCTS(emu, S + 1, 1.0, 1.0)
+    e = EmuMCTS(emu, S + 1, 1.0, 1.0)
     e.reset()
     e.search(S, P)
     assert np.array_equal(visits, e.root()[0])

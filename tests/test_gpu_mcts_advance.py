@@ -9,8 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from emu import mcts_advance_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS
 import mcts_advance_common as ma
 import mcts_common as mc
 import search_common as sc
@@ -126,7 +125,7 @@ def test_byte_identical_to_the_emulator_at_11x11(hb):
         env.step(outputs=False)
     emu = emu_pair(N, G, 31)
     t = hb.MCTS(env, 2 * S + 1, c_puct=1.25, fpu=0.0)
-    e = mcts_advance_emu.EmuMCTS(emu, 2 * S + 1, 1.25, 0.0)
+    e = EmuMCTS(emu, 2 * S + 1, 1.25, 0.0)
     t.reset(first_playout=7)
     e.reset(first_playout=7)
     kept = 0
@@ -259,5 +258,5 @@ def test_reuse_example_matches_the_emulator(hb):
     assert (r["reuse_wins"], r["reuse_black_wins"], r["reuse_white_wins"]) == REUSE_WINS_5X5
     emu = EmuBatch(1, 5, 64, seed=0, raw=True)
     emu.reset()
-    w, colour, held = mcts_reuse.play(emu, lambda: mcts_advance_emu.EmuMCTS(emu, 81, 1.25, 0.0), 40, 2, lambda x: x, lambda x: x)
+    w, colour, held = mcts_reuse.play(emu, lambda: EmuMCTS(emu, 81, 1.25, 0.0), 40, 2, lambda x: x, lambda x: x)
     assert mcts_reuse.summary(w, colour, held, 40, 2)["mean_visits_kept"] == r["mean_visits_kept"]

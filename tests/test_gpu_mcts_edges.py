@@ -7,8 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from emu import mcts_advance_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS
 import mcts_advance_common as ma
 import mcts_common as mc
 import search_common as sc
@@ -109,7 +108,7 @@ def test_device_equals_the_emulator(hb, N):
         else:
             dev, emu = raw_pair(hb, N, G, k, seed, rng)
         t = hb.MCTS(dev, M, c_puct=1.25, fpu=0.1)
-        e = mcts_advance_emu.EmuMCTS(emu, M, 1.25, 0.1)
+        e = EmuMCTS(emu, M, 1.25, 0.1)
         t.reset(first_playout=3 * N)
         e.reset(first_playout=3 * N)
         t.search(S, P)
@@ -135,7 +134,7 @@ def test_device_equals_the_emulator(hb, N):
         same(t, e)
     if N == 3:                                                        # the most playouts per leaf the ABI takes
         dev, emu = raw_pair(hb, N, 3, 1, 7, rng, fill=0.9)
-        t, e = hb.MCTS(dev, 4, c_puct=1.25, fpu=0.1), mcts_advance_emu.EmuMCTS(emu, 4, 1.25, 0.1)
+        t, e = hb.MCTS(dev, 4, c_puct=1.25, fpu=0.1), EmuMCTS(emu, 4, 1.25, 0.1)
         t.reset()
         e.reset()
         t.search(3, 65536)
@@ -170,7 +169,7 @@ def test_deep_lines(hb, N, S, deep, oracle):
     dev.import_boards(empty, to_move)
     emu.import_boards(empty, to_move)
     M = 2 * S + 2
-    t, e = hb.MCTS(dev, M, c_puct=1.0, fpu=-1.0), mcts_advance_emu.EmuMCTS(emu, M, 1.0, -1.0)
+    t, e = hb.MCTS(dev, M, c_puct=1.0, fpu=-1.0), EmuMCTS(emu, M, 1.0, -1.0)
     t.reset()
     e.reset()
     orc = mc.oracle_trees(emu.export(), 4, 0, 1, M, 1.0, -1.0, 0) if oracle else None
@@ -218,7 +217,7 @@ def test_float_edges(hb, c_puct, fpu):
     rng = np.random.default_rng(50 + mc.EDGE_SETTINGS.index((c_puct, fpu)))
     for variant, N in ((0, 4), (1, 5)):
         dev, emu = raw_pair(hb, N, 7, variant, 11, rng)
-        t, e = hb.MCTS(dev, 24, c_puct=c_puct, fpu=fpu), mcts_advance_emu.EmuMCTS(emu, 24, c_puct, fpu)
+        t, e = hb.MCTS(dev, 24, c_puct=c_puct, fpu=fpu), EmuMCTS(emu, 24, c_puct, fpu)
         t.reset()
         e.reset()
         orc = mc.oracle_trees(emu.export(), 11, 0, variant, 24, c_puct, fpu, 0)
@@ -236,7 +235,7 @@ def test_a_nan_child_gets_no_more_visits(hb, nan):
     board, to_move = np.full((G, N, N), 2, np.int8), np.zeros(G, np.int8)
     dev.import_boards(board, to_move)
     emu.import_boards(board, to_move)
-    t, e = hb.MCTS(dev, 64, c_puct=1.0, fpu=0.0), mcts_advance_emu.EmuMCTS(emu, 64, 1.0, 0.0)
+    t, e = hb.MCTS(dev, 64, c_puct=1.0, fpu=0.0), EmuMCTS(emu, 64, 1.0, 0.0)
     t.reset()
     e.reset()
     orc = mc.oracle_trees(emu.export(), 3, 0, 1, 64, 1.0, 0.0, 0)
@@ -266,7 +265,7 @@ def test_playout_key_past_2_to_the_32(hb, N):
     rng = np.random.default_rng(N)
     for variant in (0, 1):
         dev, emu = raw_pair(hb, N, 5, variant, 5, rng, game_offset=off)
-        t, e = hb.MCTS(dev, S + 1), mcts_advance_emu.EmuMCTS(emu, S + 1, 1.25, 0.0)
+        t, e = hb.MCTS(dev, S + 1), EmuMCTS(emu, S + 1, 1.25, 0.0)
         t.reset(first_playout=first)
         e.reset(first_playout=first)
         t.search(S, P)
@@ -302,7 +301,7 @@ def test_tree_past_4_gib(hb):
         n = hi - lo
         emu = EmuBatch(1, N, n, seed=8, game_offset=lo, raw=True)
         emu.import_boards(boards[lo:hi], to_move[lo:hi])
-        e = mcts_advance_emu.EmuMCTS(emu, M, 1.25, 0.0)
+        e = EmuMCTS(emu, M, 1.25, 0.0)
         e.reset(first_playout=11)
         e.search(S, P)
         part = np.concatenate([head, t.tree[128 + lo * rb:128 + hi * rb].cpu().numpy()])

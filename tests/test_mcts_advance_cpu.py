@@ -7,8 +7,7 @@ import ctypes
 import numpy as np
 import pytest
 
-from emu import mcts_advance_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS
 from oracle import mcts
 from hex_gym_env_b200 import _native
 import mcts_advance_common as ma
@@ -31,7 +30,7 @@ class Pair(object):
 
     def __init__(self, batch, seed, variant, max_nodes, first=1, root_mask=None, game_offset=0, live=None):
         self.batch, self.seed, self.variant, self.max_nodes, self.off = batch, seed, variant, max_nodes, game_offset
-        self.e = mcts_advance_emu.EmuMCTS(batch, max_nodes, C_PUCT, FPU)
+        self.e = EmuMCTS(batch, max_nodes, C_PUCT, FPU)
         self.e.reset(root_mask, first)
         om = root_mask if live is None else (live if root_mask is None else root_mask & live)
         self.orc = mc.oracle_trees(batch.export(), seed, game_offset, variant, max_nodes, C_PUCT, FPU, first, om)
@@ -362,7 +361,7 @@ def test_sharding_does_not_change_the_advance():
     for off, n in ((0, G), (0, H), (H, G - H)):
         raw = EmuBatch(0, N, n, seed=5, game_offset=off, raw=True)
         raw.import_boards(boards[off:off + n], to_move[off:off + n])
-        t = mcts_advance_emu.EmuMCTS(raw, 40)
+        t = EmuMCTS(raw, 40)
         t.reset()
         for m in range(3):
             t.search(30, 2)
@@ -386,11 +385,11 @@ def test_abi_argument_checks_without_a_gpu():
 def test_emulated_advance_on_a_foreign_buffer_writes_nothing():
     rng = np.random.default_rng(1)
     raw = raw_batch(5, 6, 1, 1, rng)
-    t = mcts_advance_emu.EmuMCTS(raw, 20)
+    t = EmuMCTS(raw, 20)
     t.advance(first_playout=5)                                                        # never initialised
     assert not t.tree.any()
     other = raw_batch(5, 7, 1, 1, rng)
-    u = mcts_advance_emu.EmuMCTS(other, 20)
+    u = EmuMCTS(other, 20)
     u.reset()
     u.search(10, 2)
     t.tree = u.tree.copy()                                                            # G differs

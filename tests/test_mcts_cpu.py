@@ -7,8 +7,7 @@ import ctypes
 import numpy as np
 import pytest
 
-from emu import mcts_emu, search_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS, copy_games, playouts
 from oracle import mcts, playout
 from hex_gym_env_b200 import _native
 import mcts_common as mc
@@ -34,7 +33,7 @@ def raw_batch(N, G, seed, variant, rng, game_offset=0):
 
 def fused(batch, seed, game_offset, variant, max_nodes, S, P, c_puct=1.5, fpu=0.25, first=3, root_mask=None, calls=(None,)):
     """The emulated tree after S simulations (in the given split of calls) and the oracle's trees after the same."""
-    t = mcts_emu.EmuMCTS(batch, max_nodes, c_puct, fpu)
+    t = EmuMCTS(batch, max_nodes, c_puct, fpu)
     t.reset(root_mask, first)
     for k in (calls if calls != (None,) else (S,)):
         t.search(k, P)
@@ -48,7 +47,7 @@ def fused(batch, seed, game_offset, variant, max_nodes, S, P, c_puct=1.5, fpu=0.
 def split(batch, seed, variant, max_nodes, S, rng, c_puct=1.1, fpu=-0.2, root_mask=None, check_obs=None, live=None):
     """S select / expand rounds with seeded priors and values on the emulator and the oracle; leaf obs, masks and pending flags
     compared every round. live: the games ever reset (an export does not show it), None = all."""
-    t = mcts_emu.EmuMCTS(batch, max_nodes, c_puct, fpu)
+    t = EmuMCTS(batch, max_nodes, c_puct, fpu)
     t.reset(root_mask)
     om = root_mask if live is None else (live if root_mask is None else root_mask & live)
     orc = mc.oracle_trees(batch.export(), seed, 0, variant, max_nodes, c_puct, fpu, 0, om)
@@ -184,8 +183,8 @@ def test_split_search_13x13_and_inactive_roots():
 def test_search_calls_add_up():
     """search(a); search(b) equals search(a + b): the same bytes for every root."""
     env = env_batch(6, 9, 2, 1, 2, False)
-    a = mcts_emu.EmuMCTS(env, 80, 1.3, 0.0)
-    b = mcts_emu.EmuMCTS(env, 80, 1.3, 0.0)
+    a = EmuMCTS(env, 80, 1.3, 0.0)
+    b = EmuMCTS(env, 80, 1.3, 0.0)
     a.reset(first_playout=11)
     b.reset(first_playout=11)
     a.search(17, 4)
@@ -199,11 +198,11 @@ def test_one_simulation_is_the_playout_value():
     P, first = 37, 9
     for variant, agent_mode, opp_first in sc.ENV_KINDS:
         env = env_batch(7, 20, 3 + variant, variant, agent_mode, opp_first)
-        t = mcts_emu.EmuMCTS(env, 10)
+        t = EmuMCTS(env, 10)
         t.reset(first_playout=first)
         t.search(1, P)
         visits, q, value, used = t.root()
-        wins = search_emu.playouts(env, P, first)
+        wins = playouts(env, P, first)
         ok = wins >= 0
         assert ((used > 0) == ok).all()
         want = (np.float32(2) * wins.astype(np.float32) - np.float32(P)) / np.float32(P)
@@ -220,7 +219,7 @@ def test_results_do_not_depend_on_sharding():
     for off, n in ((0, G), (0, H), (H, G - H)):
         raw = EmuBatch(1, N, n, seed=21, game_offset=off, raw=True)
         raw.import_boards(boards[off:off + n], to_move[off:off + n])
-        t = mcts_emu.EmuMCTS(raw, 40)
+        t = EmuMCTS(raw, 40)
         t.reset()
         t.search(30, 3)
         trees.append(mc.parse_tree(t.tree, N, n))
@@ -237,7 +236,7 @@ def test_split_leaf_obs_is_copy_ply_encode():
 
         def check(orc, obs, mask, pending):
             raw = EmuBatch(variant, N, G, raw=True)
-            search_emu.copy_games(raw, env)
+            copy_games(raw, env)
             paths = [o.leaf["cells"][1:] if o is not None and o.leaf is not None else [] for o in orc]
             for d in range(max(len(p) for p in paths)):
                 acts = np.full(G, -1, np.int32)
@@ -268,13 +267,13 @@ def test_abi_argument_checks_without_a_gpu():
 def test_emulated_calls_on_a_foreign_buffer_write_nothing():
     """A buffer that holds no tree of this batch (never initialised, or another batch's) is left alone."""
     env = env_batch(5, 6, 1, 1, 2, False)
-    t = mcts_emu.EmuMCTS(env, 20)
+    t = EmuMCTS(env, 20)
     t.search(5, 2)                                                                    # before any reset
     t.select()
     t.expand(np.ones((6, 25), np.float32), np.zeros(6, np.float32))
     assert not t.tree.any()
     other = env_batch(5, 7, 1, 1, 2, False)
-    u = mcts_emu.EmuMCTS(other, 20)
+    u = EmuMCTS(other, 20)
     u.reset()
     t.tree = u.tree.copy()                                                            # G differs
     t.search(5, 2)

@@ -5,8 +5,7 @@ that wrap mod 2^32 part-way through a simulation's playouts."""
 import numpy as np
 import pytest
 
-from emu import mcts_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, EmuMCTS
 from oracle import mcts
 import mcts_common as mc
 import search_common as sc
@@ -67,7 +66,7 @@ def one_root(N, board, to_move, c_puct, fpu):
     """A raw one-game batch holding `board`, and the emulator's and the oracle's trees on it."""
     raw = EmuBatch(1, N, 1, seed=3, raw=True)
     raw.import_boards(board[None], np.array([to_move], np.int8))
-    t = mcts_emu.EmuMCTS(raw, 64, c_puct, fpu)
+    t = EmuMCTS(raw, 64, c_puct, fpu)
     t.reset()
     o = mc.oracle_trees(raw.export(), 3, 0, 1, 64, c_puct, fpu, 0)
     return t, o
@@ -131,7 +130,7 @@ def test_float_edges_match_the_oracle(c_puct, fpu):
     rng = np.random.default_rng(mc.EDGE_SETTINGS.index((c_puct, fpu)))
     for variant, N in ((0, 4), (1, 5)):
         raw = raw_pair(N, 6, 11, variant, rng)
-        t = mcts_emu.EmuMCTS(raw, 20, c_puct, fpu)
+        t = EmuMCTS(raw, 20, c_puct, fpu)
         t.reset()
         orc = mc.oracle_trees(raw.export(), 11, 0, variant, 20, c_puct, fpu, 0)
         split_rounds(t, orc, 30, lambda mask: mc.edge_inputs(rng, raw.G, raw.C))
@@ -152,7 +151,7 @@ def test_playout_key_past_2_to_the_32(N):
         env.step()
     batches.append((env, 1))
     for b, variant in batches:
-        t = mcts_emu.EmuMCTS(b, S + 1, 1.25, 0.0)
+        t = EmuMCTS(b, S + 1, 1.25, 0.0)
         t.reset(first_playout=first)
         t.search(S, P)
         orc = mc.oracle_trees(b.export(), 5, off, variant, S + 1, 1.25, 0.0, first)

@@ -6,8 +6,7 @@ import ctypes
 import numpy as np
 import pytest
 
-from emu import search_emu
-from emu.emu import EmuBatch
+from emu.emu import EmuBatch, copy_games, playouts
 from oracle import hexref, playout
 from hex_gym_env_b200 import _native
 import search_common as sc
@@ -43,24 +42,24 @@ def test_emulated_playouts_match_the_oracle(N):
     for variant, agent_mode, opp_first in sc.ENV_KINDS:
         seed = 1000 * N + 10 * variant + agent_mode
         env = env_batch(N, G, seed, variant, agent_mode, opp_first)
-        assert np.array_equal(search_emu.playouts(env, P, first), oracle_wins(env, seed, 0, first, P)), (variant, agent_mode)
+        assert np.array_equal(playouts(env, P, first), oracle_wins(env, seed, 0, first, P)), (variant, agent_mode)
     for variant in (0, 1):
         raw = EmuBatch(variant, N, G, seed=77, game_offset=5, raw=True)
         boards, to_move = sc.random_boards(rng, G, N)
         raw.import_boards(boards, to_move)
-        assert np.array_equal(search_emu.playouts(raw, P, first), oracle_wins(raw, 77, 5, first, P)), variant
+        assert np.array_equal(playouts(raw, P, first), oracle_wins(raw, 77, 5, first, P)), variant
 
 
 def test_emulated_playouts_skip_finished_masked_and_unreset_games():
     N, G = 5, 64
     fresh = EmuBatch(1, N, G, seed=3, agent_mode=2)
-    assert (search_emu.playouts(fresh, 8) == -1).all()                       # never reset
+    assert (playouts(fresh, 8) == -1).all()                       # never reset
     env = env_batch(N, G, 3, 1, 2, False, steps=7, auto_reset=False)
     done = env.export()["done"].astype(bool)
     assert done.any() and not done.all()
     mask = np.ones(G, np.uint8)
     mask[::3] = 0
-    w = search_emu.playouts(env, 8, 0, mask)
+    w = playouts(env, 8, 0, mask)
     assert ((w == -1) == (done | (mask == 0))).all()
     assert ((w >= 0) & (w <= 8))[~done & (mask == 1)].all()
 
@@ -68,7 +67,7 @@ def test_emulated_playouts_skip_finished_masked_and_unreset_games():
 def test_emulated_playouts_first_playout_offsets_the_streams():
     """Playouts [0, 40) in one call are the sum of [0, 17) and [17, 40)."""
     env = env_batch(7, 8, 11, 1, 2, False)
-    assert np.array_equal(search_emu.playouts(env, 40, 0), search_emu.playouts(env, 17, 0) + search_emu.playouts(env, 23, 17))
+    assert np.array_equal(playouts(env, 40, 0), playouts(env, 17, 0) + playouts(env, 23, 17))
 
 
 @pytest.mark.parametrize("N", (3, 4, 5, 8, 11))
@@ -122,7 +121,7 @@ def test_emulated_env_to_raw_copy_exports_the_source_game(N, variant, agent_mode
     rng = np.random.default_rng(N)
     si = rng.permutation(G)
     di = si[::-1].copy()
-    search_emu.copy_games(dst, src, si, di)
+    copy_games(dst, src, si, di)
     a, b = src.export(), dst.export()
     for k in STATE_KEYS:
         assert np.array_equal(b[k][di], a[k][si]), k
@@ -154,15 +153,15 @@ def test_emulated_copy_broadcast_raw_to_raw_and_out_of_range():
     boards, to_move = sc.random_boards(np.random.default_rng(1), G, N)
     src.import_boards(boards, to_move)
     dst = EmuBatch(1, N, G * C + 2, raw=True)
-    search_emu.copy_games(dst, src, np.repeat(np.arange(G), C), None)     # null dst_index: identity
+    copy_games(dst, src, np.repeat(np.arange(G), C), None)     # null dst_index: identity
     a, b = src.export(), dst.export()
     for k in STATE_KEYS:
         assert np.array_equal(b[k][:G * C], np.repeat(a[k], C, axis=0)), k
     snap = dst.export()
-    search_emu.copy_games(dst, src, np.array([-1, G, 0, 1]), np.array([0, 1, G * C + 2, -5]))   # every pair out of range
+    copy_games(dst, src, np.array([-1, G, 0, 1]), np.array([0, 1, G * C + 2, -5]))   # every pair out of range
     for k in STATE_KEYS:
         assert np.array_equal(dst.export()[k], snap[k]), k
-    search_emu.copy_games(src, src, np.array([0]), np.array([3]))          # same batch, disjoint sets
+    copy_games(src, src, np.array([0]), np.array([3]))          # same batch, disjoint sets
     assert np.array_equal(src.export()["regions"][3], a["regions"][0])
 
 
